@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the merge hot path (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one calibration batch of RegMean Gram caching for VLMo-base all_moe (configs[1] of
@@ -142,6 +142,31 @@ def make_timed_cache(vlm):
     return TimedCache
 
 
+DUMP_GRAM_SAMPLES = 1 << 15
+
+
+def dump_outputs(path, logits, cache):
+    """What the timed calibration run hands its caller, as DIR/<name>.npy: `logits.npy`, the similarity logits of the
+    last timed step (float32), and one `gram.<module name>.npy` per Gram the run accumulated, in the cache's element
+    type (float32, or float64 for the RegMean-grade precisions).  A Gram file holds the Gram's diagonal followed by its
+    entries at DUMP_GRAM_SAMPLES upper-triangle positions drawn from a generator seeded with the Gram's width, so every
+    run and every build samples the same positions (VLMo-base: 96 files, 13 MB in float32)."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "logits.npy"), logits.float().cpu().numpy())
+    picks = {}
+    for name in cache.live_names():
+        g = cache.gram(name)
+        d = g.shape[0]
+        if d not in picks:
+            ij = torch.randint(0, d, (2, DUMP_GRAM_SAMPLES), generator=torch.Generator().manual_seed(d))
+            diag = torch.arange(d)
+            picks[d] = (torch.cat([diag, ij.min(0).values]).to(g.device), torch.cat([diag, ij.max(0).values]).to(g.device))
+        rows, cols = picks[d]
+        np.save(os.path.join(path, f"gram.{name}.npy"), g[rows, cols].cpu().numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
 
@@ -266,10 +291,13 @@ def run_ours(args):
     cache.reset()
     launches0 = vlm._lib.launch_count()
     cache.timing, cache.events = True, []
-    ms, t0, t1, ar_ms = timed(lambda i: step(dev_batches[i % 2]), args.steps, with_allreduce=True)
+    last = {}
+    ms, t0, t1, ar_ms = timed(lambda i: last.__setitem__("logits", step(dev_batches[i % 2])), args.steps, with_allreduce=True)
     cache.timing = False
     launches = vlm._lib.launch_count() - launches0
     n_live, reduce_bytes = len(cache.live_names()), getattr(cache, "last_reduce_bytes", 0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["logits"], cache)   # before the exchange below overwrites the Grams
     ar_alone_ms = None
     if world > 1:
         # the exchange step on its own, ranks aligned by a barrier first (the in-region figure also contains the wait
@@ -1198,7 +1226,11 @@ def main():
     ap.add_argument("--no-gpu-baseline", action="store_true", help="skip timing the reference's fp64 hook with the model on the GPU")
     ap.add_argument("--profile", action="store_true",
                     help="for ncu launch lists: run exactly --warmup + --steps calibration steps and exit (no JSON line)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's logits and a fixed sample of every Gram as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.profile):
+        ap.error("--dump-outputs writes the results of the timed GPU run: it needs --impl ours and no --profile")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -30,8 +30,16 @@ def test_reference_arm_line():
 
 
 @pytest.mark.gpu
-def test_gpu_arm_line():
-    d = _run(["--model", "tiny", "--steps", "3", "--warmup", "3", "--batch", "8"])
+def test_gpu_arm_line(tmp_path):
+    import numpy as np
+
+    d = _run(["--model", "tiny", "--steps", "3", "--warmup", "3", "--batch", "8", "--dump-outputs", str(tmp_path)])
+    logits = np.load(tmp_path / "logits.npy")
+    assert logits.shape == (8, 8) and logits.dtype == np.float32 and np.isfinite(logits).all()
+    grams = sorted(tmp_path.glob("gram.*.npy"))
+    assert len(grams) == 96 and sum(f.stat().st_size for f in tmp_path.iterdir()) <= 64 << 20
+    g = np.load(grams[0])
+    assert g.dtype == np.float32 and g.shape == (192 + (1 << 15),) and (g[:192] > 0).all()   # diagonal, then the sample
     assert BASE_KEYS | {"roofline", "clocks", "merge"} <= set(d)
     assert d["n_gpus"] == 1 and d["steps"] == 3 and d["warmup"] >= 3 and d["scaling"] == "weak" and d["value"] > 0
     r = d["roofline"]
