@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define VLM_ABI_VERSION 1
+#define VLM_ABI_VERSION 2
 
 typedef enum {
   VLM_OK = 0,
@@ -53,7 +53,7 @@ uint64_t    vlm_launch_count(void);
  *     flatten_input = input.reshape(-1, D).to(float64); gram = flatten_input.T @ flatten_input
  *     middle_representations[name] += gram.cpu()
  * G[r][c] += sum_k X[k][r] * X[k][c]  for every c >= r (upper triangle; elements below the
- * diagonal are scratch until vlm_sym_finalize).  X is the hooked activation viewed as
+ * diagonal are scratch until vlm_sym_mirror_batch).  X is the hooked activation viewed as
  * [rows, d] (f32 -> rounded to TF32 by TMA -> TF32 tensor cores, bf16/f16 -> f16-kind tensor cores), accumulation is fp32
  * in TMEM and fp32 in G.  Requires x 16-byte aligned and ldx*sizeof(elem) % 16 == 0, g 16-byte
  * aligned and ldg % 4 == 0; otherwise VLM_ERR_ALIGNMENT (use vlm_syrk_accum_simt).
@@ -78,10 +78,9 @@ int vlm_tf32_split(const float* x, int64_t rows, int d, int64_t ldx, int64_t seg
  * operands), which regmean's inverse (src/vilt/modules/vilt_module.py:432-434) amplifies on ill-conditioned
  * Gram sums; this entry point is the RegMean-grade mode (GramCache(precision="fp64")).  x: f32 / bf16 / f16,
  * any alignment (16-byte aligned rows take the cp.async path), optionally row-segmented (seg_rows = 0: plain
- * rows).  Upper block triangle only, like vlm_syrk_accum; vlm_sym_finalize_f64 mirrors it. */
+ * rows).  Upper block triangle only, like vlm_syrk_accum; vlm_sym_mirror_batch (dtype VLM_F64) mirrors it. */
 int vlm_syrk_accum_f64(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows,
                        int64_t seg_stride, double* g, int64_t ldg, void* stream);
-int vlm_sym_finalize_f64(double* g, int d, int64_t ldg, void* stream);
 
 /* The same Gram, exact, on the INTEGER tensor cores: each column is scaled by a power of two above its maximum in
  * this call and every value becomes four balanced int8 digits (q = rint(x * 2^(26-E_c)) = sum D_p * 128^(3-p));
@@ -128,24 +127,16 @@ int vlm_syrk_accum_strided(const void* x, int dtype, int64_t rows, int d, int64_
 int vlm_syrk_accum_simt(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
                         float* g, int64_t ldg, void* stream);
 
-/* Mirror the upper triangle into the lower one (G[c][r] = G[r][c], c > r) and, if out_f64 is not
- * NULL, also write the full symmetric matrix widened to fp64 — the dtype of the reference's Gram
- * file (src/cache_gram_matrices.py:251,349). */
-int vlm_sym_finalize(float* g, int d, int64_t ldg, double* out_f64, int64_t ld64, void* stream);
-
-/* Packed form of a Gram for the on-disk container (vl-merging_b200/gramfile.py; replaces the 2.15 GB fp64 pickle
- * of src/cache_gram_matrices.py:349 <-> src/vilt/modules/vilt_module.py:386 with 0.54 GB): row-major upper
- * triangle, row r = columns r..d-1 at element offset r*d - r*(r-1)/2, d*(d+1)/2 floats in all.  Only the upper
- * triangle of g is read (valid before or after vlm_sym_finalize). */
-int vlm_sym_pack_upper(const float* g, int d, int64_t ldg, float* packed, void* stream);
-/* Inverse: the full symmetric d x d matrix, as fp32 (out_dtype VLM_F32) or widened to fp64 (VLM_F64, the
- * reference's Gram dtype). */
-int vlm_sym_unpack(const float* packed, int d, void* out, int out_dtype, int64_t ldo, void* stream);
-/* The same for fp64 Grams (the int8x4 / fp64 cache modes): packed fp64 upper triangle <-> full symmetric fp64. */
-int vlm_sym_pack_upper_f64(const double* g, int d, int64_t ldg, double* packed, void* stream);
-int vlm_sym_unpack_f64(const double* packed, int d, double* out, int64_t ldo, void* stream);
-/* All Grams of a cache in ONE launch: items[i] = {full (d x d, pitch ld), packed, d}; every item has the element type
- * `dtype` (VLM_F32 or VLM_F64) on both sides.  pack reads `full`, unpack writes it (both triangles). */
+/* Symmetric Gram storage.  The SYRK entry points above form only the upper triangle of G; the packed form of a Gram is
+ * its row-major upper triangle, row r = columns r..d-1 at element offset r*d - r*(r-1)/2, d*(d+1)/2 values in all: the
+ * on-disk container (vl-merging_b200/gramfile.py; replaces the 2.15 GB fp64 pickle of src/cache_gram_matrices.py:349
+ * <-> src/vilt/modules/vilt_module.py:386 with 0.54 GB) and the exchange buffer of GramCache.all_reduce.
+ * Each call below treats all its Grams in ONE launch: items[i] = {full (d x d, pitch ld), packed, d}, every item of the
+ * element type `dtype` (VLM_F32 or VLM_F64) on both sides.
+ *   vlm_sym_pack_upper_batch  reads the upper triangle of `full` (below the diagonal is never read) into `packed`;
+ *   vlm_sym_unpack_batch      writes both triangles of `full` from `packed`;
+ *   vlm_sym_mirror_batch      in place: the lower triangle of `full` from its upper one (G[c][r] = G[r][c], c > r);
+ *                             `packed` is ignored and may be NULL. */
 typedef struct vlm_sym_item {
   const void* full;
   void* packed;
@@ -155,6 +146,7 @@ typedef struct vlm_sym_item {
 } vlm_sym_item;
 int vlm_sym_pack_upper_batch(const vlm_sym_item* items, int n, int dtype, void* stream);
 int vlm_sym_unpack_batch(const vlm_sym_item* items, int n, int dtype, void* stream);
+int vlm_sym_mirror_batch(const vlm_sym_item* items, int n, int dtype, void* stream);
 
 /* The exchange step of data-parallel Gram caching as ONE kernel over NVSwitch multicast memory (the reference has no
  * reduction: every DDP rank overwrites the same file, src/cache_gram_matrices.py:349).  multicast_base: the multicast
@@ -173,8 +165,6 @@ typedef struct vlm_sym_span {
 } vlm_sym_span;
 int vlm_sym_allreduce_multimem(void* multicast_base, const vlm_sym_span* spans, int n, int dtype, int rank, int world,
                                void* stream);
-/* Local, in place, one launch: the lower triangle of every Gram in `spans` (offsets from `base`) from its upper one. */
-int vlm_sym_mirror_batch(void* base, const vlm_sym_span* spans, int n, int dtype, void* stream);
 
 /* Host-only view of vlm_syrk_accum's work decomposition for (rows, d) on a device with nsm SMs
  * (elem_bytes 4 = f32, 2 = bf16/f16): writes segments as 5 int32 each {row_block_col0, col_block_col0,
@@ -232,7 +222,7 @@ int vlm_copy_batch(void* dst_base, const uint64_t* dst_off_bytes, const void* co
  *   later_weight += W.double() @ G (:424,475)   vlm_regmean_rhs
  *   matmul(later_weight, inverse(summed_gram)) (:432-434,:483-484)   vlm_spd_solve_right
  * All fp64 like the reference.  g_dtype is VLM_F64 (the reference's Gram file) or VLM_F32 (our
- * on-device Gram buffers); G must be the full symmetric matrix (after vlm_sym_finalize). */
+ * on-device Gram buffers); G must be the full symmetric matrix (after vlm_sym_mirror_batch). */
 int vlm_gram_scale_accum(const void* g, int g_dtype, int d, int64_t ldg, double alpha,
                          double* out, int64_t ldo, int accumulate, void* stream);
 /* acc[out_f][in_f] (+)= sum_k W[out_f][k] * Ghat[k][in_f];  W fp32 (out_f x in_f), G (in_f x in_f). */

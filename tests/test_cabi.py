@@ -25,7 +25,7 @@ def test_header_symbols_are_exported_and_bound():
     for n in names:
         assert hasattr(h, n), f"{n} declared in include/vlmerge.h but not exported"
     assert sorted(vlm._lib.SIGNATURES) == names  # the ctypes shim binds exactly the header
-    assert vlm._lib.lib().vlm_version() == 1
+    assert vlm._lib.lib().vlm_version() == 2
     assert vlm._lib.lib().vlm_last_error() is not None
 
 
@@ -40,7 +40,7 @@ def test_argument_validation_happens_before_any_cuda_call():
     assert L.vlm_syrk_accum(None, 0, 16, 128, 128, None, 128, None) == -1       # g is NULL
     assert b"g is NULL" in L.vlm_last_error()
     assert L.vlm_syrk_accum(None, 7, 16, 128, 128, None, 128, None) == -1       # bad dtype
-    assert L.vlm_sym_finalize(None, 128, 128, None, 0, None) == -1
+    assert L.vlm_sym_mirror_batch(None, 1, vlm._lib.VLM_F32, None) == -1
     assert L.vlm_merge_plan_run(None, None) == -1
     assert L.vlm_regmean_rhs(None, 1, 1, 1, None, 3, 1, 1.0, None, 1, 0, None) == -1
     # the integer-tensor-core Gram: dtype, width and alignment are checked up front

@@ -1,4 +1,4 @@
-"""GPU: the packed Gram container end to end — pack / unpack kernels bit-exact against numpy, GramCache ->
+"""GPU: the packed Gram container end to end — pack / unpack / mirror kernels bit-exact against numpy, GramCache ->
 packed file -> regmean identical to regmean on the live cache, and both conversions with the reference's
 own Gram file (torch.save of fp64 matrices, src/cache_gram_matrices.py:349)."""
 import os
@@ -18,29 +18,11 @@ from test_gramfile import _write_by_hand  # noqa: E402
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("d", [1, 31, 32, 33, 192, 768, 1000])
-def test_pack_unpack_bit_exact(d):
-    torch.manual_seed(d)
-    a = torch.randn(d, d, device="cuda")
-    upper = torch.triu(a) + torch.tril(torch.full_like(a, float("nan")), -1)    # garbage below the diagonal
-    lib, stream = _lib.lib(), torch.cuda.current_stream().cuda_stream
-    packed = torch.empty(d * (d + 1) // 2, device="cuda")
-    _lib.check(lib.vlm_sym_pack_upper(upper.data_ptr(), d, upper.stride(0), packed.data_ptr(), stream))
-    want = a.cpu().numpy()[np.triu_indices(d)]
-    assert np.array_equal(packed.cpu().numpy(), want)
-    sym = (torch.triu(a) + torch.triu(a, 1).t()).cpu().numpy()
-    for dtype, code in ((torch.float32, _lib.VLM_F32), (torch.float64, _lib.VLM_F64)):
-        out = torch.full((d, d + 3), -1.0, dtype=dtype, device="cuda")         # padded leading dimension
-        _lib.check(lib.vlm_sym_unpack(packed.data_ptr(), d, out.data_ptr(), code, out.stride(0), stream))
-        got = out.cpu().numpy()
-        assert np.array_equal(got[:, :d], sym.astype(got.dtype))
-        assert (got[:, d:] == -1.0).all()
-
-
 @pytest.mark.parametrize("dtype,code", [(torch.float32, 0), (torch.float64, 3)])
 def test_batched_pack_unpack_bit_exact(dtype, code):
-    """vlm_sym_pack_upper_batch / vlm_sym_unpack_batch: Grams of mixed widths in one launch each (the exchange buffer of
-    GramCache.all_reduce and the packed Gram file), fp32 and fp64, padded leading dimensions."""
+    """vlm_sym_pack_upper_batch / vlm_sym_unpack_batch / vlm_sym_mirror_batch: Grams of mixed widths in one launch each
+    (the exchange buffer of GramCache.all_reduce, the packed Gram file, GramCache.finalize), fp32 and fp64, padded
+    leading dimensions."""
     dims = [1, 31, 32, 33, 192, 768, 1000, 5, 256]
     torch.manual_seed(7)
     full = [torch.randn(d, d + (i % 3), dtype=dtype, device="cuda")[:, :d] for i, d in enumerate(dims)]
@@ -49,12 +31,7 @@ def test_batched_pack_unpack_bit_exact(dtype, code):
     sizes = [d * (d + 1) // 2 for d in dims]
     flat = torch.full((sum(sizes),), -7.0, dtype=dtype, device="cuda")
     lib, stream = _lib.lib(), torch.cuda.current_stream().cuda_stream
-    esz = flat.element_size()
-    items = (_lib.SymItem * len(dims))()
-    off = 0
-    for it, u, d, sz in zip(items, upper, dims, sizes):
-        it.full, it.packed, it.d, it.ld = u.data_ptr(), flat.data_ptr() + esz * off, d, u.stride(0)
-        off += sz
+    items = _lib.sym_items(upper, flat)
     _lib.check(lib.vlm_sym_pack_upper_batch(items, len(dims), code, stream))
     got = flat.cpu().numpy()
     off = 0
@@ -62,13 +39,23 @@ def test_batched_pack_unpack_bit_exact(dtype, code):
         assert np.array_equal(got[off: off + sz], a.cpu().numpy()[np.triu_indices(d)]), d
         off += sz
     outs = [torch.full((d, d + 2), -1.0, dtype=dtype, device="cuda") for d in dims]
-    for it, o in zip(items, outs):
-        it.full, it.ld = o.data_ptr(), o.stride(0)
-    _lib.check(lib.vlm_sym_unpack_batch(items, len(dims), code, stream))
+    _lib.check(lib.vlm_sym_unpack_batch(_lib.sym_items([o[:, :d] for o, d in zip(outs, dims)], flat), len(dims), code,
+                                        stream))
     for a, o, d in zip(full, outs, dims):
         sym = (torch.triu(a) + torch.triu(a, 1).t()).cpu().numpy()
         assert np.array_equal(o.cpu().numpy()[:, :d], sym) and (o.cpu().numpy()[:, d:] == -1.0).all(), d
     assert lib.vlm_sym_pack_upper_batch(items, len(dims), 1, stream) == -1          # bf16 is not a Gram type
+    # the mirror, in place: the NaNs below the diagonal become the transpose of the upper triangle; the upper triangle,
+    # the diagonal and the padding columns stay as they are
+    padded = [torch.randn(d, d + 1 + i % 3, dtype=dtype, device="cuda") for i, d in enumerate(dims)]
+    for p, d in zip(padded, dims):
+        p[:, :d] = torch.triu(p[:, :d]) + torch.tril(torch.full_like(p[:, :d], float("nan")), -1)
+    before = [p.cpu().numpy() for p in padded]
+    _lib.check(lib.vlm_sym_mirror_batch(_lib.sym_items([p[:, :d] for p, d in zip(padded, dims)]), len(dims), code, stream))
+    for p, b, d in zip(padded, before, dims):
+        got = p.cpu().numpy()
+        assert np.array_equal(got[:, :d], np.triu(b[:, :d]) + np.triu(b[:, :d], 1).T), d
+        assert np.array_equal(got[:, d:], b[:, d:]), d
 
 
 def test_hand_written_file_loads(tmp_path):

@@ -63,18 +63,14 @@ for it in range(3):
         L = _lib.lib()
         mc = int(cache._symm.multicast_ptr)
         timed("multimem kernel alone", lambda: _lib.check(L.vlm_sym_allreduce_multimem(mc, spans, len(live), 0, rank, world, st)))
-        timed("local mirror alone", lambda: _lib.check(L.vlm_sym_mirror_batch(arena.data_ptr(), spans, len(live), 0, st)))
+        items = _lib.sym_items([cache.buffers[n] for n in live])
+        timed("local mirror alone", lambda: _lib.check(L.vlm_sym_mirror_batch(items, len(live), 0, st)))
     else:
         from vl_merging_b200 import _lib
         live = cache.live_names()
-        sizes = [cache.buffers[n].shape[0] * (cache.buffers[n].shape[0] + 1) // 2 for n in live]
-        flat = torch.empty(sum(sizes), device=dev)
-        items = (_lib.SymItem * len(live))()
-        off = 0
-        for it_, n, sz in zip(items, live, sizes):
-            g = cache.buffers[n]
-            it_.full, it_.packed, it_.d, it_.ld = g.data_ptr(), flat.data_ptr() + 4 * off, g.shape[0], g.stride(0)
-            off += sz
+        grams = [cache.buffers[n] for n in live]
+        flat = torch.empty(sum(g.shape[0] * (g.shape[0] + 1) // 2 for g in grams), device=dev)
+        items = _lib.sym_items(grams, flat)
         st = torch.cuda.current_stream().cuda_stream
         L = _lib.lib()
         timed("pack (one launch)", lambda: _lib.check(L.vlm_sym_pack_upper_batch(items, len(live), 0, st)))

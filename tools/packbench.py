@@ -9,18 +9,15 @@ dev = torch.device("cuda")
 arena = torch.randn(sum(d * d for d in dims), device=dev)
 sizes = [d * (d + 1) // 2 for d in dims]
 flat = torch.empty(sum(sizes), device=dev)
-items = (_lib.SymItem * len(dims))()
-spans = (_lib.SymSpan * len(dims))()
-off = poff = 0
-for it, sp, d, sz in zip(items, spans, dims, sizes):
-    it.full, it.packed, it.d, it.ld = arena.data_ptr() + 4 * off, flat.data_ptr() + 4 * poff, d, d
-    sp.offset_bytes, sp.d, sp.ld = 4 * off, d, d
+grams, off = [], 0
+for d in dims:
+    grams.append(arena[off: off + d * d].view(d, d))
     off += d * d
-    poff += sz
+items = _lib.sym_items(grams, flat)
 L, st = _lib.lib(), torch.cuda.current_stream().cuda_stream
 fns = {"pack": lambda: L.vlm_sym_pack_upper_batch(items, len(dims), 0, st),
        "unpack": lambda: L.vlm_sym_unpack_batch(items, len(dims), 0, st),
-       "mirror": lambda: L.vlm_sym_mirror_batch(arena.data_ptr(), spans, len(dims), 0, st)}
+       "mirror": lambda: L.vlm_sym_mirror_batch(items, len(dims), 0, st)}
 for name, fn in fns.items():
     for _ in range(2):
         _lib.check(fn())

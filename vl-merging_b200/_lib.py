@@ -3,6 +3,7 @@
 There is no fallback: if the library is missing, or a call fails, the caller gets an exception.
 """
 import ctypes
+import itertools
 import os
 import subprocess
 from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_uint64, c_void_p
@@ -32,6 +33,20 @@ class MergeSeg(ctypes.Structure):
 class SymItem(ctypes.Structure):
     """vlm_sym_item"""
     _fields_ = [("full", c_void_p), ("packed", c_void_p), ("d", c_int32), ("reserved", c_int32), ("ld", c_int64)]
+
+
+def sym_items(grams, packed=None, offsets=None):
+    """vlm_sym_item array for the square row-major tensors `grams`.  packed: the flat tensor of the packed upper
+    triangles, Gram i's from element offsets[i] on (offsets None: back to back in list order); None for
+    vlm_sym_mirror_batch, which reads no packed form."""
+    items = (SymItem * len(grams))()
+    if offsets is None:
+        offsets = itertools.accumulate((g.shape[0] * (g.shape[0] + 1) // 2 for g in grams), initial=0)
+    for it, g, off in zip(items, grams, offsets):
+        it.full, it.d, it.ld = g.data_ptr(), g.shape[0], g.stride(0)
+        if packed is not None:
+            it.packed = packed.data_ptr() + packed.element_size() * off
+    return items
 
 
 class SymSpan(ctypes.Structure):
@@ -72,20 +87,14 @@ SIGNATURES = {
     "vlm_syrk_i8x4_scratch_bytes": (c_uint64, [c_int64, c_int]),
     "vlm_syrk_accum_i8x4": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_int64, c_int64, c_void_p, c_uint64,
                                     c_void_p, c_int64, c_void_p]),
-    "vlm_sym_finalize_f64": (c_int, [c_void_p, c_int, c_int64, c_void_p]),
     "vlm_syrk_accum_batch": (c_int, [POINTER(SyrkProblem), c_int, c_int, c_void_p]),
     "vlm_syrk_accum_strided": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_int64, c_int64, c_void_p, c_int64,
                                        c_void_p]),
     "vlm_syrk_accum_simt": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_void_p, c_int64, c_void_p]),
-    "vlm_sym_finalize": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_int64, c_void_p]),
-    "vlm_sym_pack_upper": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p]),
-    "vlm_sym_unpack": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, c_void_p]),
-    "vlm_sym_pack_upper_f64": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p]),
-    "vlm_sym_unpack_f64": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_void_p]),
     "vlm_sym_pack_upper_batch": (c_int, [POINTER(SymItem), c_int, c_int, c_void_p]),
     "vlm_sym_unpack_batch": (c_int, [POINTER(SymItem), c_int, c_int, c_void_p]),
     "vlm_sym_allreduce_multimem": (c_int, [c_void_p, POINTER(SymSpan), c_int, c_int, c_int, c_int, c_void_p]),
-    "vlm_sym_mirror_batch": (c_int, [c_void_p, POINTER(SymSpan), c_int, c_int, c_void_p]),
+    "vlm_sym_mirror_batch": (c_int, [POINTER(SymItem), c_int, c_int, c_void_p]),
     "vlm_syrk_schedule_host": (c_int, [c_int64, c_int, c_int, c_int, POINTER(c_int32), c_int, POINTER(c_int32),
                                        c_int, POINTER(c_int)]),
     "vlm_syrk_pair_schedule_host": (c_int, [c_int64, c_int, c_int, c_int, POINTER(c_int32), c_int, POINTER(c_int32),
@@ -136,8 +145,8 @@ def lib():
             fn = getattr(h, name)
             fn.restype = restype
             fn.argtypes = argtypes
-        if h.vlm_version() != 1:
-            raise RuntimeError(f"libvlmerge ABI version {h.vlm_version()} != 1")
+        if h.vlm_version() != 2:
+            raise RuntimeError(f"libvlmerge ABI version {h.vlm_version()} != 2: rebuild it (make -C vl-merging_b200/csrc)")
         _lib = h
     return _lib
 

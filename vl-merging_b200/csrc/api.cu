@@ -230,12 +230,6 @@ extern "C" int vlm_syrk_accum_i8x4(const void* x, int dtype, int64_t rows, int d
   return syrk_i8x4_launch(x, dtype, rows, d, ldx, seg_rows, seg_stride, scratch, g, ldg, static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int vlm_sym_finalize(float* g, int d, int64_t ldg, double* out_f64, int64_t ld64, void* stream) {
-  VLM_REQUIRE(g != nullptr && d > 0 && ldg >= d, VLM_ERR_INVALID_ARG, "vlm_sym_finalize: bad arguments");
-  VLM_REQUIRE(out_f64 == nullptr || ld64 >= d, VLM_ERR_INVALID_ARG, "vlm_sym_finalize: ld64 < d");
-  return sym_finalize_launch(g, d, ldg, out_f64, ld64, static_cast<cudaStream_t>(stream));
-}
-
 // Host-only view of the SYRK work decomposition (tests/test_schedule.py): fills up to cap segments
 // as 5 ints each {col_a, col_b, w, k0, k1} and ncta+1 offsets; returns the number of segments or
 // a negative vlm_status.

@@ -44,6 +44,12 @@ static inline float frand() {  // uniform (-1, 1)
 
 static int g_fail = 0;
 
+// the lower triangle of one d x d Gram (pitch ld) from its upper one
+static void mirror(void* g, int d, int64_t ld, int dtype) {
+  const vlm_sym_item it = {g, nullptr, d, 0, ld};
+  VK(vlm_sym_mirror_batch(&it, 1, dtype, nullptr));
+}
+
 struct Timer {
   cudaEvent_t a, b;
   Timer() {
@@ -194,7 +200,7 @@ static void syrk_case(const char* name, int dtype, int64_t rows, int d, int mode
   }
 
   // finalize: mirror check
-  VK(vlm_sym_finalize(g_tc, d, d, nullptr, 0, nullptr));
+  mirror(g_tc, d, d, VLM_F32);
   CK(cudaDeviceSynchronize());
   CK(cudaMemcpy(out.data(), g_tc, out.size() * 4, cudaMemcpyDeviceToHost));
   size_t asym = 0;
@@ -330,7 +336,7 @@ static void syrk_f64_case(const char* name, int dtype, int nseg, int n_tok, int 
   const int64_t sr = nseg > 1 ? seg_rows : 0;
   VK(vlm_syrk_accum_f64(slice, dtype, rows, d, d, sr, (int64_t)n_tok * d, g, d, nullptr));
   VK(vlm_syrk_accum_f64(slice, dtype, rows, d, d, sr, (int64_t)n_tok * d, g, d, nullptr));
-  VK(vlm_sym_finalize_f64(g, d, d, nullptr));
+  mirror(g, d, d, VLM_F64);
   cudaError_t e = cudaDeviceSynchronize();
   if (e != cudaSuccess) {
     printf("F64   %-27s KERNEL FAILED: %s\n", name, cudaGetErrorString(e));
@@ -402,7 +408,7 @@ static void syrk_i8_case(const char* name, int dtype, int nseg, int n_tok, int o
   const int64_t sr = nseg > 1 ? seg_rows : 0;
   VK(vlm_syrk_accum_i8x4(slice, dtype, rows, d, d, sr, (int64_t)n_tok * d, scratch, sbytes, g, d, nullptr));
   VK(vlm_syrk_accum_i8x4(slice, dtype, rows, d, d, sr, (int64_t)n_tok * d, scratch, sbytes, g, d, nullptr));
-  VK(vlm_sym_finalize_f64(g, d, d, nullptr));
+  mirror(g, d, d, VLM_F64);
   cudaError_t e = cudaDeviceSynchronize();
   if (e != cudaSuccess) {
     printf("I8X4  %-27s KERNEL FAILED: %s\n", name, cudaGetErrorString(e));
@@ -643,43 +649,47 @@ static void syrk_strided_case(const char* name, int dtype, int nseg, int n_tok, 
   CK(cudaFree(g3));
 }
 
-// ---- packed upper triangle (sympack.cu) ------------------------------------------------------
+// ---- symmetric storage (sympack.cu): pack, unpack and mirror of one Gram with a padded pitch ------------------
+// `g` and `out` start as copies of one random matrix; pack g, unpack into out, mirror g: both must then hold the
+// symmetric matrix of g's upper triangle, with the padding columns untouched.
+template <typename T>
 static void pack_case(int d, int pad) {
+  const int dtype = sizeof(T) == 4 ? VLM_F32 : VLM_F64;
   const int64_t ld = d + pad;
-  std::vector<float> h((size_t)d * ld);
+  std::vector<T> h((size_t)d * ld);
   for (auto& v : h) v = frand();
-  float *g, *packed, *o32;
-  double* o64;
+  T *g, *packed, *out;
   const size_t np = (size_t)d * (d + 1) / 2;
-  CK(cudaMalloc(&g, h.size() * 4));
-  CK(cudaMalloc(&packed, np * 4));
-  CK(cudaMalloc(&o32, (size_t)d * ld * 4));
-  CK(cudaMalloc(&o64, (size_t)d * ld * 8));
-  CK(cudaMemcpy(g, h.data(), h.size() * 4, cudaMemcpyHostToDevice));
-  VK(vlm_sym_pack_upper(g, d, ld, packed, nullptr));
-  VK(vlm_sym_unpack(packed, d, o32, VLM_F32, ld, nullptr));
-  VK(vlm_sym_unpack(packed, d, o64, VLM_F64, ld, nullptr));
+  CK(cudaMalloc(&g, h.size() * sizeof(T)));
+  CK(cudaMalloc(&packed, np * sizeof(T)));
+  CK(cudaMalloc(&out, h.size() * sizeof(T)));
+  CK(cudaMemcpy(g, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(out, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice));
+  vlm_sym_item it = {g, packed, d, 0, ld};
+  VK(vlm_sym_pack_upper_batch(&it, 1, dtype, nullptr));
+  it.full = out;
+  VK(vlm_sym_unpack_batch(&it, 1, dtype, nullptr));
+  mirror(g, d, ld, dtype);
   CK(cudaDeviceSynchronize());
-  std::vector<float> hp(np), h32((size_t)d * ld);
-  std::vector<double> h64((size_t)d * ld);
-  CK(cudaMemcpy(hp.data(), packed, np * 4, cudaMemcpyDeviceToHost));
-  CK(cudaMemcpy(h32.data(), o32, h32.size() * 4, cudaMemcpyDeviceToHost));
-  CK(cudaMemcpy(h64.data(), o64, h64.size() * 8, cudaMemcpyDeviceToHost));
+  std::vector<T> hp(np), hu(h.size()), hm(h.size());
+  CK(cudaMemcpy(hp.data(), packed, np * sizeof(T), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(hu.data(), out, hu.size() * sizeof(T), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(hm.data(), g, hm.size() * sizeof(T), cudaMemcpyDeviceToHost));
   size_t bad = 0, k = 0;
   for (int r = 0; r < d; ++r)
     for (int c = r; c < d; ++c, ++k) bad += hp[k] != h[(size_t)r * ld + c];
   for (int r = 0; r < d; ++r)
-    for (int c = 0; c < d; ++c) {
-      const float want = c >= r ? h[(size_t)r * ld + c] : h[(size_t)c * ld + r];
-      bad += h32[(size_t)r * ld + c] != want;
-      bad += h64[(size_t)r * ld + c] != (double)want;
+    for (int c = 0; c < ld; ++c) {
+      const T want = c < r ? h[(size_t)c * ld + r] : h[(size_t)r * ld + c];
+      bad += hu[(size_t)r * ld + c] != want;
+      bad += hm[(size_t)r * ld + c] != want;
     }
-  printf("PACK d=%-5d ld=%-5lld mismatches=%zu  %s\n", d, (long long)ld, bad, bad == 0 ? "OK" : "FAIL");
+  printf("PACK %s d=%-5d ld=%-5lld mismatches=%zu  %s\n", dtype == VLM_F32 ? "f32" : "f64", d, (long long)ld, bad,
+         bad == 0 ? "OK" : "FAIL");
   if (bad) ++g_fail;
   CK(cudaFree(g));
   CK(cudaFree(packed));
-  CK(cudaFree(o32));
-  CK(cudaFree(o64));
+  CK(cudaFree(out));
 }
 
 // ---- merge ---------------------------------------------------------------------------------
@@ -950,8 +960,11 @@ int main(int argc, char** argv) {
                     atoi(argv[4]), 5e-5);
     return g_fail;
   }
-  if (argc >= 2 && !strcmp(argv[1], "pack")) {  // packed upper-triangle kernels only (for compute-sanitizer)
-    for (int d : {1, 31, 33, 192, 768, 1000}) pack_case(d, d % 2 ? 3 : 0);
+  if (argc >= 2 && !strcmp(argv[1], "pack")) {  // pack / unpack / mirror kernels only (for compute-sanitizer)
+    for (int d : {1, 31, 33, 192, 768, 1000}) {
+      pack_case<float>(d, d % 2 ? 3 : 0);
+      pack_case<double>(d, d % 2 ? 3 : 0);
+    }
     return g_fail;
   }
   if (argc >= 9 && !strcmp(argv[1], "strided")) {  // selftest strided <f32|bf16> <nseg> <n_tok> <off> <seg_rows> <d> <iters>
@@ -977,7 +990,10 @@ int main(int argc, char** argv) {
   merge_case("mean3-misaligned", VLM_MERGE_MEAN, 3, 70001, 1, 0);
   merge_case("wsum2-misaligned", VLM_MERGE_WSUM, 2, 70001, 3, 0);
 
-  for (int d : {1, 33, 768}) pack_case(d, d % 2 ? 3 : 0);
+  for (int d : {1, 33, 768}) {
+    pack_case<float>(d, d % 2 ? 3 : 0);
+    pack_case<double>(d, d % 2 ? 3 : 0);
+  }
 
   regmean_case(96, 128, 1.0);
   regmean_case(200, 192, 0.9);

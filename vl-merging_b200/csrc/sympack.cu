@@ -1,9 +1,11 @@
-// sympack.cu — packed-upper-triangle form of a Gram matrix (the on-disk container of gramfile.py).
+// sympack.cu — the storage rule of every Gram, in three batched launches.
 //
 // A Gram is symmetric, and the SYRK kernels only ever form its upper triangle; the reference nevertheless
 // writes the full matrix in fp64 (src/cache_gram_matrices.py:251,349: 2.15 GB for VLMo-base, 7.65 GB for ViT-L).
 // Packed row-major upper triangle in fp32 — row r holds columns r..d-1 at offset r*d - r(r-1)/2 — is a quarter
-// of that.  Both kernels are HBM-bound copies; unpack goes through a 32x32 shared-memory tile so that the mirrored
+// of that.  pack / unpack convert between a full Gram and that form (the on-disk container of gramfile.py and the
+// exchange buffer of GramCache.all_reduce); mirror fills the lower triangle of a full Gram from its upper one, in
+// place.  All three are HBM-bound copies; unpack and mirror go through 32x32 shared-memory tiles so that the mirrored
 // half is written with coalesced rows too.
 #include <vector>
 
@@ -17,51 +19,12 @@ __device__ __forceinline__ int64_t packed_row_offset(int r, int d) {
   return (int64_t)r * d - ((int64_t)r * (r - 1)) / 2;
 }
 
-// one warp per row, rows interleaved over the grid (row r has d - r elements: interleaving balances the warps)
-template <typename T>
-__global__ void __launch_bounds__(256) sym_pack_kernel(const T* __restrict__ g, int d, int64_t ldg,
-                                                       T* __restrict__ packed) {
-  const int lane = threadIdx.x & 31;
-  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int nwarp = (gridDim.x * blockDim.x) >> 5;
-  for (int r = warp; r < d; r += nwarp) {
-    const T* src = g + (int64_t)r * ldg;
-    T* dst = packed + packed_row_offset(r, d) - r;
-    for (int c = r + lane; c < d; c += 32) dst[c] = src[c];
-  }
-}
-
-// tile (bi, bj), bj >= bi: read the packed rows of the tile once, write out[r][c] and, transposed, out[c][r]
-template <typename IN, typename OUT>
-__global__ void __launch_bounds__(256) sym_unpack_kernel(const IN* __restrict__ packed, int d,
-                                                         OUT* __restrict__ out, int64_t ldo) {
-  const int bi = blockIdx.y, bj = blockIdx.x;
-  if (bj < bi) return;
-  __shared__ IN t[32][33];
-  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-  for (int rr = ty; rr < 32; rr += 8) {
-    const int r = bi * 32 + rr, c = bj * 32 + tx;
-    IN v = 0;
-    if (r < d && c < d) {
-      v = (c >= r) ? packed[packed_row_offset(r, d) + (c - r)] : packed[packed_row_offset(c, d) + (r - c)];
-      out[(int64_t)r * ldo + c] = (OUT)v;
-    }
-    t[rr][tx] = v;
-  }
-  if (bj == bi) return;
-  __syncthreads();
-  for (int rr = ty; rr < 32; rr += 8) {
-    const int r = bj * 32 + rr, c = bi * 32 + tx;  // mirrored position, below the diagonal
-    if (r < d && c < d) out[(int64_t)r * ldo + c] = (OUT)t[tx][rr];
-  }
-}
-
-// ---- batched forms: all Grams of a cache in ONE launch (the exchange buffer of GramCache.all_reduce packs / unpacks
-// 96 Grams).  A block owns one 32-row BAND of one Gram and walks its tiles from the diagonal to the right edge with
-// several independent loads in flight per thread: the first version (one 32 x 32 tile per block, 262 K blocks moving
-// 8 KB each) ran at 1 TB/s — block turnover, not memory, was the limit. ------------------------------------------
+// All Grams of a cache in ONE launch (GramCache.all_reduce packs / unpacks 96 Grams, finalize mirrors them).  A block
+// owns one 32-row BAND of one Gram and walks its tiles from the diagonal to the right edge with several independent
+// loads in flight per thread: the first version (one 32 x 32 tile per block, 262 K blocks moving 8 KB each) ran at
+// 1 TB/s — block turnover, not memory, was the limit.
 struct SymItemDev {
-  const void* full_c;   // pack: source; unpack: destination (cast away const)
+  const void* full_c;   // pack: source; unpack: destination, mirror: read and written (cast away const)
   void* packed;
   int d;
   int first_band;       // index of this problem's first 32-row band in the flattened grid
@@ -149,14 +112,57 @@ __global__ void __launch_bounds__(256) sym_unpack_batch_kernel(const SymItemDev*
   }
 }
 
-int sym_batch(const vlm_sym_item* items, int n, int dtype, bool pack, cudaStream_t s, const char* who) {
+// in place, the band's tiles two at a time through shared memory: the upper tiles are read and their transposes
+// written below the diagonal (inside the diagonal tile only the elements below it)
+template <typename T>
+__global__ void __launch_bounds__(256) sym_mirror_batch_kernel(const SymItemDev* __restrict__ items, int n) {
+  int bi;
+  const SymItemDev it = locate_band(items, n, blockIdx.x, &bi);
+  const int d = it.d, nt = (d + 31) / 32;
+  T* g = static_cast<T*>(const_cast<void*>(it.full_c));
+  __shared__ T tile[2][32][33];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  for (int bj0 = bi; bj0 < nt; bj0 += 2) {
+#pragma unroll
+    for (int u = 0; u < 2; ++u)
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const int r = bi * 32 + ty + 8 * k, c = (bj0 + u) * 32 + tx;
+        tile[u][ty + 8 * k][tx] = (bj0 + u < nt && r < d && c < d) ? g[(int64_t)r * it.ld + c] : T(0);
+      }
+    __syncthreads();
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {
+      if (bj0 + u >= nt) continue;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const int rr = ty + 8 * k;
+        const int r = (bj0 + u) * 32 + rr, c = bi * 32 + tx;      // mirrored position
+        if (r < d && c < d && (bj0 + u != bi || tx < rr)) g[(int64_t)r * it.ld + c] = tile[u][tx][rr];
+      }
+    }
+    __syncthreads();
+  }
+}
+
+enum class SymOp { kPack, kUnpack, kMirror };
+
+template <typename T>
+void launch_sym(SymOp op, unsigned bands, const SymItemDev* items, int n, cudaStream_t s) {
+  if (op == SymOp::kPack) sym_pack_batch_kernel<T><<<bands, 256, 0, s>>>(items, n);
+  else if (op == SymOp::kUnpack) sym_unpack_batch_kernel<T><<<bands, 256, 0, s>>>(items, n);
+  else sym_mirror_batch_kernel<T><<<bands, 256, 0, s>>>(items, n);
+}
+
+int sym_batch(const vlm_sym_item* items, int n, int dtype, SymOp op, cudaStream_t s, const char* who) {
   VLM_REQUIRE(items != nullptr && n >= 0, VLM_ERR_INVALID_ARG, "%s: bad arguments", who);
   VLM_REQUIRE(dtype == VLM_F32 || dtype == VLM_F64, VLM_ERR_INVALID_ARG, "%s: dtype must be VLM_F32 or VLM_F64 (got %d)", who, dtype);
   if (n == 0) return 0;
   std::vector<SymItemDev> host(n);
   int64_t bands = 0;
   for (int i = 0; i < n; ++i) {
-    VLM_REQUIRE(items[i].full != nullptr && items[i].packed != nullptr && items[i].d > 0 && items[i].ld >= items[i].d,
+    VLM_REQUIRE(items[i].full != nullptr && (items[i].packed != nullptr || op == SymOp::kMirror) && items[i].d > 0 &&
+                    items[i].ld >= items[i].d,
                 VLM_ERR_INVALID_ARG, "%s: bad item %d", who, i);
     VLM_REQUIRE(bands + (items[i].d + 31) / 32 < ((int64_t)1 << 31), VLM_ERR_INVALID_ARG, "%s: too many bands", who);
     host[i] = {items[i].full, items[i].packed, items[i].d, (int)bands, items[i].ld};
@@ -166,13 +172,8 @@ int sym_batch(const vlm_sym_item* items, int n, int dtype, bool pack, cudaStream
   if (int rc = keep_async_pool()) return rc;
   VLM_CUDA(cudaMallocAsync(&dev, sizeof(SymItemDev) * n, s));
   VLM_CUDA(cudaMemcpyAsync(dev, host.data(), sizeof(SymItemDev) * n, cudaMemcpyHostToDevice, s));   // pageable: staged before return
-  if (pack) {
-    if (dtype == VLM_F32) sym_pack_batch_kernel<float><<<(unsigned)bands, 256, 0, s>>>(dev, n);
-    else sym_pack_batch_kernel<double><<<(unsigned)bands, 256, 0, s>>>(dev, n);
-  } else {
-    if (dtype == VLM_F32) sym_unpack_batch_kernel<float><<<(unsigned)bands, 256, 0, s>>>(dev, n);
-    else sym_unpack_batch_kernel<double><<<(unsigned)bands, 256, 0, s>>>(dev, n);
-  }
+  if (dtype == VLM_F32) launch_sym<float>(op, (unsigned)bands, dev, n, s);
+  else launch_sym<double>(op, (unsigned)bands, dev, n, s);
   VLM_CUDA(cudaGetLastError());
   VLM_CUDA(cudaFreeAsync(dev, s));
   count_launch();
@@ -185,59 +186,11 @@ int sym_batch(const vlm_sym_item* items, int n, int dtype, bool pack, cudaStream
 using namespace vlm;
 
 extern "C" int vlm_sym_pack_upper_batch(const vlm_sym_item* items, int n, int dtype, void* stream) {
-  return sym_batch(items, n, dtype, true, static_cast<cudaStream_t>(stream), "vlm_sym_pack_upper_batch");
+  return sym_batch(items, n, dtype, SymOp::kPack, static_cast<cudaStream_t>(stream), "vlm_sym_pack_upper_batch");
 }
 extern "C" int vlm_sym_unpack_batch(const vlm_sym_item* items, int n, int dtype, void* stream) {
-  return sym_batch(items, n, dtype, false, static_cast<cudaStream_t>(stream), "vlm_sym_unpack_batch");
+  return sym_batch(items, n, dtype, SymOp::kUnpack, static_cast<cudaStream_t>(stream), "vlm_sym_unpack_batch");
 }
-
-extern "C" int vlm_sym_pack_upper(const float* g, int d, int64_t ldg, float* packed, void* stream) {
-  VLM_REQUIRE(g != nullptr && packed != nullptr && d > 0 && ldg >= d, VLM_ERR_INVALID_ARG,
-              "vlm_sym_pack_upper: bad arguments");
-  int nsm = 0;
-  if (int rc = device_sm_count(&nsm)) return rc;
-  const int blocks = std::min(nsm * 8, (d + 7) / 8);
-  sym_pack_kernel<float><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(g, d, ldg, packed);
-  VLM_CUDA(cudaGetLastError());
-  count_launch();
-  return 0;
-}
-
-// fp64 Grams (the RegMean-grade cache modes): the exchange buffer of GramCache.all_reduce
-extern "C" int vlm_sym_pack_upper_f64(const double* g, int d, int64_t ldg, double* packed, void* stream) {
-  VLM_REQUIRE(g != nullptr && packed != nullptr && d > 0 && ldg >= d, VLM_ERR_INVALID_ARG,
-              "vlm_sym_pack_upper_f64: bad arguments");
-  int nsm = 0;
-  if (int rc = device_sm_count(&nsm)) return rc;
-  const int blocks = std::min(nsm * 8, (d + 7) / 8);
-  sym_pack_kernel<double><<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(g, d, ldg, packed);
-  VLM_CUDA(cudaGetLastError());
-  count_launch();
-  return 0;
-}
-
-extern "C" int vlm_sym_unpack_f64(const double* packed, int d, double* out, int64_t ldo, void* stream) {
-  VLM_REQUIRE(packed != nullptr && out != nullptr && d > 0 && ldo >= d, VLM_ERR_INVALID_ARG,
-              "vlm_sym_unpack_f64: bad arguments");
-  const int nt = (d + 31) / 32;
-  sym_unpack_kernel<double, double><<<dim3(nt, nt), 256, 0, static_cast<cudaStream_t>(stream)>>>(packed, d, out, ldo);
-  VLM_CUDA(cudaGetLastError());
-  count_launch();
-  return 0;
-}
-
-extern "C" int vlm_sym_unpack(const float* packed, int d, void* out, int out_dtype, int64_t ldo, void* stream) {
-  VLM_REQUIRE(packed != nullptr && out != nullptr && d > 0 && ldo >= d, VLM_ERR_INVALID_ARG,
-              "vlm_sym_unpack: bad arguments");
-  VLM_REQUIRE(out_dtype == VLM_F32 || out_dtype == VLM_F64, VLM_ERR_INVALID_ARG,
-              "vlm_sym_unpack: out_dtype must be VLM_F32 or VLM_F64 (got %d)", out_dtype);
-  const int nt = (d + 31) / 32;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (out_dtype == VLM_F32)
-    sym_unpack_kernel<float, float><<<dim3(nt, nt), 256, 0, s>>>(packed, d, static_cast<float*>(out), ldo);
-  else
-    sym_unpack_kernel<float, double><<<dim3(nt, nt), 256, 0, s>>>(packed, d, static_cast<double*>(out), ldo);
-  VLM_CUDA(cudaGetLastError());
-  count_launch();
-  return 0;
+extern "C" int vlm_sym_mirror_batch(const vlm_sym_item* items, int n, int dtype, void* stream) {
+  return sym_batch(items, n, dtype, SymOp::kMirror, static_cast<cudaStream_t>(stream), "vlm_sym_mirror_batch");
 }

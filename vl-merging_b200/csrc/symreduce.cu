@@ -66,7 +66,7 @@ __device__ __forceinline__ SpanDev locate_band(const SpanDev* __restrict__ spans
 // (item + bi) % world; the other ranks' blocks exit at once.  A warp owns four rows of the band and walks each from
 // column 32 bi to d in fully contiguous pieces: 32 lanes x 16 bytes per multimem instruction, four instructions in
 // flight (multimem.ld_reduce x 4, then multimem.st x 4).  The sums go back into every rank's arena through the
-// switch; the lower triangles are mirrored locally afterwards (sym_mirror_batch_kernel), so every element of the
+// switch; the lower triangles are mirrored locally afterwards (vlm_sym_mirror_batch), so every element of the
 // upper triangles crosses NVLink once in each direction.  (A first version dealt 32 x 32 tiles to the ranks: 128-byte
 // runs, 1.9 ms for the 538 MB of VLMo-base at N = 2.)
 template <typename T, typename V, int VE>   // V: the access type (float4 / double), VE elements each
@@ -92,40 +92,6 @@ __global__ void __launch_bounds__(256) sym_allreduce_mc_kernel(uint8_t* __restri
       for (int u = 0; u < 4; ++u)
         if (c + u * kStep < d) mc_st(row + c + u * kStep, s[u]);
     }
-  }
-}
-
-// Local, in place, all spans in one launch: the lower triangle of every Gram from its upper one.  Same band walk, two
-// tiles at a time through shared memory.
-template <typename T>
-__global__ void __launch_bounds__(256) sym_mirror_batch_kernel(uint8_t* __restrict__ base, const SpanDev* __restrict__ spans,
-                                                               int n) {
-  int item, bi;
-  const SpanDev sp = locate_band(spans, n, blockIdx.x, &item, &bi);
-  const int d = sp.d, nt = (d + 31) / 32;
-  T* g = reinterpret_cast<T*>(base + sp.offset_bytes);
-  __shared__ T tile[2][32][33];
-  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-  for (int bj0 = bi; bj0 < nt; bj0 += 2) {
-#pragma unroll
-    for (int u = 0; u < 2; ++u)
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const int r = bi * 32 + ty + 8 * k, c = (bj0 + u) * 32 + tx;
-        tile[u][ty + 8 * k][tx] = (bj0 + u < nt && r < d && c < d) ? g[(int64_t)r * sp.ld + c] : T(0);
-      }
-    __syncthreads();
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      if (bj0 + u >= nt) continue;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const int rr = ty + 8 * k;
-        const int r = (bj0 + u) * 32 + rr, c = bi * 32 + tx;      // mirrored position
-        if (r < d && c < d && (bj0 + u != bi || tx < rr)) g[(int64_t)r * sp.ld + c] = tile[u][tx][rr];
-      }
-    }
-    __syncthreads();
   }
 }
 
@@ -169,25 +135,6 @@ extern "C" int vlm_sym_allreduce_multimem(void* multicast_base, const vlm_sym_sp
     sym_allreduce_mc_kernel<float, float4, 4><<<(unsigned)bands, 256, 0, s>>>(static_cast<uint8_t*>(multicast_base), dev, n, rank, world);
   else
     sym_allreduce_mc_kernel<double, double, 1><<<(unsigned)bands, 256, 0, s>>>(static_cast<uint8_t*>(multicast_base), dev, n, rank, world);
-  VLM_CUDA(cudaGetLastError());
-  VLM_CUDA(cudaFreeAsync(dev, s));
-  count_launch();
-  return 0;
-}
-
-extern "C" int vlm_sym_mirror_batch(void* base, const vlm_sym_span* spans, int n, int dtype, void* stream) {
-  VLM_REQUIRE(base != nullptr && spans != nullptr && n >= 0, VLM_ERR_INVALID_ARG, "vlm_sym_mirror_batch: bad arguments");
-  VLM_REQUIRE(dtype == VLM_F32 || dtype == VLM_F64, VLM_ERR_INVALID_ARG,
-              "vlm_sym_mirror_batch: dtype must be VLM_F32 or VLM_F64 (got %d)", dtype);
-  if (n == 0) return 0;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  SpanDev* dev = nullptr;
-  int64_t bands = 0;
-  if (int rc = upload_spans(spans, n, VLM_F64 /* no alignment demands here */, "vlm_sym_mirror_batch", s, &dev, &bands)) return rc;
-  if (dtype == VLM_F32)
-    sym_mirror_batch_kernel<float><<<(unsigned)bands, 256, 0, s>>>(static_cast<uint8_t*>(base), dev, n);
-  else
-    sym_mirror_batch_kernel<double><<<(unsigned)bands, 256, 0, s>>>(static_cast<uint8_t*>(base), dev, n);
   VLM_CUDA(cudaGetLastError());
   VLM_CUDA(cudaFreeAsync(dev, s));
   count_launch();

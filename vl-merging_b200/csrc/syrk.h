@@ -60,6 +60,5 @@ int syrk_pair_batch_launch(const vlm_syrk_problem* probs, int n, int dtype, cuda
 void build_syrk_pair_schedule_host(int64_t kc, int d, int nsm, std::vector<int32_t>* flat, std::vector<int>* off);
 int syrk_simt_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
                      cudaStream_t stream);
-int sym_finalize_launch(float* g, int d, int64_t ldg, double* out_f64, int64_t ld64, cudaStream_t stream);
 
 }  // namespace vlm

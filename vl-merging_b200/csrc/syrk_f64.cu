@@ -136,23 +136,6 @@ syrk_f64_kernel(const T* __restrict__ x, int64_t rows, int d, int64_t ldx, int64
     }
 }
 
-__global__ void __launch_bounds__(256) sym_mirror_f64_kernel(double* __restrict__ g, int d, int64_t ldg) {
-  __shared__ double tile[32][33];
-  // blocks over the strictly-lower 32 x 32 tiles (and the diagonal ones): read the upper tile (bx >= by), transpose
-  const int by = blockIdx.y, bx = blockIdx.x;
-  if (bx < by) return;
-  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-  for (int r = ty; r < 32; r += 8) {
-    const int row = by * 32 + r, col = bx * 32 + tx;
-    tile[r][tx] = (row < d && col < d) ? g[(int64_t)row * ldg + col] : 0.0;
-  }
-  __syncthreads();
-  for (int r = ty; r < 32; r += 8) {
-    const int row = bx * 32 + r, col = by * 32 + tx;  // transposed position
-    if (row < d && col < d && row > col) g[(int64_t)row * ldg + col] = tile[tx][r];
-  }
-}
-
 template <typename T>
 int launch_f64(const T* x, int64_t rows, int d, int64_t ldx, int64_t seg_rows, int64_t seg_stride, double* g, int64_t ldg,
                cudaStream_t stream) {
@@ -216,13 +199,4 @@ extern "C" int vlm_syrk_accum_f64(const void* x, int dtype, int64_t rows, int d,
   if (dtype == VLM_BF16)
     return launch_f64(static_cast<const __nv_bfloat16*>(x), rows, d, ldx, seg_rows, seg_stride, g, ldg, st);
   return launch_f64(static_cast<const __half*>(x), rows, d, ldx, seg_rows, seg_stride, g, ldg, st);
-}
-
-extern "C" int vlm_sym_finalize_f64(double* g, int d, int64_t ldg, void* stream) {
-  VLM_REQUIRE(g != nullptr && d > 0 && ldg >= d, VLM_ERR_INVALID_ARG, "vlm_sym_finalize_f64: bad arguments");
-  const unsigned nb = (unsigned)((d + 31) / 32);
-  sym_mirror_f64_kernel<<<dim3(nb, nb), 256, 0, static_cast<cudaStream_t>(stream)>>>(g, d, ldg);
-  VLM_CUDA(cudaGetLastError());
-  count_launch();
-  return 0;
 }

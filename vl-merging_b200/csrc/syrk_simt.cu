@@ -1,5 +1,5 @@
 // syrk_simt.cu — CUDA-core Gram accumulation (device-side debug oracle / path for activations TMA
-// cannot address) and the symmetric finalize (mirror + optional fp64 widening).
+// cannot address).
 // Same contract as the tensor-core kernel: G[r][c] += sum_k X[k][r]*X[k][c] for c >= r
 // (src/cache_gram_matrices.py:246-254 of the reference computes the full fp64 matrix).
 #include "common.cuh"
@@ -67,37 +67,6 @@ syrk_simt_kernel(const T* __restrict__ x, int64_t rows, int d, int64_t ldx, floa
     }
 }
 
-// One block per 32x32 tile pair (bj >= bi): read the upper tile, write its transpose below the
-// diagonal, optionally write both to the fp64 output.
-__global__ void __launch_bounds__(256)
-sym_finalize_kernel(float* __restrict__ g, int d, int64_t ldg, double* __restrict__ out, int64_t ldo) {
-  const int bi = blockIdx.y, bj = blockIdx.x;
-  if (bj < bi) return;
-  __shared__ float t[32][33];
-  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
-  for (int rr = ty; rr < 32; rr += 8) {
-    const int r = bi * 32 + rr, c = bj * 32 + tx;
-    float v = 0.f;
-    if (r < d && c < d) {
-      // inside a diagonal tile the authoritative copy of (r, c), c < r, is (c, r)
-      v = (c >= r) ? g[(int64_t)r * ldg + c] : g[(int64_t)c * ldg + r];
-      if (c < r) g[(int64_t)r * ldg + c] = v;
-      if (out) out[(int64_t)r * ldo + c] = (double)v;
-    }
-    t[rr][tx] = v;
-  }
-  __syncthreads();
-  if (bj == bi) return;
-  for (int rr = ty; rr < 32; rr += 8) {
-    const int r = bj * 32 + rr, c = bi * 32 + tx;  // mirrored position (below the diagonal)
-    if (r < d && c < d) {
-      const float v = t[tx][rr];
-      g[(int64_t)r * ldg + c] = v;
-      if (out) out[(int64_t)r * ldo + c] = (double)v;
-    }
-  }
-}
-
 }  // namespace
 
 int syrk_simt_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
@@ -113,14 +82,6 @@ int syrk_simt_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
         <<<grid, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(x), rows, d, ldx, g, ldg);
   else
     syrk_simt_kernel<__half><<<grid, 256, 0, stream>>>(static_cast<const __half*>(x), rows, d, ldx, g, ldg);
-  VLM_CUDA(cudaGetLastError());
-  count_launch();
-  return 0;
-}
-
-int sym_finalize_launch(float* g, int d, int64_t ldg, double* out_f64, int64_t ld64, cudaStream_t stream) {
-  const int nt = (d + 31) / 32;
-  sym_finalize_kernel<<<dim3(nt, nt), 256, 0, stream>>>(g, d, ldg, out_f64, ld64);
   VLM_CUDA(cudaGetLastError());
   count_launch();
   return 0;

@@ -179,6 +179,7 @@ class GramCache:
             raise ValueError(f"precision must be 'tf32', 'tf32x3', 'fp64' or 'int8x4' (got {precision!r})")
         self.precision = precision
         self.dtype = torch.float64 if precision in ("fp64", "int8x4") else torch.float32   # of the Gram buffers
+        self._sym_code = _lib.VLM_F64 if self.dtype == torch.float64 else _lib.VLM_F32    # vlm_sym_* dtype of the buffers
         self._planes = None    # scratch for the {hi, lo} planes of the split mode (grown on demand, reused in stream order)
         self._fn = self._lib.vlm_syrk_accum_simt if use_simt else self._lib.vlm_syrk_accum
         self.buffers = {}       # name -> fp32 [d, d] (upper triangle authoritative until finalize())
@@ -409,29 +410,26 @@ class GramCache:
             return self._all_reduce_multimem(group)
         if not packed:
             return reduce_gram_buffers(self.buffers, self._arenas, self.calls, self.rows, group)
-        names = agree_on_buffers(self.buffers, group,
-                                 lambda d: torch.zeros(d, d, dtype=self.dtype, device=self.device), device=self.device)
-        _reduce_counts(self.buffers, names, self.calls, self.rows, group)    # after this, live_names() agrees on every rank
-        live = [n for n in names if self.calls[n] > 0]
+        live = self._agree_on_live(group)
         if not live:
             return
-        f64 = self.dtype == torch.float64
-        esz = 8 if f64 else 4
-        sizes = [self.buffers[n].shape[0] * (self.buffers[n].shape[0] + 1) // 2 for n in live]
-        flat = torch.empty(sum(sizes), dtype=self.dtype, device=self.device)
+        grams = [self.buffers[n] for n in live]
+        flat = torch.empty(sum(g.shape[0] * (g.shape[0] + 1) // 2 for g in grams), dtype=self.dtype, device=self.device)
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        items = (_lib.SymItem * len(live))()
-        off = 0
-        for it, n, sz in zip(items, live, sizes):
-            g = self.buffers[n]
-            it.full, it.packed, it.d, it.ld = g.data_ptr(), flat.data_ptr() + esz * off, g.shape[0], g.stride(0)
-            off += sz
-        code = _lib.VLM_F64 if f64 else _lib.VLM_F32
-        _lib.check(self._lib.vlm_sym_pack_upper_batch(items, len(live), code, stream))       # one launch for all Grams
+        items = _lib.sym_items(grams, flat)
+        _lib.check(self._lib.vlm_sym_pack_upper_batch(items, len(live), self._sym_code, stream))   # one launch for all Grams
         dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
-        _lib.check(self._lib.vlm_sym_unpack_batch(items, len(live), code, stream))
+        _lib.check(self._lib.vlm_sym_unpack_batch(items, len(live), self._sym_code, stream))
         self._finalized = True
-        self.last_reduce_bytes = flat.numel() * esz
+        self.last_reduce_bytes = flat.numel() * flat.element_size()
+
+    def _agree_on_live(self, group):
+        """The first step of both exchanges: every rank agrees on the buffer set (creating zero buffers for names it
+        lacks) and sums the call / row counters; returns the names that fired on some rank, the same list everywhere."""
+        names = agree_on_buffers(self.buffers, group,
+                                 lambda d: torch.zeros(d, d, dtype=self.dtype, device=self.device), device=self.device)
+        _reduce_counts(self.buffers, names, self.calls, self.rows, group)
+        return [n for n in names if self.calls[n] > 0]
 
     def _all_reduce_multimem(self, group=None):
         """all_reduce() of a symmetric cache: one kernel over the NVSwitch multicast mapping of the arena, bracketed by
@@ -440,10 +438,7 @@ class GramCache:
         import torch.distributed._symmetric_memory as symm_mem
 
         group = group if group is not None else dist.group.WORLD
-        names = agree_on_buffers(self.buffers, group,
-                                 lambda d: torch.zeros(d, d, dtype=self.dtype, device=self.device), device=self.device)
-        _reduce_counts(self.buffers, names, self.calls, self.rows, group)
-        live = [n for n in names if self.calls[n] > 0]
+        live = self._agree_on_live(group)
         if not live:
             return
         if len(self._arenas) != 1:
@@ -465,13 +460,12 @@ class GramCache:
             g = self.buffers[n]
             sp.offset_bytes, sp.d, sp.ld = g.data_ptr() - lo, g.shape[0], g.stride(0)
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        code = _lib.VLM_F64 if self.dtype == torch.float64 else _lib.VLM_F32
         with torch.cuda.device(self.device):
             h.barrier(channel=0)               # every rank's Gram launches have completed
-            _lib.check(self._lib.vlm_sym_allreduce_multimem(mc, spans, len(live), code, dist.get_rank(group),
+            _lib.check(self._lib.vlm_sym_allreduce_multimem(mc, spans, len(live), self._sym_code, dist.get_rank(group),
                                                             dist.get_world_size(group), stream))
             h.barrier(channel=0)               # every rank's stores have landed everywhere
-            _lib.check(self._lib.vlm_sym_mirror_batch(lo, spans, len(live), code, stream))     # lower triangles, locally
+            self._mirror(live, stream)         # lower triangles, locally
         self._finalized = True
         esz = 8 if self.dtype == torch.float64 else 4
         self.last_reduce_bytes = sum(self.buffers[n].shape[0] * (self.buffers[n].shape[0] + 1) // 2 for n in live) * esz
@@ -481,14 +475,13 @@ class GramCache:
         self.flush()
         if self._finalized:
             return
-        stream = torch.cuda.current_stream(self.device).cuda_stream
-        for name in self.live_names():
-            g = self.buffers[name]
-            if self.dtype == torch.float64:
-                _lib.check(self._lib.vlm_sym_finalize_f64(g.data_ptr(), g.shape[0], g.stride(0), stream))
-            else:
-                _lib.check(self._lib.vlm_sym_finalize(g.data_ptr(), g.shape[0], g.stride(0), None, 0, stream))
+        self._mirror(self.live_names(), torch.cuda.current_stream(self.device).cuda_stream)
         self._finalized = True
+
+    def _mirror(self, names, stream):
+        """The lower triangles of the named Grams from their upper ones, in place: one launch."""
+        items = _lib.sym_items([self.buffers[n] for n in names])
+        _lib.check(self._lib.vlm_sym_mirror_batch(items, len(names), self._sym_code, stream))
 
     def gram(self, name):
         """Full symmetric fp32 Gram of one module, on the device."""
@@ -501,18 +494,10 @@ class GramCache:
         there; registration order here, which is the same for a sequential forward)."""
         self.finalize()
         out = defaultdict(float)
-        stream = torch.cuda.current_stream(self.device).cuda_stream
         for name in self.live_names():
-            g = self.buffers[name]
-            if self.dtype == torch.float64:
-                out[name] = g.to(device=device, dtype=dtype, copy=True)
-            elif dtype == torch.float64:
-                wide = torch.empty(g.shape, dtype=torch.float64, device=self.device)
-                _lib.check(self._lib.vlm_sym_finalize(g.data_ptr(), g.shape[0], g.stride(0), wide.data_ptr(),
-                                                      wide.stride(0), stream))
-                out[name] = wide.to(device)
-            else:
-                out[name] = g.to(device=device, dtype=dtype)
+            # dtype first, on the device (a blocking .to(device, dtype) would convert on the host, after the copy);
+            # an fp64 cache never hands out its own buffers, an fp32 one does for fp32 on its own device
+            out[name] = self.buffers[name].to(dtype).to(device, copy=self.dtype == dtype == torch.float64)
         return out
 
     def save(self, path):

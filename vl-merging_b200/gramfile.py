@@ -16,10 +16,10 @@ row-major UPPER TRIANGLE in fp32 (a quarter of the bytes) as one flat blob:
 dtype float32 is what the default cache accumulates; float64 (half the reference file instead of a quarter) keeps the
 Grams of the RegMean-grade caches (GramCache(precision="int8x4" / "fp64")) exactly.
 
-`GramCache.save_packed` / `save_packed` write it (pack kernel on the device, ONE device->host copy),
-`load_packed` reads it back as device matrices for `regmean` (ONE host->device copy + ONE unpack launch),
-and `export_reference` / `import_reference` convert to and from the reference's own file, so either side
-can consume the other's artefact.  The packing kernels are vlm_sym_pack_upper(_batch) / vlm_sym_unpack(_batch).
+`GramCache.save_packed` / `save_packed` write it (ONE pack launch on the device, ONE device->host copy),
+`load_packed` reads it back as device matrices for `regmean` (ONE host->device copy + ONE unpack launch, in the
+file's element type), and `export_reference` / `import_reference` convert to and from the reference's own file, so
+either side can consume the other's artefact.  The kernels are vlm_sym_pack_upper_batch / vlm_sym_unpack_batch.
 """
 import json
 import os
@@ -86,13 +86,11 @@ def save_packed(grams, path, rows=None, calls=None, device=None, dtype=None):
     with torch.cuda.device(device):
         packed = torch.empty(total, dtype=dtype, device=device)
         stream = torch.cuda.current_stream(device).cuda_stream
-        items, keep = (_lib.SymItem * len(entries))(), []
-        for it, e in zip(items, entries):
-            g = grams[e["name"]].detach().to(device=device, dtype=dtype)
-            if g.stride(1) != 1:
-                g = g.contiguous()
-            keep.append(g)
-            it.full, it.packed, it.d, it.ld = g.data_ptr(), packed.data_ptr() + esz * e["offset"], e["d"], g.stride(0)
+        keep = []
+        for n in names:
+            g = grams[n].detach().to(device=device, dtype=dtype)
+            keep.append(g if g.stride(1) == 1 else g.contiguous())
+        items = _lib.sym_items(keep, packed, [e["offset"] for e in entries])
         _lib.check(lib.vlm_sym_pack_upper_batch(items, len(entries), code, stream))   # one launch for all Grams
         host = torch.empty(total, dtype=dtype, pin_memory=True)
         host.copy_(packed, non_blocking=True)
@@ -132,7 +130,7 @@ def read_header(path, with_dtype=False):
 def load_packed(path, device=None, dtype=None):
     """{name: full symmetric (d, d) device tensor}: what regmean(gram_matrices=...) takes.  dtype: torch.float32 or
     torch.float64 of the returned matrices; None = the file's own.  One host->device copy of the blob, then one unpack
-    launch for all Grams (one per Gram when an fp32 file is widened to fp64)."""
+    launch for all Grams in the file's element type; another dtype is converted Gram by Gram after that."""
     device = _device_of(device)
     entries, off, fdtype = read_header(path, with_dtype=True)
     dtype = dtype or fdtype
@@ -153,26 +151,18 @@ def load_packed(path, device=None, dtype=None):
             if not n:
                 raise ValueError(f"{path}: short read")
             got += n
-    out = {}
     with torch.cuda.device(device):
         packed = host.to(device, non_blocking=True)
         stream = torch.cuda.current_stream(device).cuda_stream
-        same = dtype == fdtype or fdtype == torch.float64    # fp64 file: unpacked as fp64 (and narrowed after, if asked)
-        items = (_lib.SymItem * len(entries))()
-        for it, e in zip(items, entries):
-            g = out[e["name"]] = torch.empty(e["d"], e["d"], dtype=fdtype if same else dtype, device=device)
-            if same:                         # same element type on both sides: one launch for all Grams
-                it.full, it.packed, it.d, it.ld = g.data_ptr(), packed.data_ptr() + esz * e["offset"], e["d"], g.stride(0)
-            else:                            # fp32 file widened to the reference's fp64: one launch per Gram
-                _lib.check(lib.vlm_sym_unpack(packed.data_ptr() + 4 * e["offset"], e["d"], g.data_ptr(), _lib.VLM_F64,
-                                              g.stride(0), stream))
-        if same:
-            _lib.check(lib.vlm_sym_unpack_batch(items, len(entries), _lib.VLM_F32 if fdtype == torch.float32 else _lib.VLM_F64,
-                                                stream))
-            if dtype != fdtype:
-                out = {k: v.to(dtype) for k, v in out.items()}
+        grams = [torch.empty(e["d"], e["d"], dtype=fdtype, device=device) for e in entries]
+        items = _lib.sym_items(grams, packed, [e["offset"] for e in entries])
+        _lib.check(lib.vlm_sym_unpack_batch(items, len(grams), _lib.VLM_F32 if fdtype == torch.float32 else _lib.VLM_F64,
+                                            stream))
+        if dtype != fdtype:
+            for i in range(len(grams)):      # one Gram at a time: each file-dtype matrix is released once converted
+                grams[i] = grams[i].to(dtype)
         torch.cuda.current_stream(device).synchronize()   # `packed` and `host` may be released after this
-    return out
+    return {e["name"]: g for e, g in zip(entries, grams)}
 
 
 def export_reference(packed_path, reference_path, device=None):
