@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define VLM_ABI_VERSION 2
+#define VLM_ABI_VERSION 3
 
 typedef enum {
   VLM_OK = 0,
@@ -54,10 +54,12 @@ uint64_t    vlm_launch_count(void);
  *     middle_representations[name] += gram.cpu()
  * G[r][c] += sum_k X[k][r] * X[k][c]  for every c >= r (upper triangle; elements below the
  * diagonal are scratch until vlm_sym_mirror_batch).  X is the hooked activation viewed as
- * [rows, d] (f32 -> rounded to TF32 by TMA -> TF32 tensor cores, bf16/f16 -> f16-kind tensor cores), accumulation is fp32
- * in TMEM and fp32 in G.  Requires x 16-byte aligned and ldx*sizeof(elem) % 16 == 0, g 16-byte
- * aligned and ldg % 4 == 0; otherwise VLM_ERR_ALIGNMENT (use vlm_syrk_accum_simt).
- * rows == 0 is a no-op. */
+ * [rows, d]; any alignment and any width.  The tensor-core path (the CTA-pair kernel: f32 -> rounded to TF32 by TMA ->
+ * TF32 tensor cores, bf16/f16 -> f16-kind tensor cores, fp32 accumulation in TMEM and fp32 in G) takes X when d is a
+ * whole number of 128-byte column groups (d % 32 == 0 for f32, d % 64 == 0 for bf16/f16), x and g are 16-byte aligned,
+ * ldx*sizeof(elem) % 16 == 0 and ldg % 4 == 0.  Everything else runs on the CUDA-core kernel of vlm_syrk_accum_simt
+ * (fp32 FMA).  dtype VLM_TF32X2 has only the tensor-core path: VLM_ERR_UNSUPPORTED if d % 32 != 0, VLM_ERR_ALIGNMENT
+ * if the planes or g are not aligned as above.  rows == 0 is a no-op. */
 int vlm_syrk_accum(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
                    float* g, int64_t ldg, void* stream);
 
@@ -98,8 +100,8 @@ int vlm_syrk_accum_i8x4(const void* x, int dtype, int64_t rows, int d, int64_t l
 
 /* Several independent vlm_syrk_accum problems of the same dtype in ONE launch (e.g. the 48 small Grams of the
  * text tower of one forward, which are launch-bound one by one).  Same contract per problem; the activations
- * must stay alive and unmodified until `stream` has run the launch.  Problems TMA cannot address, or whose
- * column count is not a whole number of 128-byte groups, are issued as individual launches. */
+ * must stay alive and unmodified until `stream` has run the launch.  Problems outside the tensor-core condition of
+ * vlm_syrk_accum (for segmented ones also seg_stride*sizeof(elem) % 16 == 0) are issued as individual launches. */
 typedef struct {
   const void* x;
   int64_t     rows;        /* total rows (= number of row segments * seg_rows when segmented) */
@@ -117,13 +119,14 @@ int vlm_syrk_accum_batch(const vlm_syrk_problem* probs_host, int n, int dtype, v
  * seg_stride elements after segment s-1 — the view `h[:, a:b]` of a (B, N, D) activation that the fused
  * vision-language route feeds to the per-modality experts (src/vilt/modules/vision_transformer.py:619-637,
  * :667-677), where the reference's `input.reshape(-1, D)` (src/cache_gram_matrices.py:250) makes a copy.
- * Here the slice is read in place through a 4-D tensor map.  rows must be a multiple of seg_rows;
- * seg_stride * sizeof(elem) must be a multiple of 16.  Otherwise the contract of vlm_syrk_accum. */
+ * Here the slice is read in place through a 4-D tensor map when the tensor-core condition of vlm_syrk_accum holds and
+ * seg_stride * sizeof(elem) is a multiple of 16; otherwise each segment is one vlm_syrk_accum.  rows must be a multiple
+ * of seg_rows.  Otherwise the contract of vlm_syrk_accum. */
 int vlm_syrk_accum_strided(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows,
                            int64_t seg_stride, float* g, int64_t ldg, void* stream);
 
-/* Same contract on CUDA cores (fp32 FMA), any alignment.  Debug oracle on the device and the
- * path for activations TMA cannot address. */
+/* Same contract on CUDA cores (fp32 FMA), any alignment, whatever the shape.  Debug oracle on the device
+ * (GramCache(use_simt=True)) and the kernel vlm_syrk_accum runs outside its tensor-core condition. */
 int vlm_syrk_accum_simt(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
                         float* g, int64_t ldg, void* stream);
 
@@ -166,17 +169,11 @@ typedef struct vlm_sym_span {
 int vlm_sym_allreduce_multimem(void* multicast_base, const vlm_sym_span* spans, int n, int dtype, int rank, int world,
                                void* stream);
 
-/* Host-only view of vlm_syrk_accum's work decomposition for (rows, d) on a device with nsm SMs
- * (elem_bytes 4 = f32, 2 = bf16/f16): writes segments as 5 int32 each {row_block_col0, col_block_col0,
- * width_in_128_blocks, chunk_begin, chunk_end} and ncta+1 offsets into them.  Returns the number of
- * segments (>= 0) or a vlm_status.  No CUDA calls; used by the CPU tests. */
-int vlm_syrk_schedule_host(int64_t rows, int d, int elem_bytes, int nsm, int32_t* segs_out, int cap,
-                           int32_t* off_out, int off_cap, int* ncta_out);
-
-/* Same for the CTA-pair kernel (the default when d is a whole number of 128-byte column groups): 4 int32 per
- * segment {super_row, super_col (256-column units), chunk_begin, chunk_end} and ncluster+1 offsets.
- * elem_bytes 1 = the int8 digit-plane kernel (vlm_syrk_accum_i8x4): 32-row chunks, the phase (0, 1, 2) in bits 16.. of
- * super_col. */
+/* Host-only view of the work decomposition of vlm_syrk_accum's CTA-pair kernel for (rows, d) on a device with nsm SMs
+ * (elem_bytes 4 = f32, 2 = bf16/f16): writes segments as 4 int32 each {super_row, super_col (256-column units),
+ * chunk_begin, chunk_end} and ncluster+1 offsets into them.  elem_bytes 1 = the int8 digit-plane kernel
+ * (vlm_syrk_accum_i8x4): 32-row chunks, the phase (0, 1, 2) in bits 16.. of super_col.  Returns the number of segments
+ * (>= 0) or a vlm_status.  No CUDA calls; used by the CPU tests. */
 int vlm_syrk_pair_schedule_host(int64_t rows, int d, int elem_bytes, int nsm, int32_t* segs_out, int cap,
                                 int32_t* off_out, int off_cap, int* ncluster_out);
 

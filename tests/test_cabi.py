@@ -25,7 +25,7 @@ def test_header_symbols_are_exported_and_bound():
     for n in names:
         assert hasattr(h, n), f"{n} declared in include/vlmerge.h but not exported"
     assert sorted(vlm._lib.SIGNATURES) == names  # the ctypes shim binds exactly the header
-    assert vlm._lib.lib().vlm_version() == 2
+    assert vlm._lib.lib().vlm_version() == 3
     assert vlm._lib.lib().vlm_last_error() is not None
 
 

@@ -35,7 +35,7 @@ def _oracle_gram(x):
 @pytest.mark.parametrize("d", [768, 192, 200, 1024])
 def test_row_slices_are_read_in_place(dtype, d):
     """Text slice [0, 40) and image slice [40, N) of a (B, N, D) activation: vs the fp64 oracle on the slice, and
-    vs the same kernel on a contiguous copy.  d = 200 has no whole 128-byte column groups (first-generation kernel,
+    vs the same kernel on a contiguous copy.  d = 200 has no whole 128-byte column groups (CUDA-core kernel,
     one launch per segment)."""
     torch.manual_seed(d)
     h = torch.randn(6, 40 + 197, d, device="cuda").to(dtype)

@@ -76,6 +76,33 @@ def test_simt_and_tensor_core_paths_agree():
     assert rel_fro(a.state_dict()["g"].numpy(), ref) < 1e-3      # TF32
 
 
+@pytest.mark.parametrize("case", ["f32 start 4 bytes off", "f32 pitch d+1", "f32 d=200", "bf16 d=96"])
+def test_syrk_accum_runs_the_cuda_core_kernel_outside_the_tensor_core_condition(case):
+    """vlm_syrk_accum takes any alignment and width: an activation the CTA-pair kernel does not take runs, in one
+    launch, on the CUDA-core kernel, bit for bit what vlm_syrk_accum_simt computes.  With at most 2048 rows that kernel
+    has one row slice, so every output element is one atomic add onto zero: deterministic."""
+    rows = 2000
+    dtype, d, off, pitch = {"f32 start 4 bytes off": (torch.float32, 256, 1, 256),   # off, pitch in elements
+                            "f32 pitch d+1": (torch.float32, 256, 0, 257),
+                            "f32 d=200": (torch.float32, 200, 0, 200),
+                            "bf16 d=96": (torch.bfloat16, 96, 0, 96)}[case]
+    base = _x((rows * pitch + off,), torch.float32, 21).cuda().to(dtype)
+    x = base[off:].view(rows, pitch)[:, :d]
+    code = {torch.float32: vlm._lib.VLM_F32, torch.bfloat16: vlm._lib.VLM_BF16}[dtype]
+    L = vlm._lib.lib()
+    grams = []
+    for fn in (L.vlm_syrk_accum, L.vlm_syrk_accum_simt):
+        g = torch.zeros(d, d, device="cuda")
+        before = vlm._lib.launch_count()
+        rc = fn(x.data_ptr(), code, rows, d, pitch, g.data_ptr(), d, None)
+        assert rc == 0, L.vlm_last_error()
+        assert vlm._lib.launch_count() - before == 1
+        grams.append(g)
+    assert torch.equal(grams[0], grams[1])
+    xd = x.double()
+    assert rel_fro(grams[0].triu().cpu(), (xd.T @ xd).triu().cpu()) < 1e-5      # fp32 FMA
+
+
 @pytest.mark.parametrize("dtype,d", [(torch.float32, 768), (torch.float32, 3072), (torch.bfloat16, 3072),
                                      (torch.float16, 1024), (torch.float32, 4096)])
 def test_full_size_properties(dtype, d):
@@ -280,7 +307,7 @@ def test_side_stream_mode_matches_in_stream_launches(defer):
 def test_randomised_shape_sweep():
     """Seeded sweep over ragged shapes and dtypes: whole and partial 128-column blocks, row counts around the
     pipeline chunk (32 / 64 rows), widths that take the CTA-pair kernel (whole 128-byte groups) and widths that
-    take the first-generation kernel, pitched inputs.  Checker: the reference hook's fp64 arithmetic in torch."""
+    take the CUDA-core kernel, pitched inputs.  Checker: the reference hook's fp64 arithmetic in torch."""
     rng = np.random.default_rng(20261017)
     dtypes = [torch.float32, torch.bfloat16, torch.float16]
     for case in range(36):

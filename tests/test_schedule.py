@@ -1,5 +1,5 @@
-"""SYRK work decomposition (host logic of vlm_syrk_accum, no GPU): every (tile, chunk) is covered
-exactly once, only upper-triangular tiles appear, shares are balanced, rows are swept panel-major."""
+"""SYRK work decompositions (host logic of vlm_syrk_accum and vlm_syrk_accum_i8x4, no GPU): every (super-tile, chunk)
+is covered exactly once, only upper-triangular tiles appear, makespans are near the ideal share."""
 from collections import defaultdict
 
 import pytest
@@ -8,58 +8,6 @@ import vl_merging_b200 as vlm
 
 CASES = [(36928, 768, 4), (36928, 3072, 4), (2560, 768, 4), (2560, 3072, 2), (36928, 1024, 2), (36928, 4096, 4),
          (1, 8, 4), (64, 128, 4), (1000, 900, 4), (77, 200, 2), (5000, 129, 4)]
-
-
-@pytest.mark.parametrize("rows,d,elem", CASES)
-def test_schedule_covers_upper_triangle_once(rows, d, elem):
-    segs, off = vlm._lib.syrk_schedule(rows, d, elem, 148)
-    bk = 128 // elem
-    kc = (rows + bk - 1) // bk
-    nb = (d + 127) // 128
-    assert off[0] == 0 and off[-1] == len(segs) and 1 <= len(off) - 1 <= 148
-    cover = defaultdict(list)
-    costs = []
-    for c in range(len(off) - 1):
-        cost = 0
-        for a, b, w, k0, k1 in segs[off[c]: off[c + 1]]:
-            assert a % 128 == 0 and b % 128 == 0 and b >= a and w in (1, 2) and 0 <= k0 < k1 <= kc
-            assert b + 128 * w <= nb * 128
-            cover[(a, b, w)].append((k0, k1))
-            cost += w * (k1 - k0)
-        costs.append(cost)
-    blocks = set()
-    for (a, b, w), ivs in cover.items():
-        ivs.sort()
-        assert ivs[0][0] == 0 and ivs[-1][1] == kc
-        assert all(x[1] == y[0] for x, y in zip(ivs, ivs[1:]))  # no gap, no overlap along K
-        for u in range(w):
-            blk = (a // 128, b // 128 + u)
-            assert blk not in blocks
-            blocks.add(blk)
-    assert blocks == {(i, j) for i in range(nb) for j in range(i, nb)}
-    pc = max(32, int(40e6 / (128.0 * d)))
-    npanels = (kc + pc - 1) // pc
-    assert max(costs) - min(costs) <= 4 * npanels  # equal shares per panel up to one wide chunk
-
-
-def test_rows_are_swept_panel_major():
-    """All CTAs work on the same ~40 MB row panel at the same step of their lists (L2 locality), and
-    no accumulation runs across a panel boundary."""
-    segs, off = vlm._lib.syrk_schedule(36928, 3072, 4, 148)
-    for c in range(len(off) - 1):
-        mine = segs[off[c]: off[c + 1]]
-        pc = int(40e6 / (128.0 * 3072))                       # ~40 MB of X per panel
-        panels = [s[3] // pc for s in mine]
-        assert panels == sorted(panels)                       # panel by panel
-        assert set(panels) == set(range((1154 + pc - 1) // pc))  # every CTA takes part in every panel
-        assert all(s[3] // pc == (s[4] - 1) // pc for s in mine)
-
-
-def test_small_problems_use_fewer_ctas():
-    _, off = vlm._lib.syrk_schedule(64, 128, 4, 148)
-    assert len(off) - 1 == 1
-    _, off = vlm._lib.syrk_schedule(2560, 768, 4, 148)
-    assert len(off) - 1 < 148
 
 
 @pytest.mark.parametrize("rows,d,elem", [c for c in CASES if c[1] % (128 // c[2]) == 0])

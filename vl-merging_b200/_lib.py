@@ -95,8 +95,6 @@ SIGNATURES = {
     "vlm_sym_unpack_batch": (c_int, [POINTER(SymItem), c_int, c_int, c_void_p]),
     "vlm_sym_allreduce_multimem": (c_int, [c_void_p, POINTER(SymSpan), c_int, c_int, c_int, c_int, c_void_p]),
     "vlm_sym_mirror_batch": (c_int, [POINTER(SymItem), c_int, c_int, c_void_p]),
-    "vlm_syrk_schedule_host": (c_int, [c_int64, c_int, c_int, c_int, POINTER(c_int32), c_int, POINTER(c_int32),
-                                       c_int, POINTER(c_int)]),
     "vlm_syrk_pair_schedule_host": (c_int, [c_int64, c_int, c_int, c_int, POINTER(c_int32), c_int, POINTER(c_int32),
                                             c_int, POINTER(c_int)]),
     "vlm_merge_plan_create": (c_int, [POINTER(MergeSeg), c_int, POINTER(c_void_p)]),
@@ -145,8 +143,8 @@ def lib():
             fn = getattr(h, name)
             fn.restype = restype
             fn.argtypes = argtypes
-        if h.vlm_version() != 2:
-            raise RuntimeError(f"libvlmerge ABI version {h.vlm_version()} != 2: rebuild it (make -C vl-merging_b200/csrc)")
+        if h.vlm_version() != 3:
+            raise RuntimeError(f"libvlmerge ABI version {h.vlm_version()} != 3: rebuild it (make -C vl-merging_b200/csrc)")
         _lib = h
     return _lib
 
@@ -158,18 +156,6 @@ def check(rc):
 
 def launch_count():
     return int(lib().vlm_launch_count())
-
-
-def syrk_schedule(rows, d, elem_bytes=4, nsm=148):
-    """Host-side view of the SYRK work decomposition: (list of (col_a, col_b, w, k0, k1), offsets)."""
-    cap = 1 << 16
-    segs = (c_int32 * (5 * cap))()
-    off = (c_int32 * (nsm + 2))()
-    ncta = c_int(0)
-    n = lib().vlm_syrk_schedule_host(rows, d, elem_bytes, nsm, segs, cap, off, nsm + 2, ctypes.byref(ncta))
-    if n < 0:
-        check(n)
-    return [tuple(segs[5 * i: 5 * i + 5]) for i in range(n)], list(off[: ncta.value + 1])
 
 
 def syrk_pair_schedule(rows, d, elem_bytes=4, nsm=148):

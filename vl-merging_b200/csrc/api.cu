@@ -46,6 +46,21 @@ int device_sm_count(int* out) {
   return 0;
 }
 
+int tensor_map_encoder(EncodeTiledFn* out) {
+  static EncodeTiledFn encode = nullptr;
+  std::lock_guard<std::mutex> lk(g_dev_mu);
+  if (!encode) {
+    void* fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    VLM_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
+    VLM_REQUIRE(fn != nullptr && qres == cudaDriverEntryPointSuccess, VLM_ERR_DRIVER,
+                "cuTensorMapEncodeTiled not available from the driver");
+    encode = reinterpret_cast<EncodeTiledFn>(fn);
+  }
+  *out = encode;
+  return 0;
+}
+
 // The small descriptor tables of the batched launches come from cudaMallocAsync.  With its default release threshold
 // (0) the pool hands its memory back to the driver at every synchronisation and the next call pays a real allocation
 // (~0.3 ms, measured around the pack / unpack launches of GramCache.all_reduce): keep the pool's memory instead.
@@ -98,15 +113,15 @@ extern "C" int vlm_syrk_accum(const void* x, int dtype, int64_t rows, int d, int
   if (int rc = check_syrk_args("vlm_syrk_accum", x, dtype, rows, d, ldx, g, ldg)) return rc;
   if (rows == 0) return 0;
   if (int rc = require_sm100()) return rc;
-  // the CTA-pair kernel whenever the activation has whole 128-byte column groups, else the single-CTA kernel
-  if (dtype == VLM_TF32X2) {
-    VLM_REQUIRE(syrk_pair_supported(dtype, d, ldx), VLM_ERR_UNSUPPORTED,
+  const bool pair = syrk_pair_supported(dtype, x, d, ldx, 0, g, ldg);
+  if (dtype == VLM_TF32X2) {  // the planes exist only for the CTA-pair kernel
+    VLM_REQUIRE(d % 32 == 0, VLM_ERR_UNSUPPORTED,
                 "vlm_syrk_accum: VLM_TF32X2 needs d %% 32 == 0 (got %d); use vlm_syrk_accum_simt on the fp32 activation", d);
-    return syrk_pair_launch(x, dtype, rows, d, ldx, 0, 0, g, ldg, static_cast<cudaStream_t>(stream));
+    VLM_REQUIRE(pair, VLM_ERR_ALIGNMENT,
+                "vlm_syrk_accum: VLM_TF32X2 planes and g must be 16-byte aligned with ldx and ldg multiples of 4");
   }
-  if (syrk_pair_supported(dtype, d, ldx))
-    return syrk_pair_launch(x, dtype, rows, d, ldx, 0, 0, g, ldg, static_cast<cudaStream_t>(stream));
-  return syrk_tc_launch(x, dtype, rows, d, ldx, g, ldg, static_cast<cudaStream_t>(stream));
+  if (pair) return syrk_pair_launch(x, dtype, rows, d, ldx, 0, 0, g, ldg, static_cast<cudaStream_t>(stream));
+  return syrk_simt_launch(x, dtype, rows, d, ldx, g, ldg, static_cast<cudaStream_t>(stream));
 }
 
 namespace {
@@ -117,14 +132,7 @@ int check_segments(const char* who, int dtype, int64_t rows, int64_t seg_rows, i
   (void)dtype;
   return 0;
 }
-bool tma_addressable(const void* x, int elem, int64_t ldx, const float* g, int64_t ldg) {
-  return (reinterpret_cast<uintptr_t>(x) & 15) == 0 && ((ldx * elem) & 15) == 0 &&
-         (reinterpret_cast<uintptr_t>(g) & 15) == 0 && (ldg & 3) == 0;
-}
 }  // namespace
-
-extern "C" int vlm_syrk_accum_simt(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
-                                   void* stream);
 
 extern "C" int vlm_syrk_accum_strided(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows,
                                       int64_t seg_stride, float* g, int64_t ldg, void* stream) {
@@ -135,16 +143,13 @@ extern "C" int vlm_syrk_accum_strided(const void* x, int dtype, int64_t rows, in
   VLM_REQUIRE(dtype != VLM_TF32X2, VLM_ERR_INVALID_ARG,
               "vlm_syrk_accum_strided: VLM_TF32X2 planes are packed by vlm_tf32_split, they have no row segments");
   if (int rc = require_sm100()) return rc;
-  const int elem = dtype == VLM_F32 ? 4 : 2;
-  if (tma_addressable(x, elem, ldx, g, ldg) && ((seg_stride * elem) & 15) == 0 && syrk_pair_supported(dtype, d, ldx))
+  if (syrk_pair_supported(dtype, x, d, ldx, seg_stride, g, ldg))
     return syrk_pair_launch(x, dtype, rows, d, ldx, seg_rows, seg_stride, g, ldg, static_cast<cudaStream_t>(stream));
-  // shapes the CTA-pair kernel does not take: one launch per segment through the contiguous entry points
+  // row segments the CTA-pair kernel cannot read in one launch: one vlm_syrk_accum per segment
+  const int elem = dtype == VLM_F32 ? 4 : 2;
   for (int64_t s = 0; s < rows / seg_rows; ++s) {
     const char* xs = static_cast<const char*>(x) + (size_t)s * seg_stride * elem;
-    const bool ok = tma_addressable(xs, elem, ldx, g, ldg);
-    if (int rc = ok ? vlm_syrk_accum(xs, dtype, seg_rows, d, ldx, g, ldg, stream)
-                    : vlm_syrk_accum_simt(xs, dtype, seg_rows, d, ldx, g, ldg, stream))
-      return rc;
+    if (int rc = vlm_syrk_accum(xs, dtype, seg_rows, d, ldx, g, ldg, stream)) return rc;
   }
   return 0;
 }
@@ -158,21 +163,19 @@ extern "C" int vlm_syrk_accum_batch(const vlm_syrk_problem* probs, int n, int dt
     const vlm_syrk_problem& q = probs[p];
     if (int rc = check_syrk_args("vlm_syrk_accum_batch", q.x, dtype, q.rows, q.d, q.ldx, q.g, q.ldg)) return rc;
     if (q.rows == 0) continue;
-    const int elem = (dtype == VLM_F32 || dtype == VLM_TF32X2) ? 4 : 2;
     const bool segmented = dtype != VLM_TF32X2 && q.seg_rows > 0 && q.seg_rows < q.rows;
-    VLM_REQUIRE(dtype != VLM_TF32X2 || (tma_addressable(q.x, 4, q.ldx, q.g, q.ldg) && syrk_pair_supported(dtype, q.d, q.ldx)),
-                VLM_ERR_UNSUPPORTED, "vlm_syrk_accum_batch: VLM_TF32X2 needs d %% 32 == 0 and 16-byte aligned planes");
+    const bool pair = syrk_pair_supported(dtype, q.x, q.d, q.ldx, segmented ? q.seg_stride : 0, q.g, q.ldg);
+    VLM_REQUIRE(dtype != VLM_TF32X2 || pair, VLM_ERR_UNSUPPORTED,
+                "vlm_syrk_accum_batch: VLM_TF32X2 needs d %% 32 == 0 and 16-byte aligned planes");
     if (segmented) {
       if (int rc = check_segments("vlm_syrk_accum_batch", dtype, q.rows, q.seg_rows, q.seg_stride)) return rc;
     }
-    const bool tma_ok = tma_addressable(q.x, elem, q.ldx, q.g, q.ldg) && (!segmented || ((q.seg_stride * elem) & 15) == 0);
-    if (tma_ok && syrk_pair_supported(dtype, q.d, q.ldx)) {
+    if (pair) {
       grouped.push_back(q);
     } else if (segmented) {
       if (int rc = vlm_syrk_accum_strided(q.x, dtype, q.rows, q.d, q.ldx, q.seg_rows, q.seg_stride, q.g, q.ldg, stream))
         return rc;
-    } else if (int rc = tma_ok ? vlm_syrk_accum(q.x, dtype, q.rows, q.d, q.ldx, q.g, q.ldg, stream)
-                               : vlm_syrk_accum_simt(q.x, dtype, q.rows, q.d, q.ldx, q.g, q.ldg, stream)) {
+    } else if (int rc = vlm_syrk_accum(q.x, dtype, q.rows, q.d, q.ldx, q.g, q.ldg, stream)) {
       return rc;
     }
   }
@@ -228,31 +231,6 @@ extern "C" int vlm_syrk_accum_i8x4(const void* x, int dtype, int64_t rows, int d
               (unsigned long long)syrk_i8x4_scratch_bytes(rows, d));
   if (int rc = require_sm100()) return rc;
   return syrk_i8x4_launch(x, dtype, rows, d, ldx, seg_rows, seg_stride, scratch, g, ldg, static_cast<cudaStream_t>(stream));
-}
-
-// Host-only view of the SYRK work decomposition (tests/test_schedule.py): fills up to cap segments
-// as 5 ints each {col_a, col_b, w, k0, k1} and ncta+1 offsets; returns the number of segments or
-// a negative vlm_status.
-extern "C" int vlm_syrk_schedule_host(int64_t rows, int d, int elem_bytes, int nsm, int32_t* segs_out, int cap,
-                                      int32_t* off_out, int off_cap, int* ncta_out) {
-  VLM_REQUIRE(rows > 0 && d > 0 && (elem_bytes == 2 || elem_bytes == 4) && nsm > 0 && ncta_out, VLM_ERR_INVALID_ARG,
-              "vlm_syrk_schedule_host: bad arguments");
-  const int bk = 128 / elem_bytes;
-  std::vector<SyrkSeg> segs;
-  std::vector<int> off;
-  build_syrk_schedule((rows + bk - 1) / bk, d, nsm, &segs, &off);
-  *ncta_out = (int)off.size() - 1;
-  VLM_REQUIRE((int)segs.size() <= cap && (int)off.size() <= off_cap, VLM_ERR_INVALID_ARG,
-              "vlm_syrk_schedule_host: output capacity too small (%d segments)", (int)segs.size());
-  for (size_t i = 0; i < segs.size(); ++i) {
-    segs_out[5 * i + 0] = segs[i].col_a;
-    segs_out[5 * i + 1] = segs[i].col_b;
-    segs_out[5 * i + 2] = segs[i].w;
-    segs_out[5 * i + 3] = segs[i].k0;
-    segs_out[5 * i + 4] = segs[i].k1;
-  }
-  for (size_t i = 0; i < off.size(); ++i) off_out[i] = off[i];
-  return (int)segs.size();
 }
 
 extern "C" int vlm_syrk_pair_schedule_host(int64_t rows, int d, int elem_bytes, int nsm, int32_t* segs_out, int cap,

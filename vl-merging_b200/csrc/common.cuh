@@ -35,6 +35,11 @@ inline void count_launch(uint64_t n = 1) { g_launches.fetch_add(n, std::memory_o
   } while (0)
 
 int device_sm_count(int* out);
+// cuTensorMapEncodeTiled from the driver, looked up once per process
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+int tensor_map_encoder(EncodeTiledFn* out);
 int require_sm100();
 int keep_async_pool();   // before cudaMallocAsync: do not return the pool's memory to the driver at every sync
 

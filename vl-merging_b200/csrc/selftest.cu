@@ -1003,11 +1003,11 @@ int main(int argc, char** argv) {
   syrk_case<float>("f32 1 tile", VLM_F32, 64, 128, 0, true, 0, 2e-3);
   syrk_case<float>("f32 wide tile", VLM_F32, 200, 256, 0, true, 0, 2e-3);
   syrk_case<float>("f32 d=768 ragged rows", VLM_F32, 1000, 768, 0, true, 0, 2e-3);
-  syrk_case<float>("f32 d=200 ragged cols", VLM_F32, 333, 200, 1, true, 0, 2e-3);
-  syrk_case<float>("f32 d=900 oob group", VLM_F32, 130, 900, 0, true, 0, 2e-3);
+  syrk_case<float>("f32 d=200 CUDA-core route", VLM_F32, 333, 200, 1, true, 0, 2e-3);
+  syrk_case<float>("f32 d=900 CUDA-core route", VLM_F32, 130, 900, 0, true, 0, 2e-3);
   syrk_case<__nv_bfloat16>("bf16 d=768", VLM_BF16, 1000, 768, 0, true, 0, 1e-5);
   syrk_case<__half>("f16 d=768 positive", VLM_F16, 1000, 768, 1, true, 0, 1e-5);
-  syrk_case<__nv_bfloat16>("bf16 d=200 ragged", VLM_BF16, 77, 200, 1, true, 0, 1e-5);
+  syrk_case<__nv_bfloat16>("bf16 d=200 CUDA-core route", VLM_BF16, 77, 200, 1, true, 0, 1e-5);
   syrk_case<float>("f32 d=768 positive", VLM_F32, 2560, 768, 1, true, 0, 2e-3);
 
   // reference precision (fp64 DMMA)
@@ -1045,7 +1045,7 @@ int main(int argc, char** argv) {
   syrk_strided_case<float>("f32 text slice", VLM_F32, 8, 617, 0, 40, 768, true, 0, 2e-3);
   syrk_strided_case<float>("f32 image slice", VLM_F32, 4, 617, 40, 577, 768, true, 0, 2e-3);
   syrk_strided_case<__nv_bfloat16>("bf16 image slice", VLM_BF16, 4, 617, 40, 577, 768, true, 0, 1e-5);
-  syrk_strided_case<float>("f32 d=200 (gen-1 path)", VLM_F32, 3, 50, 7, 33, 200, true, 0, 2e-3);
+  syrk_strided_case<float>("f32 d=200 CUDA-core route", VLM_F32, 3, 50, 7, 33, 200, true, 0, 2e-3);
   syrk_strided_case<float>("f32 image slice x64", VLM_F32, 64, 617, 40, 577, 768, false, 20, 2e-4);
   syrk_strided_case<float>("f32 text slice x64", VLM_F32, 64, 617, 0, 40, 768, false, 20, 2e-4);
 

@@ -18,7 +18,6 @@
 //   Output: [m][splits][10] values (descending; -inf padded) and int32 columns (-1 padded); the `splits` partial
 //   lists of a row are merged by the caller (a stable sort of 10 * splits candidates).
 #include <algorithm>
-#include <mutex>
 
 #include "common.cuh"
 #include "umma.cuh"
@@ -199,31 +198,16 @@ sim_topk_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
   if (warp == 2) tmem_dealloc(tmem_base, 512);
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn g_encode_sim = nullptr;
-std::mutex g_sim_mu;
-
 int encode_feat_map(const void* p, int dtype, int64_t rows, int d, int64_t ld, int box_rows, CUtensorMap* tm) {
-  {
-    std::lock_guard<std::mutex> lk(g_sim_mu);
-    if (!g_encode_sim) {
-      void* fn = nullptr;
-      cudaDriverEntryPointQueryResult qres;
-      VLM_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-      VLM_REQUIRE(fn != nullptr && qres == cudaDriverEntryPointSuccess, VLM_ERR_DRIVER,
-                  "cuTensorMapEncodeTiled not available from the driver");
-      g_encode_sim = reinterpret_cast<EncodeTiledFn>(fn);
-    }
-  }
+  EncodeTiledFn encode = nullptr;
+  if (int rc = tensor_map_encoder(&encode)) return rc;
   cuuint64_t gdim[2] = {(cuuint64_t)d, (cuuint64_t)rows};
   cuuint64_t gstr[1] = {(cuuint64_t)ld * 2};
   cuuint32_t box[2] = {(cuuint32_t)sTK, (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode_sim(tm, dtype == VLM_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2,
-                            const_cast<void*>(p), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = encode(tm, dtype == VLM_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2,
+                      const_cast<void*>(p), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   VLM_REQUIRE(r == CUDA_SUCCESS, VLM_ERR_DRIVER, "cuTensorMapEncodeTiled(features) failed: CUresult %d", (int)r);
   return 0;
 }

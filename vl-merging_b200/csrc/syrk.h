@@ -1,8 +1,6 @@
 // syrk.h — declarations shared by the SYRK translation units.
 #pragma once
-#include <algorithm>
 #include <cstdint>
-#include <cstdlib>
 #include <vector>
 
 #include <cuda_runtime.h>
@@ -11,26 +9,6 @@
 
 namespace vlm {
 
-// One unit of work of the tcgen05 SYRK kernel: output tile rows [col_a, col_a+128), columns
-// [col_b, col_b+128*w) of G, accumulated over row chunks [k0, k1) of X (chunk = BK rows).
-struct SyrkSeg {
-  int32_t col_a, col_b, w, k0, k1;
-};
-
-// Rows of X are processed in panels small enough to stay in L2 while every tile re-reads them: one chunk
-// (BK rows) of all d columns is always d * 128 bytes, and a panel is ~40 MB of X (VLM_SYRK_PANEL_MB), at
-// least 32 chunks.  VLM_SYRK_PANEL_CHUNKS overrides the result (experiments).
-inline int64_t syrk_panel_chunks(int d) {
-  if (const char* e = getenv("VLM_SYRK_PANEL_CHUNKS")) return std::max(1, atoi(e));
-  double mb = 40.0;
-  if (const char* e = getenv("VLM_SYRK_PANEL_MB")) mb = std::max(1.0, atof(e));
-  return std::max<int64_t>(32, (int64_t)(mb * 1e6 / (128.0 * d)));
-}
-
-void build_syrk_schedule(int64_t kc, int d, int nsm, std::vector<SyrkSeg>* segs, std::vector<int>* off);
-
-int syrk_tc_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
-                   cudaStream_t stream);
 // One unit of work of a CLUSTER (CTA-pair kernels): super-tile (sa, sb) in 256-column units, row chunks [k0, k1).
 struct PairSeg {
   int32_t sa, sb, k0, k1;
@@ -46,9 +24,10 @@ int syrk_i8x4_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
 
 void build_syrk_i8_schedule_host(int64_t kc, int d, int nsm, std::vector<int32_t>* flat, std::vector<int>* off);
 
-// CTA-pair kernel (syrk_pair.cu + syrk_2sm.cuh: one tcgen05.mma.cta_group::2 stream per pair); needs whole 128-byte
-// column groups
-bool syrk_pair_supported(int dtype, int d, int64_t ldx);
+// CTA-pair kernel (syrk_pair.cu + syrk_2sm.cuh: one tcgen05.mma.cta_group::2 stream per pair).  The one statement of
+// what it takes: whole 128-byte column groups, x and g 16-byte aligned, row pitch and segment stride multiples of
+// 16 bytes, ldg % 4 == 0.  Every other Gram goes to the CUDA-core kernel (syrk_simt_launch).
+bool syrk_pair_supported(int dtype, const void* x, int d, int64_t ldx, int64_t seg_stride, const float* g, int64_t ldg);
 // seg_rows > 0: X is rows/seg_rows row segments of seg_rows rows, seg_stride elements apart (0: contiguous rows)
 int syrk_pair_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows, int64_t seg_stride,
                     float* g, int64_t ldg, cudaStream_t stream);

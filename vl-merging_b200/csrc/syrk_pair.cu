@@ -6,10 +6,11 @@
 // (its 128 rows of A and of the accumulator) and column block 2b+r (its half of B).  X is described to TMA as a 3-D
 // tensor {column in group, row, column group} (strides: element, row pitch, 128 B), so ONE cp.async.bulk.tensor box
 // {128 B, BK rows, groups per block} fetches a whole 128-column block in exactly the [group][row][128 B] order of
-// the canonical MN-major UMMA layout: 2 TMA instructions and 32 KB per CTA per stage.  History (DESIGN.md 4a): a
-// single-CTA kernel (syrk_tc.cu, still the path for widths that are not whole 128-byte column groups), then CTA
-// pairs with two cta_group::1 streams and TMA multicast (48 KB taken in per SM per stage: ingest-bound at 84 % tensor
-// pipe), then this one (93 %).
+// the canonical MN-major UMMA layout: 2 TMA instructions and 32 KB per CTA per stage.  Widths that are not whole
+// 128-byte column groups, and operands TMA cannot address, run on the CUDA-core kernel instead (syrk_simt.cu; the
+// condition is syrk_pair_supported).  History (DESIGN.md 4a): a single-CTA kernel (removed), then CTA pairs with two
+// cta_group::1 streams and TMA multicast (48 KB taken in per SM per stage: ingest-bound at 84 % tensor pipe), then
+// this one (93 %).
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
@@ -87,26 +88,41 @@ struct DeviceSchedule2 {
   int* d_off = nullptr;
 };
 std::mutex g_mu2;
-std::map<std::tuple<int, int64_t, int, int, int>, DeviceSchedule2> g_sched2;
+typedef std::tuple<int, int64_t, int, int, int> ScheduleKey;  // (device, chunks, d, chunk rows or -8 for int8, SMs)
+std::map<ScheduleKey, DeviceSchedule2> g_sched2;
 // schedules evicted from the cache: freed at the NEXT eviction, after a device synchronisation, never while a
 // launch that was handed their pointers may still be pending (the lock is held from lookup to launch)
 std::vector<DeviceSchedule2> g_retired2;
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn g_encode2 = nullptr;
-
-int ensure_encode() {
-  std::lock_guard<std::mutex> lk(g_mu2);
-  if (!g_encode2) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    VLM_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-    VLM_REQUIRE(fn != nullptr && qres == cudaDriverEntryPointSuccess, VLM_ERR_DRIVER,
-                "cuTensorMapEncodeTiled not available from the driver");
-    g_encode2 = reinterpret_cast<EncodeTiledFn>(fn);
+// The device copy of the schedule `build` makes for `key`, built and uploaded on first use.  Call with g_mu2 held
+// until the launch that reads it is enqueued.
+template <typename Build>
+int cached_schedule(const ScheduleKey& key, Build build, cudaStream_t stream, const DeviceSchedule2** out) {
+  auto it = g_sched2.find(key);
+  if (it == g_sched2.end()) {
+    if (g_sched2.size() >= 512) {  // ragged workloads (a new row count every call): start over, do not grow forever
+      VLM_CUDA(cudaDeviceSynchronize());  // launches that read the schedules retired LAST time have finished
+      for (auto& ds : g_retired2) {
+        cudaFree(ds.d_segs);
+        cudaFree(ds.d_off);
+      }
+      g_retired2.clear();
+      for (auto& kv : g_sched2) g_retired2.push_back(kv.second);
+      g_sched2.clear();
+    }
+    std::vector<PairSeg> segs;
+    std::vector<int> off;
+    build(&segs, &off);
+    DeviceSchedule2 ds;
+    ds.nclusters = (int)off.size() - 1;
+    VLM_CUDA(cudaMalloc(&ds.d_segs, std::max<size_t>(1, segs.size()) * sizeof(PairSeg)));
+    VLM_CUDA(cudaMalloc(&ds.d_off, off.size() * sizeof(int)));
+    VLM_CUDA(cudaMemcpyAsync(ds.d_segs, segs.data(), segs.size() * sizeof(PairSeg), cudaMemcpyHostToDevice, stream));
+    VLM_CUDA(cudaMemcpyAsync(ds.d_off, off.data(), off.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
+    VLM_CUDA(cudaStreamSynchronize(stream));
+    it = g_sched2.emplace(key, ds).first;
   }
+  *out = &it->second;
   return 0;
 }
 
@@ -118,8 +134,8 @@ inline int chunk_rows(int dtype) { return dtype == VLM_TF32X2 ? 16 : 128 / elem_
 // seg_rows > 0: 4-D, {column in group, row in segment, column group, segment}.
 // VLM_TF32X2: 4-D, {column in group, row, column group, plane}, planes rows * ldx elements apart, and one box
 // fetches both planes of a 128-column block for 16 rows.
-int encode_maps(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows, int64_t seg_stride,
-                float* g, int64_t ldg, CUtensorMap* tm_x, CUtensorMap* tm_g) {
+int encode_maps(EncodeTiledFn encode, const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows,
+                int64_t seg_stride, float* g, int64_t ldg, CUtensorMap* tm_x, CUtensorMap* tm_g) {
   const int elem = elem_bytes(dtype);
   const int bk = chunk_rows(dtype), gc = 128 / elem;
   {
@@ -141,8 +157,8 @@ int encode_maps(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int6
                          (cuuint32_t)(split ? 2 : 1)};
     cuuint32_t estr[4] = {1, 1, 1, 1};
     const CUtensorMapSwizzle swz = elem == 4 ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B;
-    CUresult r = g_encode2(tm_x, dt, rank, const_cast<void*>(x), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = encode(tm_x, dt, rank, const_cast<void*>(x), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     VLM_REQUIRE(r == CUDA_SUCCESS, VLM_ERR_DRIVER, "cuTensorMapEncodeTiled(X, %d-D) failed: CUresult %d", rank, (int)r);
   }
   {
@@ -150,20 +166,10 @@ int encode_maps(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int6
     cuuint64_t gstr[1] = {(cuuint64_t)ldg * 4};
     cuuint32_t box[2] = {32, 128};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = g_encode2(tm_g, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, g, gdim, gstr, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = encode(tm_g, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, g, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     VLM_REQUIRE(r == CUDA_SUCCESS, VLM_ERR_DRIVER, "cuTensorMapEncodeTiled(G) failed: CUresult %d", (int)r);
   }
-  return 0;
-}
-
-int check_alignment(const void* x, int elem, int64_t rows, int64_t ldx, const float* g, int64_t ldg) {
-  VLM_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && ((ldx * elem) & 15) == 0, VLM_ERR_ALIGNMENT,
-              "vlm_syrk_accum: x must be 16-byte aligned with a row pitch that is a multiple of 16 bytes");
-  VLM_REQUIRE((reinterpret_cast<uintptr_t>(g) & 15) == 0 && (ldg & 3) == 0, VLM_ERR_ALIGNMENT,
-              "vlm_syrk_accum: g must be 16-byte aligned with ldg %% 4 == 0");
-  VLM_REQUIRE(rows < (int64_t)1 << 31, VLM_ERR_INVALID_ARG, "vlm_syrk_accum: rows too large");
   return 0;
 }
 
@@ -336,8 +342,11 @@ void build_syrk_i8_schedule_host(int64_t kc, int d, int nsm, std::vector<int32_t
   }
 }
 
-bool syrk_pair_supported(int dtype, int d, int64_t ldx) {
-  return d % (128 / elem_bytes(dtype)) == 0 && ldx >= d;  // whole 128-byte column groups (the 3-D tensor map needs them)
+bool syrk_pair_supported(int dtype, const void* x, int d, int64_t ldx, int64_t seg_stride, const float* g, int64_t ldg) {
+  const int elem = elem_bytes(dtype);
+  return d % (128 / elem) == 0 &&  // whole 128-byte column groups (the 3-D tensor map needs them)
+         (reinterpret_cast<uintptr_t>(x) & 15) == 0 && ((ldx * elem) & 15) == 0 && ((seg_stride * elem) & 15) == 0 &&
+         (reinterpret_cast<uintptr_t>(g) & 15) == 0 && (ldg & 3) == 0;
 }
 
 // chunks per row segment (0 = contiguous) and in total
@@ -353,53 +362,34 @@ static inline void seg_chunks(int64_t rows, int64_t seg_rows, int bk, int64_t* c
 
 int syrk_pair_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows, int64_t seg_stride,
                     float* g, int64_t ldg, cudaStream_t stream) {
-  const int elem = elem_bytes(dtype);
   const int bk = chunk_rows(dtype);
-  if (int rc = check_alignment(x, elem, rows, ldx, g, ldg)) return rc;
+  VLM_REQUIRE(rows < (int64_t)1 << 31, VLM_ERR_INVALID_ARG, "vlm_syrk_accum: rows too large");
   if (seg_rows >= rows || dtype == VLM_TF32X2) seg_rows = 0;  // one segment: plain rows
   int dev = 0, nsm = 0;
   VLM_CUDA(cudaGetDevice(&dev));
   if (int rc = device_sm_count(&nsm)) return rc;
-  if (int rc = ensure_encode()) return rc;
+  EncodeTiledFn encode = nullptr;
+  if (int rc = tensor_map_encoder(&encode)) return rc;
   int64_t cps, kc;
   seg_chunks(rows, seg_rows, bk, &cps, &kc);
   VLM_REQUIRE(kc < (int64_t)1 << 30, VLM_ERR_INVALID_ARG, "vlm_syrk_accum: too many row chunks");
   CUtensorMap tm_x, tm_g;
-  if (int rc = encode_maps(x, dtype, rows, d, ldx, seg_rows, seg_stride, g, ldg, &tm_x, &tm_g)) return rc;
+  if (int rc = encode_maps(encode, x, dtype, rows, d, ldx, seg_rows, seg_stride, g, ldg, &tm_x, &tm_g)) return rc;
   const int smem = k2SmemBytes;
   PairKernel kernel = pick_kernel<false>(dtype);
 
   // lookup and launch under one lock: an eviction by another host thread cannot free a schedule between the two
   std::lock_guard<std::mutex> lk(g_mu2);
-  auto key = std::make_tuple(dev, kc, d, bk, nsm);
-  auto it = g_sched2.find(key);
-  if (it == g_sched2.end()) {
-    if (g_sched2.size() >= 512) {  // ragged workloads (a new row count every call): start over, do not grow forever
-      VLM_CUDA(cudaDeviceSynchronize());  // launches that read the schedules retired LAST time have finished
-      for (auto& ds : g_retired2) {
-        cudaFree(ds.d_segs);
-        cudaFree(ds.d_off);
-      }
-      g_retired2.clear();
-      for (auto& kv : g_sched2) g_retired2.push_back(kv.second);
-      g_sched2.clear();
-    }
-    std::vector<PairSeg> segs;
-    std::vector<int> off;
-    build_pair_schedule(kc, d, nsm / 2, &segs, &off);
-    DeviceSchedule2 ds;
-    ds.nclusters = (int)off.size() - 1;
-    VLM_CUDA(cudaMalloc(&ds.d_segs, std::max<size_t>(1, segs.size()) * sizeof(PairSeg)));
-    VLM_CUDA(cudaMalloc(&ds.d_off, off.size() * sizeof(int)));
-    VLM_CUDA(cudaMemcpyAsync(ds.d_segs, segs.data(), segs.size() * sizeof(PairSeg), cudaMemcpyHostToDevice, stream));
-    VLM_CUDA(cudaMemcpyAsync(ds.d_off, off.data(), off.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
-    VLM_CUDA(cudaStreamSynchronize(stream));
-    it = g_sched2.emplace(key, ds).first;
-  }
-  const DeviceSchedule2& sched = it->second;
+  const DeviceSchedule2* sched = nullptr;
+  if (int rc = cached_schedule(std::make_tuple(dev, kc, d, bk, nsm),
+                               [&](std::vector<PairSeg>* segs, std::vector<int>* off) {
+                                 build_pair_schedule(kc, d, nsm / 2, segs, off);
+                               },
+                               stream, &sched))
+    return rc;
   VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  kernel<<<2 * sched.nclusters, kThreads, smem, stream>>>(tm_x, tm_g, nullptr, sched.d_segs, sched.d_off, d, (int)cps,
-                                                          l2_hints());
+  kernel<<<2 * sched->nclusters, kThreads, smem, stream>>>(tm_x, tm_g, nullptr, sched->d_segs, sched->d_off, d, (int)cps,
+                                                           l2_hints());
   VLM_CUDA(cudaGetLastError());
   count_launch();
   return 0;
@@ -499,7 +489,8 @@ int syrk_i8x4_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
   int dev = 0, nsm = 0;
   VLM_CUDA(cudaGetDevice(&dev));
   if (int rc = device_sm_count(&nsm)) return rc;
-  if (int rc = ensure_encode()) return rc;
+  EncodeTiledFn encode = nullptr;
+  if (int rc = tensor_map_encoder(&encode)) return rc;
   if (seg_rows >= rows) seg_rows = 0;
   int8_t* planes = static_cast<int8_t*>(scratch);
   int* exps = reinterpret_cast<int*>(planes + (((size_t)4 * rows * d + 15) & ~(size_t)15));
@@ -522,9 +513,9 @@ int syrk_i8x4_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
     cuuint64_t gstr[3] = {(cuuint64_t)d, 128, (cuuint64_t)rows * d};
     cuuint32_t box[4] = {128, (cuuint32_t)(ph == 2 ? 128 : 32), 1, np};
     cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = g_encode2(&tm_p[ph], CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, planes, gdim, gstr, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = encode(&tm_p[ph], CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, planes, gdim, gstr, box, estr,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     VLM_REQUIRE(r == CUDA_SUCCESS, VLM_ERR_DRIVER, "cuTensorMapEncodeTiled(int8 planes) failed: CUresult %d", (int)r);
   }
   // G as a 2-D fp64 tensor for the epilogue's TMA reduce-adds: box = 16 columns (128 bytes) x 128 rows
@@ -534,46 +525,37 @@ int syrk_i8x4_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
     cuuint64_t gstr[1] = {(cuuint64_t)ldg * 8};
     cuuint32_t box[2] = {16, 128};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = g_encode2(&tm_g, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, g, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = encode(&tm_g, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, g, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     VLM_REQUIRE(r == CUDA_SUCCESS, VLM_ERR_DRIVER, "cuTensorMapEncodeTiled(G fp64) failed: CUresult %d", (int)r);
   }
   const int64_t kc = (rows + 31) / 32;
   VLM_REQUIRE(kc < (int64_t)1 << 30, VLM_ERR_INVALID_ARG, "vlm_syrk_accum_i8x4: too many row chunks");
   std::lock_guard<std::mutex> lk(g_mu2);
-  auto key = std::make_tuple(dev, kc, d, -8, nsm);   // bk = -8: the int8 schedule
-  auto it = g_sched2.find(key);
-  if (it == g_sched2.end()) {
-    std::vector<PairSeg> segs;
-    std::vector<int> off;
-    build_i8_schedule(kc, d, nsm / 2, &segs, &off);
-    DeviceSchedule2 ds;
-    ds.nclusters = (int)off.size() - 1;
-    VLM_CUDA(cudaMalloc(&ds.d_segs, std::max<size_t>(1, segs.size()) * sizeof(PairSeg)));
-    VLM_CUDA(cudaMalloc(&ds.d_off, off.size() * sizeof(int)));
-    VLM_CUDA(cudaMemcpyAsync(ds.d_segs, segs.data(), segs.size() * sizeof(PairSeg), cudaMemcpyHostToDevice, stream));
-    VLM_CUDA(cudaMemcpyAsync(ds.d_off, off.data(), off.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
-    VLM_CUDA(cudaStreamSynchronize(stream));
-    it = g_sched2.emplace(key, ds).first;
-  }
-  const DeviceSchedule2& sched = it->second;
+  const DeviceSchedule2* sched = nullptr;
+  if (int rc = cached_schedule(std::make_tuple(dev, kc, d, -8, nsm),  // chunk rows -8: the int8 schedule
+                               [&](std::vector<PairSeg>* segs, std::vector<int>* off) {
+                                 build_i8_schedule(kc, d, nsm / 2, segs, off);
+                               },
+                               stream, &sched))
+    return rc;
   const int smem = kI8SmemBytes;
   VLM_CUDA(cudaFuncSetAttribute(syrk_i8x4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   I8Args args{g, ldg, exps};
-  syrk_i8x4_kernel<<<2 * sched.nclusters, kThreads, smem, stream>>>(tm_p[0], tm_p[1], tm_p[2], tm_g, sched.d_segs, sched.d_off,
-                                                                    d, args);
+  syrk_i8x4_kernel<<<2 * sched->nclusters, kThreads, smem, stream>>>(tm_p[0], tm_p[1], tm_p[2], tm_g, sched->d_segs,
+                                                                     sched->d_off, d, args);
   VLM_CUDA(cudaGetLastError());
   count_launch();
   return 0;
 }
 
 int syrk_pair_batch_launch(const vlm_syrk_problem* probs, int n, int dtype, cudaStream_t stream) {
-  const int elem = elem_bytes(dtype);
   const int bk = chunk_rows(dtype);
   int dev = 0, nsm = 0;
   VLM_CUDA(cudaGetDevice(&dev));
   if (int rc = device_sm_count(&nsm)) return rc;
-  if (int rc = ensure_encode()) return rc;
+  EncodeTiledFn encode = nullptr;
+  if (int rc = tensor_map_encoder(&encode)) return rc;
   const int C = nsm / 2;
   std::vector<CUtensorMap> maps(2 * (size_t)n);
   std::vector<std::vector<BatchSeg>> per(C);
@@ -597,9 +579,9 @@ int syrk_pair_batch_launch(const vlm_syrk_problem* probs, int n, int dtype, cuda
   const int64_t min_piece = batch_work >= (int64_t)8 * 64 * C ? 64 : 0;
   for (int p = 0; p < n; ++p) {
     const vlm_syrk_problem& q = probs[p];
-    if (int rc = check_alignment(q.x, elem, q.rows, q.ldx, q.g, q.ldg)) return rc;
+    VLM_REQUIRE(q.rows < (int64_t)1 << 31, VLM_ERR_INVALID_ARG, "vlm_syrk_accum: rows too large");
     const int64_t seg_rows = (dtype != VLM_TF32X2 && q.seg_rows > 0 && q.seg_rows < q.rows) ? q.seg_rows : 0;
-    if (int rc = encode_maps(q.x, dtype, q.rows, q.d, q.ldx, seg_rows, q.seg_stride, q.g, q.ldg, &maps[2 * p],
+    if (int rc = encode_maps(encode, q.x, dtype, q.rows, q.d, q.ldx, seg_rows, q.seg_stride, q.g, q.ldg, &maps[2 * p],
                              &maps[2 * p + 1]))
       return rc;
     int64_t cps, kc;

@@ -1,46 +1,10 @@
-// umma.cuh — tile geometry and tcgen05 descriptor helpers shared by the SYRK kernels.
+// umma.cuh — tile geometry and the single-CTA tcgen05.mma wrapper shared by the tensor-core kernels.
 #pragma once
 #include "common.cuh"
 
 namespace vlm {
 
 constexpr int kBlockBytes = 16384;  // one 128-column block of X for one pipeline stage
-
-template <int ELEM_BYTES>
-struct Geo {
-  static constexpr int GC = 128 / ELEM_BYTES;       // columns per 128-byte group (TMA box width)
-  static constexpr int GB = ELEM_BYTES;             // groups per 128-column block
-  static constexpr int BK = 128 / ELEM_BYTES;       // rows per stage: 32 (fp32) / 64 (16-bit)
-  static constexpr int BOX_BYTES = BK * 128;        // one TMA box
-  static constexpr int UMMA_K = 32 / ELEM_BYTES;    // rows per tcgen05.mma: 8 (tf32) / 16 (f16)
-  static constexpr int KSTEP_BYTES = UMMA_K * 128;  // smem advance per MMA
-  static constexpr int NUM_MMA = BK / UMMA_K;       // 4
-  // rows per swizzle atom: 8 (SWIZZLE_128B) for 16-bit operands, 4 (SWIZZLE_128B_BASE32B) for TF32
-  static constexpr int LAYOUT_TYPE = ELEM_BYTES == 4 ? 1 : 2;
-  static constexpr int SBO_BYTES = ELEM_BYTES == 4 ? 512 : 1024;
-  static_assert(GB * BOX_BYTES == kBlockBytes, "block geometry");
-};
-
-// UMMA shared-memory descriptor for the MN-major canonical layouts (see header comment).
-// layout_type 2 = SWIZZLE_128B (16-byte chunks XOR row%8, 8-row atoms: bf16/f16),
-// layout_type 1 = SWIZZLE_128B_BASE32B (32-byte chunks XOR row%4, 4-row atoms): the only swizzled
-// layout tcgen05 accepts for MN-major TF32 operands; its TMA twin is SWIZZLE_128B_ATOM_32B.
-template <int LAYOUT_TYPE>
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);             // start address      bits [0,14)
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16;    // leading byte off.  bits [16,30)
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32;    // stride byte off.   bits [32,46)
-  d |= (uint64_t)1 << 46;                               // descriptor version (Blackwell) bits [46,48)
-  d |= (uint64_t)LAYOUT_TYPE << 61;                     // layout type        bits [61,64)
-  return d;
-}
-
-// tcgen05 instruction descriptor: D fp32, A/B format fmt (0 f16, 1 bf16, 2 tf32), both MN-major, M=128.
-__host__ __device__ constexpr uint32_t make_idesc(int fmt, int n) {
-  return (1u << 4) | ((uint32_t)fmt << 7) | ((uint32_t)fmt << 10) | (1u << 15) | (1u << 16) |
-         ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
 
 template <int FMT>
 __device__ __forceinline__ void umma(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,

@@ -181,7 +181,7 @@ class GramCache:
         self.dtype = torch.float64 if precision in ("fp64", "int8x4") else torch.float32   # of the Gram buffers
         self._sym_code = _lib.VLM_F64 if self.dtype == torch.float64 else _lib.VLM_F32    # vlm_sym_* dtype of the buffers
         self._planes = None    # scratch for the {hi, lo} planes of the split mode (grown on demand, reused in stream order)
-        self._fn = self._lib.vlm_syrk_accum_simt if use_simt else self._lib.vlm_syrk_accum
+        self._use_simt = bool(use_simt)   # every fp32-Gram launch on the CUDA-core kernel (device-side oracle)
         self.buffers = {}       # name -> fp32 [d, d] (upper triangle authoritative until finalize())
         self._arenas = []      # flat fp32 arenas the registered buffers are views of
         self.calls = defaultdict(int)
@@ -232,9 +232,12 @@ class GramCache:
                 x2 = x2.contiguous()
             rows, ldx, keep = x2.shape[0], (x2.stride(0) if x2.shape[0] > 1 else d), x2
         ptr = keep.data_ptr()
-        simt = self._fn is self._lib.vlm_syrk_accum_simt or (ptr % 16) or ((ldx * elem) % 16)
-        if self.precision == "tf32x3" and keep.dtype == torch.float32 and d % 32:
-            simt = True                  # widths the split kernel does not take: CUDA cores, exact fp32 products
+        # tf32x3 splits fp32 activations that vlm_tf32_split and the split kernel take (d % 32 == 0, 16-byte aligned x,
+        # ldx and seg_stride multiples of 4); any other one goes to the CUDA-core kernel (exact fp32 products) at once:
+        # it must not join a deferred group, which flush() issues as split planes
+        split = self.precision == "tf32x3" and keep.dtype == torch.float32
+        simt = self._use_simt or (split and bool(d % 32 or ptr % 16 or ldx % 4 or seg_stride % 4))
+        split = split and not simt
         if simt and seg_rows:
             keep = x.contiguous()        # the CUDA-core kernel takes plain rows only
             ptr, ldx, seg_rows, seg_stride = keep.data_ptr(), d, 0, 0
@@ -266,7 +269,7 @@ class GramCache:
                 self.flush()
             return
         stream = self._launch_stream(keep)
-        if self._split_ok(code, simt, d):
+        if split:
             planes = self._plane_scratch(2 * rows * d)
             _lib.check(self._lib.vlm_tf32_split(ptr, rows, d, ldx, seg_rows, seg_stride, planes.data_ptr(), stream))
             _lib.check(self._lib.vlm_syrk_accum(planes.data_ptr(), _lib.VLM_TF32X2, rows, d, d, g.data_ptr(),
@@ -275,11 +278,8 @@ class GramCache:
             _lib.check(self._lib.vlm_syrk_accum_strided(ptr, code, rows, d, ldx, seg_rows, seg_stride, g.data_ptr(),
                                                         g.stride(0), stream))
         else:
-            fn = self._lib.vlm_syrk_accum_simt if simt else self._fn
+            fn = self._lib.vlm_syrk_accum_simt if simt else self._lib.vlm_syrk_accum
             _lib.check(fn(ptr, code, rows, d, ldx, g.data_ptr(), g.stride(0), stream))
-
-    def _split_ok(self, code, simt, d):
-        return self.precision == "tf32x3" and code == _lib.VLM_F32 and not simt and d % 32 == 0
 
     def _plane_scratch(self, numel):
         """fp32 scratch of at least `numel` elements for the {hi, lo} planes.  One buffer, reused by every launch:
@@ -331,12 +331,14 @@ class GramCache:
         for code in sorted({p[0] for p in pending}):
             group = [p for p in pending if p[0] == code]
             probs = (_lib.SyrkProblem * len(group))()
-            split = [self._split_ok(code, False, p[5]) for p in group]
-            if any(split):      # split mode: the planes of every problem of the group, back to back in the scratch
-                planes = self._plane_scratch(sum(2 * p[4] * p[5] for p, s in zip(group, split) if s))
+            # split mode: accumulate() defers only fp32 activations the split takes, so all of this group is split; the
+            # planes of every problem, back to back in the scratch
+            split = self.precision == "tf32x3" and code == _lib.VLM_F32
+            if split:
+                planes = self._plane_scratch(sum(2 * p[4] * p[5] for p in group))
                 off = 0
-            for q, (_, _keep, g, ptr, rows, d, ldx, seg_rows, seg_stride), sp in zip(probs, group, split):
-                if sp:
+            for q, (_, _keep, g, ptr, rows, d, ldx, seg_rows, seg_stride) in zip(probs, group):
+                if split:
                     dst = planes.data_ptr() + off * 4
                     _lib.check(self._lib.vlm_tf32_split(ptr, rows, d, ldx, seg_rows, seg_stride, dst, stream))
                     off += 2 * rows * d
@@ -344,8 +346,7 @@ class GramCache:
                 else:
                     q.x, q.rows, q.ldx, q.g, q.ldg, q.d = ptr, rows, ldx, g.data_ptr(), g.stride(0), d
                     q.seg_rows, q.seg_stride = seg_rows, seg_stride
-            _lib.check(self._lib.vlm_syrk_accum_batch(probs, len(group), _lib.VLM_TF32X2 if any(split) else code,
-                                                      stream))
+            _lib.check(self._lib.vlm_syrk_accum_batch(probs, len(group), _lib.VLM_TF32X2 if split else code, stream))
         self._join()
         # `pending` (and with it the activations) is released here: the launches are already ordered on the stream
 
