@@ -84,13 +84,17 @@ int vlm_tf32_split(const float* x, int64_t rows, int d, int64_t ldx, int64_t seg
 int vlm_syrk_accum_f64(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows,
                        int64_t seg_stride, double* g, int64_t ldg, void* stream);
 
-/* The same Gram, exact, on the INTEGER tensor cores: each column is scaled by a power of two above its maximum in
- * this call and every value becomes four balanced int8 digits (q = rint(x * 2^(26-E_c)) = sum D_p * 128^(3-p));
+/* The same Gram, exact, on the INTEGER tensor cores: column c is scaled by 2^(26-E_c), 2^E_c the power of two just
+ * above its maximum in this call (2^(E_c-1) <= max < 2^E_c; E_c = 0 for a zero column), and every value becomes four
+ * balanced int8 digits (q = rint(x * 2^(26-E_c)) = sum D_p * 128^(3-p));
  * the thirteen digit-plane products with p + q <= 4 run as tcgen05.mma kind::i8 (int32 accumulation: exact) and are
- * added to the fp64 Gram with their power-of-two scales (fp64 TMA reduce-adds).  Error: 2^-27 of the column maximum
- * per element (unbiased quantisation) + the dropped products (< 1e-9 of sqrt(G_ii G_jj)) — measured 1e-10 on normal
- * data, 3e-9 on LayerNorm outputs: RegMean-grade — at about 3.5x the cost of the single TF32 pass instead of the fp64
- * path's 28x.  x: VLM_F32 / VLM_F16 / VLM_BF16 (16-bit values are widened exactly), 16-byte aligned, ldx % 4 == 0,
+ * added to the fp64 Gram with their power-of-two scales (fp64 TMA reduce-adds).  Error: at most 2^(E_c-27) per
+ * element, i.e. 2^-27 to 2^-26 of the column maximum (unbiased quantisation) + the dropped products (< 1e-9 of
+ * sqrt(G_ii G_jj)) — measured 1e-10 on normal data, 3e-9 on LayerNorm outputs: RegMean-grade — at about 3.5x the cost
+ * of the single TF32 pass instead of the fp64 path's 28x.  E_c is clamped below at -100 so that the float scale
+ * 2^(26-E_c) stays finite: a column whose maximum is below 2^-101 is quantised with the fixed step 2^-126, an error of
+ * up to 2^-127 per element, which is 2^-127 / max of the column maximum (2^-17 for a maximum of 2^-110) instead of
+ * 2^-27.  x: VLM_F32 / VLM_F16 / VLM_BF16 (16-bit values are widened exactly), 16-byte aligned, ldx % 4 == 0,
  * optionally row-segmented; d % 128 == 0 (VLM_ERR_UNSUPPORTED otherwise: use vlm_syrk_accum_f64); scratch:
  * vlm_syrk_i8x4_scratch_bytes(rows, d) bytes of device memory, 16-byte aligned, borrowed for the call.  G as for
  * vlm_syrk_accum_f64, 16-byte aligned with an even ldg (TMA). */

@@ -246,7 +246,8 @@ def test_deferred_activation_modified_in_place_is_refused():
 @pytest.mark.parametrize("precision", ["tf32x3", "fp64", "int8x4"])
 def test_precision_modes_match_the_fp64_hook(precision):
     """The RegMean-grade Gram modes on the shapes of the hook path: 3-D inputs, a row slice of a (B, N, D) activation,
-    bf16 inputs, an odd width (tf32x3: CUDA-core fallback; fp64: scalar-load path), immediate and grouped."""
+    bf16 inputs, an odd width (tf32x3: CUDA-core fallback; fp64: partial 128-column tiles, still on the cp.async path
+    since 200 fp32 columns make 16-byte rows), immediate and grouped."""
     gen = torch.Generator(device="cuda").manual_seed(4)
     joint = torch.randn(6, 617, 256, device="cuda", generator=gen)
     joint64 = torch.randn(64, 617, 256, device="cuda", generator=gen) - 0.3     # big enough for the int8 path

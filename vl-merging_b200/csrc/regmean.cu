@@ -340,6 +340,23 @@ __global__ void __launch_bounds__(256) widen_add_kernel(const float* __restrict_
     dst[r * ldd + c] = __dadd_rn(dst[r * ldd + c], (double)src[r * lds + c]);
   }
 }
+
+// potrf's status word can miss a pivot that is not positive: a 768 x 768 diagonal matrix whose last entry is -1
+// factors with status 0 and a NaN at the end of the diagonal (B200, cuSOLVER of CUDA 12.8).  Every diagonal entry of
+// a Cholesky factor is finite and positive, so the factor itself says whether potrf succeeded: if the status is 0
+// and an entry is not, report the first such pivot (1-based, as potrf does).  One block, stream-ordered.
+__global__ void __launch_bounds__(256) potrf_status_kernel(const double* __restrict__ l, int n, int64_t ld,
+                                                           int* __restrict__ info) {
+  __shared__ int first;
+  if (threadIdx.x == 0) first = n;
+  __syncthreads();
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const double v = l[(int64_t)i * ld + i];
+    if (!(v > 0.0 && isfinite(v))) atomicMin(&first, i);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0 && *info == 0 && first < n) *info = first + 1;
+}
 }  // namespace
 }  // namespace vlm
 
@@ -426,8 +443,10 @@ int enqueue_spd_solve(double* s, int in_f, int64_t lds, double* r, int out_f, in
               "cusolverDnDpotrf_bufferSize failed");
   if (int rc = solve_ctx(st, (size_t)std::max(lwork, 1), &c)) return rc;
   cusolverStatus_t cs1 = g_cs.potrf(c.h, uplo_lower, in_f, s, (int)lds, c.work, lwork, info_dev);
+  potrf_status_kernel<<<1, 256, 0, st>>>(s, in_f, lds, info_dev);
+  VLM_CUDA(cudaGetLastError());
   cusolverStatus_t cs2 = g_cs.potrs(c.h, uplo_lower, in_f, out_f, s, (int)lds, r, (int)ldr, info_dev + 1);
-  count_launch(2);
+  count_launch(3);
   VLM_REQUIRE(cs1 == 0 && cs2 == 0, VLM_ERR_INTERNAL, "cuSOLVER potrf/potrs status %d/%d", cs1, cs2);
   return 0;
 }
