@@ -34,28 +34,30 @@ def _oracle_gram(x):
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16, torch.float16])
 @pytest.mark.parametrize("d", [768, 192, 200, 1024])
 def test_row_slices_are_read_in_place(dtype, d):
-    """Text slice [0, 40) and image slice [40, N) of a (B, N, D) activation: vs the fp64 oracle on the slice, and
-    vs the same kernel on a contiguous copy.  d = 200 has no whole 128-byte column groups (CUDA-core kernel,
-    one launch per segment)."""
+    """Text slice [0, 40) and image slice [40, N) of a (B, N, D) activation, for 224- and 384-pixel images: vs the
+    fp64 oracle on the slice, and vs the same kernel on a contiguous copy.  d = 200 has no whole 128-byte column
+    groups (CUDA-core kernel, one launch per segment)."""
     torch.manual_seed(d)
-    h = torch.randn(6, 40 + 197, d, device="cuda").to(dtype)
-    for lo, hi in ((0, 40), (40, 237), (3, 4), (3, 8)):       # (3, 8): 5-row segments, shorter than one K chunk
-        x = h[:, lo:hi]
-        assert not x.is_contiguous()
-        cache = vlm.GramCache()
-        before = vlm._lib.launch_count()
-        cache.accumulate("s", x)
-        cache.accumulate("s", x)
-        launches = vlm._lib.launch_count() - before
-        cache.accumulate("c", x.contiguous())
-        cache.accumulate("c", x.contiguous())
-        sd = cache.state_dict()
-        want = 2 * _oracle_gram(x)
-        assert _rel(sd["s"].numpy(), want) < 1e-3
-        assert _rel(sd["s"].numpy(), sd["c"].numpy()) < 2e-4
-        if d != 200:
-            assert launches == 2          # one launch per call: no copy kernel, no per-segment launches
-        assert cache.rows["s"] == 2 * 6 * (hi - lo)
+    tol = 1e-3 if dtype == torch.float32 else 1e-5      # 16-bit products are exact: only the fp32 accumulation is left
+    for b, n in ((6, 40 + 197), (4, 40 + 577)):
+        h = torch.randn(b, n, d, device="cuda").to(dtype)
+        for lo, hi in ((0, 40), (40, n), (3, 4), (3, 8)):       # (3, 8): 5-row segments, shorter than one K chunk
+            x = h[:, lo:hi]
+            assert not x.is_contiguous()
+            cache = vlm.GramCache()
+            before = vlm._lib.launch_count()
+            cache.accumulate("s", x)
+            cache.accumulate("s", x)
+            launches = vlm._lib.launch_count() - before
+            cache.accumulate("c", x.contiguous())
+            cache.accumulate("c", x.contiguous())
+            sd = cache.state_dict()
+            want = 2 * _oracle_gram(x)
+            assert _rel(sd["s"].numpy(), want) < tol, (b, n, lo, hi)
+            assert _rel(sd["s"].numpy(), sd["c"].numpy()) < 2e-4
+            if d != 200:
+                assert launches == 2          # one launch per call: no copy kernel, no per-segment launches
+            assert cache.rows["s"] == 2 * b * (hi - lo)
 
 
 def test_deferred_row_slices_go_through_the_grouped_launch():
@@ -74,6 +76,21 @@ def test_deferred_row_slices_go_through_the_grouped_launch():
     sd = cache.state_dict()
     for name, x in (("t", h[:, :40]), ("i", h[:, 40:]), ("whole", h), ("wide", h2[:, 40:])):
         assert _rel(sd[name].numpy(), _oracle_gram(x)) < 1e-3, name
+    # at calibration size (64 x 617 tokens): each slice and a packed copy of it in one grouped launch, and the slice
+    # through the immediate launch, against the packed copy's Gram
+    big = torch.randn(64, 617, 768, device="cuda")
+    for lo, hi in ((40, 617), (0, 40)):
+        x = big[:, lo:hi]
+        grouped, now = vlm.GramCache(defer_bytes=1 << 30), vlm.GramCache()
+        grouped.accumulate("s", x)
+        grouped.accumulate("c", x.contiguous())
+        before = vlm._lib.launch_count()
+        grouped.flush()
+        assert vlm._lib.launch_count() == before + 1
+        now.accumulate("s", x)
+        packed = grouped.gram("c").double()
+        for g in (grouped.gram("s"), now.gram("s")):
+            assert ((g.double() - packed).norm() / packed.norm()).item() < 2e-4, (lo, hi)
 
 
 def test_unaligned_or_odd_slices_fall_back_correctly():

@@ -203,6 +203,7 @@ def test_regmean_rhs_matches_fp64_gemm(lib, case, diff, alpha):
         else:
             want, bound = ref, 2 * (in_f + 2) * U * absprod
         _assert_within(acc.m, want, bound, what=f"{case} accumulate={accumulate}")
+        assert ((acc.m - want).norm() / want.norm()).item() < 1e-13   # and as a whole, in the norm regmean sees
         assert acc.sentinels_intact()
     assert w.sentinels_intact() and wb.sentinels_intact() and g.sentinels_intact()
 
@@ -246,7 +247,8 @@ def test_solves_match_fp64_solve(lib, in_f, out_f):
             assert info == [0, 0]
         rel = ((x - ref).norm() / ref.norm()).item()
         resid = ((x @ s_full - r_full).norm() / (x.norm() * s_full.norm())).item()
-        assert rel < 1e-11 and resid < 1e-13, (which, rel, resid)
+        resid_r = ((x @ s_full - r_full).norm() / r_full.norm()).item()
+        assert rel < 1e-11 and resid < 1e-13 and resid_r < 1e-10, (which, rel, resid, resid_r)
 
 
 @pytest.mark.parametrize("in_f,k", [(8, 0), (200, 137), (768, 767)])

@@ -19,7 +19,7 @@ def _feats(m, n, d, dtype, seed):
 
 @pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16], ids=["f16", "bf16"])
 @pytest.mark.parametrize("m,n,d", [(1, 1, 8), (7, 5, 64), (130, 300, 192), (128, 256, 768), (129, 257, 776), (300, 1000, 1024),
-                                   (5000, 700, 768), (40, 9000, 768)])
+                                   (5000, 700, 768), (40, 9000, 768), (5000, 25000, 768)])
 def test_sim_topk_matches_torch(m, n, d, dtype):
     a, b = _feats(m, n, d, dtype, seed=m * 31 + n)
     k = min(10, n)
