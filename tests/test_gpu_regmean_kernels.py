@@ -6,8 +6,9 @@ Frobenius norm, in which an error confined to a partial edge tile, a padded pitc
 vanishes.  Here every entry is checked on its own:
 
 * sentinels: every output (and every input) lives inside a larger allocation whose pad columns (ld > width), guard
-  rows and lead-in elements are NaN.  A stray write shows as a sentinel that is no longer NaN; a stray read of an input
-  shows as a NaN in the result.  Every address stays inside the allocation.
+  rows and lead-in elements are sentinels (sentinel_buffers.py): NaN around inputs, so that a stray read shows as a NaN
+  in the result; a finite value, compared bit for bit, around outputs a kernel adds into, so that a stray write or a
+  stray add shows.  Every address stays inside the allocation.
 * element-wise bounds: a computed sum of n fp64 products, in any order, is within
   2 (n + 2) 2^-53 (|A| @ |B|)_ij of the exact one (the factor 2 also covers the fp64 reference itself).  A dropped,
   doubled or mis-scaled single term is an error of about (|A||B|)_ij / n, far above that.
@@ -17,12 +18,12 @@ vanishes.  Here every entry is checked on its own:
 import pytest
 import torch
 
+from sentinel_buffers import NAN, OUT_SENTINEL, Padded, Segmented
 from vl_merging_b200 import _lib
 
 pytestmark = pytest.mark.gpu
 
 U = 2.0 ** -53
-NAN = float("nan")
 F32, F64, BF16, F16 = torch.float32, torch.float64, torch.bfloat16, torch.float16
 VLM_DTYPE = {F32: _lib.VLM_F32, BF16: _lib.VLM_BF16, F16: _lib.VLM_F16, F64: _lib.VLM_F64}
 SHORT = {F32: "f32", F64: "f64", BF16: "bf16", F16: "f16"}
@@ -41,45 +42,6 @@ def _randn(*shape, seed, dtype=F64):
 def _sym(d, seed, dtype=F64):
     a = _randn(d, d, seed=seed)
     return (a + a.T + 4 * torch.eye(d, dtype=F64, device="cuda")).to(dtype)
-
-
-class Padded:
-    """A rows x cols matrix with row pitch ld inside a NaN-filled allocation: `lead` elements before it, the pad columns
-    cols..ld-1 of every row and `guard` whole rows after it are sentinels.  `m` is the matrix view."""
-
-    def __init__(self, rows, cols, ld, dtype, fill=None, lead=0, guard=2):
-        n = lead + (rows + guard) * ld
-        self.buf = torch.full((n,), NAN, dtype=dtype, device="cuda")
-        self.m = self.buf[lead:lead + rows * ld].view(rows, ld)[:, :cols]
-        if fill is not None:
-            self.m.copy_(fill)
-        self.ld = ld
-        inside = torch.zeros(n, dtype=torch.bool, device="cuda")
-        inside[lead:lead + rows * ld].view(rows, ld)[:, :cols] = True
-        self._outside = ~inside
-
-    @property
-    def ptr(self):
-        return self.m.data_ptr()
-
-    def sentinels_intact(self):
-        return bool(torch.isnan(self.buf[self._outside]).all())
-
-
-class Segmented:
-    """nseg segments of seg_rows rows (row pitch ldx, segment s starting seg_stride elements after segment s - 1) inside
-    a NaN-filled allocation, as vlm_syrk_accum_f64 / _i8x4 read them.  `rows` is the (nseg * seg_rows) x d matrix they
-    describe."""
-
-    def __init__(self, x, seg_rows, ldx, seg_stride, lead=0):
-        rows, d = x.shape
-        nseg = rows // seg_rows
-        assert nseg * seg_rows == rows and seg_stride >= seg_rows * ldx and ldx >= d
-        self.buf = torch.full((lead + nseg * seg_stride + ldx,), NAN, dtype=x.dtype, device="cuda")
-        view = self.buf.as_strided((nseg, seg_rows, d), (seg_stride, ldx, 1), lead)
-        view.copy_(x.view(nseg, seg_rows, d))
-        self.rows = view.reshape(rows, d)
-        self.ptr = view.data_ptr()
 
 
 def _check(rc):
@@ -120,7 +82,7 @@ def scaled_gram(g64, alpha):
 def test_gram_scale_accum_is_bit_exact(lib, gdt, d, alpha, accumulate):
     g = Padded(d, d, d + 3, gdt, fill=_sym(d, seed=d, dtype=gdt))
     out0 = _randn(d, d, seed=d + 1)
-    out = Padded(d, d, d + 5, F64, fill=out0)
+    out = Padded(d, d, d + 5, F64, fill=out0, sentinel=OUT_SENTINEL)
     _check(lib.vlm_gram_scale_accum(g.ptr, VLM_DTYPE[gdt], d, g.ld, alpha, out.ptr, out.ld, accumulate, None))
     ref = scaled_gram(g.m.double(), alpha)
     if accumulate:
@@ -135,7 +97,7 @@ def test_gram_scale_accum_is_bit_exact(lib, gdt, d, alpha, accumulate):
 def test_widen_add_is_bit_exact(lib, rows, cols):
     src = Padded(rows, cols, cols + 3, F32, fill=_randn(rows, cols, seed=rows, dtype=F32))
     dst0 = _randn(rows, cols, seed=cols)
-    dst = Padded(rows, cols, cols + 1, F64, fill=dst0)
+    dst = Padded(rows, cols, cols + 1, F64, fill=dst0, sentinel=OUT_SENTINEL)
     _check(lib.vlm_widen_add(src.ptr, rows, cols, src.ld, dst.ptr, dst.ld, None))
     assert torch.equal(dst.m, dst0 + src.m.double())
     assert dst.sentinels_intact() and src.sentinels_intact()
@@ -188,7 +150,9 @@ def test_regmean_rhs_matches_fp64_gemm(lib, case, diff, alpha):
     acc0 = _randn(out_f, in_f, seed=seed + 3)
     for accumulate in (0, 1):
         # accumulate = 0 must not read acc: start from NaN there; accumulate = 1 adds onto a non-zero acc
-        acc = Padded(out_f, in_f, ldacc, F64, fill=acc0 if accumulate else None, lead=acc_lead)
+        acc = Padded(out_f, in_f, ldacc, F64, fill=acc0 if accumulate else None, lead=acc_lead, sentinel=OUT_SENTINEL)
+        if not accumulate:
+            acc.m.fill_(NAN)
         ptrs = [w.ptr, g.ptr, acc.ptr] + ([wb.ptr] if diff else [])
         assert rhs_kernel_for(in_f, ldw, ldg, gdt, ldacc, ptrs) == case.split("-")[0]
         if diff:
@@ -289,7 +253,7 @@ def _f64_gram_twice(lib, x_ptr, rows, d, ldx, seg_rows, seg_stride, dtype, x64, 
     """Two vlm_syrk_accum_f64 calls on the same X into a G that starts non-zero: upper triangle against
     G0 + 2 X^T X entry by entry, sentinels around G untouched."""
     g0 = _randn(d, d, seed=seed)
-    g = Padded(d, d, d + 3, F64, fill=g0)
+    g = Padded(d, d, d + 3, F64, fill=g0, sentinel=OUT_SENTINEL)
     for _ in range(2):
         _check(lib.vlm_syrk_accum_f64(x_ptr, VLM_DTYPE[dtype], rows, d, ldx, seg_rows, seg_stride, g.ptr, g.ld, None))
     # widened f32 / bf16 / f16 products are exact in fp64: only the 2 rows additions (and the one onto G0) round
@@ -342,7 +306,7 @@ def test_syrk_f64_segmented_rows(lib, path, seg_rows, nseg):
     x = Segmented(_randn(rows, d, seed=seg_rows, dtype=dtype), seg_rows, ldx, seg_stride)
     assert f64_path_for(x.ptr, ldx, seg_stride, d, dtype) == path
     _f64_gram_twice(lib, x.ptr, rows, d, ldx, seg_rows, seg_stride, dtype, x.rows.double(), seed=nseg)
-    assert bool(torch.isnan(x.buf).sum() == x.buf.numel() - rows * d)   # the input itself is untouched
+    assert x.sentinels_intact()   # the input itself is untouched
 
 
 # ---- vlm_syrk_accum_i8x4 -------------------------------------------------------------------------------------------
@@ -381,7 +345,7 @@ def i8_bound(x64):
 def _i8_gram_twice(lib, x_ptr, rows, d, ldx, seg_rows, seg_stride, dtype, x64, seed):
     ldg = d + 2                                    # even: the epilogue's TMA needs 16-byte G rows
     g0 = _randn(d, d, seed=seed)
-    g = Padded(d, d, ldg, F64, fill=g0)
+    g = Padded(d, d, ldg, F64, fill=g0, sentinel=OUT_SENTINEL)
     nbytes = lib.vlm_syrk_i8x4_scratch_bytes(rows, d)
     scratch = torch.empty(nbytes, dtype=torch.uint8, device="cuda")
     for _ in range(2):
