@@ -48,6 +48,19 @@ const char* vlm_last_error(void);       /* thread-local, never NULL */
 /* number of kernels this library has launched in the calling process (bench.py gpu_launches) */
 uint64_t    vlm_launch_count(void);
 
+/* Deterministic Gram accumulation: a thread-local mode (like vlm_last_error), off by default, read by every Gram entry
+ * point the calling thread uses afterwards: vlm_syrk_accum, _strided, _batch, _simt, _f64 and _i8x4.  By default their
+ * kernels add partial tiles from different CTAs into G in whatever order the hardware completes them, so the last
+ * bits of G can differ from run to run.  With the mode on, no two CTAs add into the same G element: every partial lands
+ * in its own slot of a per-call workspace (stream-ordered cudaMallocAsync / cudaFreeAsync on the launch stream), and
+ * one extra reduction launch per call adds each tile's slots, in schedule order, into G.
+ * Guarantee: bit-identical G for the same inputs (X and the starting G), dtype, shape and pitch, on a device with the
+ * same SM count, from the same library build.  The results differ in rounding from the default mode's, within the same
+ * error bounds.  Not covered: anything outside these entry points (the multi-GPU exchange, vlm_sim_topk).
+ * vlm_set_deterministic returns 0; vlm_get_deterministic returns the calling thread's mode (0 or 1). */
+int         vlm_set_deterministic(int on);
+int         vlm_get_deterministic(void);
+
 /* ---- (a) Gram accumulation -----------------------------------------------------------------
  * Replaces hook_gram_input, src/cache_gram_matrices.py:246-254:
  *     flatten_input = input.reshape(-1, D).to(float64); gram = flatten_input.T @ flatten_input

@@ -80,6 +80,8 @@ SIGNATURES = {
     "vlm_version": (c_int, []),
     "vlm_last_error": (c_char_p, []),
     "vlm_launch_count": (c_uint64, []),
+    "vlm_set_deterministic": (c_int, [c_int]),
+    "vlm_get_deterministic": (c_int, []),
     "vlm_syrk_accum": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_void_p, c_int64, c_void_p]),
     "vlm_tf32_split": (c_int, [c_void_p, c_int64, c_int, c_int64, c_int64, c_int64, c_void_p, c_void_p]),
     "vlm_syrk_accum_f64": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_int64, c_int64, c_void_p, c_int64,
@@ -140,6 +142,8 @@ def lib():
                 "or `make -C vl-merging_b200/csrc`.  There is no CPU fallback for the merge hot path.")
         h = ctypes.CDLL(LIB_PATH)
         for name, (restype, argtypes) in SIGNATURES.items():
+            if not hasattr(h, name):
+                raise RuntimeError(f"{LIB_PATH} does not export {name}: rebuild it (make -C vl-merging_b200/csrc)")
             fn = getattr(h, name)
             fn.restype = restype
             fn.argtypes = argtypes

@@ -104,9 +104,21 @@ int check_syrk_args(const char* who, const void* x, int dtype, int64_t rows, int
 
 using namespace vlm;
 
+namespace vlm {
+namespace {
+thread_local bool t_deterministic = false;
+}  // namespace
+bool deterministic_mode() { return t_deterministic; }
+}  // namespace vlm
+
 extern "C" int vlm_version(void) { return VLM_ABI_VERSION; }
 extern "C" const char* vlm_last_error(void) { return last_error_ref().c_str(); }
 extern "C" uint64_t vlm_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
+extern "C" int vlm_set_deterministic(int on) {
+  t_deterministic = on != 0;
+  return 0;
+}
+extern "C" int vlm_get_deterministic(void) { return t_deterministic ? 1 : 0; }
 
 extern "C" int vlm_syrk_accum(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
                               void* stream) {

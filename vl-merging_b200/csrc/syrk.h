@@ -40,4 +40,25 @@ void build_syrk_pair_schedule_host(int64_t kc, int d, int nsm, std::vector<int32
 int syrk_simt_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
                      cudaStream_t stream);
 
+// ---- deterministic mode (vlm_set_deterministic; syrk_det.cu) ---------------------------------------------------------
+// The calling thread's mode, read by every Gram launch.  In it no two CTAs add into the same G element: every
+// (tile, K range) partial lands in its own te x te slot of a per-call workspace (slot i at element offset i * te * te,
+// row pitch te), and one reduction launch then forms G_tile += ((s0 + s1) + s2) + ... over each tile's slots.
+bool deterministic_mode();
+// One upper tile of one Gram: slots [slot_begin, slot_end) summed in that order into G rows row0.., columns col0..
+// (entries inside d only).  mode 0: the whole tile; 1: a 256 x 256 diagonal tile of the CTA-pair kernels, whose block
+// below the diagonal (local rows >= 128, columns < 128) is never formed; 2: only c >= r (the CUDA-core kernel).
+struct DetItem {
+  int32_t pid, d, row0, col0, mode, slot_begin, slot_end, pad;
+};
+struct DetGram {  // G of problem pid in a grouped launch
+  void* g;
+  int64_t ldg;
+};
+// Stream-ordered workspace: slot_bytes of slots, then (when items is not NULL) a copy of *items.  Free with cudaFreeAsync.
+int det_workspace(size_t slot_bytes, const std::vector<DetItem>* items, cudaStream_t stream, void** ws, DetItem** d_items);
+// The reduction launch.  f64: slots and G are fp64, else fp32.  grams NULL: every item adds into g1 / ldg1.
+int det_reduce_launch(const DetItem* d_items, int nitems, int te, bool f64, const void* ws, void* g1, int64_t ldg1,
+                      const DetGram* grams, cudaStream_t stream);
+
 }  // namespace vlm

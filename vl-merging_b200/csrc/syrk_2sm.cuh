@@ -120,13 +120,15 @@ __device__ __forceinline__ void umma2(uint32_t d_tmem, uint64_t adesc, uint64_t 
 // BATCH = false: one problem, tensor maps in kernel parameters.  BATCH = true: the segments of several problems
 // (e.g. all Grams of the text tower of one forward) share the grid; tensor maps live in global memory (`maps`:
 // [2*pid] = X, [2*pid+1] = G), written by the host before the launch.  SPLIT: tm_x is the 4-D {hi, lo} map (see header); cps is ignored.
-template <int ELEM_BYTES, int FMT, bool BATCH, bool SPLIT>
+// DET (deterministic mode, syrk_det.cu): the G map (tm_g1, or every maps[2*pid+1]) describes the slot workspace, fp32
+// {256 columns, slots * 256 rows}, and the segments are BatchSegs whose `slot` says where the partial goes.
+template <int ELEM_BYTES, int FMT, bool BATCH, bool SPLIT, bool DET>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 syrk_2sm_kernel(const __grid_constant__ CUtensorMap tm_x1, const __grid_constant__ CUtensorMap tm_g1,
                 const CUtensorMap* __restrict__ maps, const void* __restrict__ segs_raw,
                 const int* __restrict__ seg_off, int d1, int cps1, int l2_hints) {
   using G = Geo2<ELEM_BYTES, SPLIT>;
-  using Seg = typename std::conditional<BATCH, BatchSeg, PairSeg>::type;
+  using Seg = typename std::conditional<BATCH || DET, BatchSeg, PairSeg>::type;
   const Seg* __restrict__ segs = static_cast<const Seg*>(segs_raw);
   auto map_x = [&](const Seg& sg) -> const CUtensorMap* {
     if constexpr (BATCH) return maps + 2 * sg.pid; else return &tm_x1;
@@ -331,7 +333,22 @@ syrk_2sm_kernel(const __grid_constant__ CUtensorMap tm_x1, const __grid_constant
         fence_proxy_async_smem();
         named_bar_sync(1, 128);
         if (epi_tid == 0) {
-          tma_reduce_add_2d_hint(tm_g, buf, col0 + sl * 32, row0, pol_g);
+          if constexpr (DET) {
+            // this CTA's 128 rows of the slot: the segment that opens the slot stores, later segments of this
+            // cluster on the same tile add.  Before adding, wait for COMPLETION (not just the source reads) of every
+            // earlier bulk operation of this thread, the previous store / reduce-add into this slot among them: PTX
+            // ISA, cp.async.bulk.wait_group — without .read, the wait lasts until the bulk async-groups are complete,
+            // writes to their destinations included.  The adds into a slot are then in segment order.
+            const int srow = (seg.slot >> 1) * 256 + (int)rank * 128, scol = n_off * 128 + sl * 32;
+            if (seg.slot & 1) {
+              if (sl == 0) bulk_wait_group<0>();
+              tma_reduce_add_2d_hint(tm_g, buf, scol, srow, pol_g);
+            } else {
+              tma_store_2d_hint(tm_g, buf, scol, srow, pol_g);
+            }
+          } else {
+            tma_reduce_add_2d_hint(tm_g, buf, col0 + sl * 32, row0, pol_g);
+          }
           bulk_commit_group();
         }
         ++slab_counter;

@@ -16,6 +16,7 @@
 // small Grams fill the GPU; every CTA adds its tile with red.global.add.f64 — the split-K reduction and the `+=`
 // across hook calls in one mechanism, like the TMA reduce-add of the tcgen05 kernels.
 #include <algorithm>
+#include <vector>
 
 #include "common.cuh"
 #include "syrk.h"
@@ -49,7 +50,9 @@ __device__ __forceinline__ double widen(__nv_bfloat16 v) { return (double)__bflo
 __device__ __forceinline__ double widen(__half v) { return (double)__half2float(v); }
 
 // VEC: rows and columns allow 16-byte cp.async chunks (x 16-byte aligned, ldx / seg_stride / d multiples of 16 bytes)
-template <typename T, bool VEC>
+// DET (deterministic mode, syrk_det.cu): g is the slot workspace; the CTA of tile blockIdx.x and K piece blockIdx.y
+// stores its whole 128 x 128 tile into slot blockIdx.x * gridDim.y + blockIdx.y (ldg unused)
+template <typename T, bool DET, bool VEC>
 __global__ void __launch_bounds__(512, 1)
 syrk_f64_kernel(const T* __restrict__ x, int64_t rows, int d, int64_t ldx, int64_t seg_rows, int64_t seg_stride,
                 double* __restrict__ g, int64_t ldg, int nb, int64_t rows_per_piece) {
@@ -124,6 +127,16 @@ syrk_f64_kernel(const T* __restrict__ x, int64_t rows, int d, int64_t ldx, int64
         for (int j = 0; j < 4; ++j) dmma_f64(c[i][j][0], c[i][j][1], a[i], b[j]);
     }
   }
+  if constexpr (DET) {
+    double* slot = g + ((size_t)blockIdx.x * gridDim.y + blockIdx.y) * FT * FT;
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        *reinterpret_cast<double2*>(slot + (wm + i * 8 + (lane >> 2)) * FT + wn + j * 8 + (lane & 3) * 2) =
+            make_double2(c[i][j][0], c[i][j][1]);
+    return;
+  }
 #pragma unroll
   for (int i = 0; i < 4; ++i)
 #pragma unroll
@@ -161,12 +174,30 @@ int launch_f64(const T* x, int64_t rows, int d, int64_t ldx, int64_t seg_rows, i
   const bool vec = (reinterpret_cast<uintptr_t>(x) & 15) == 0 && ldx % ev == 0 && seg_stride % ev == 0 && d % ev == 0;
   dim3 grid((unsigned)tiles, (unsigned)pieces);
   const int smem = (int)sizeof(F64Smem<T>);
+  if (deterministic_mode()) {
+    // tile t (row-major over the block-upper triangle, as the kernel numbers them): slots t * pieces .. + pieces
+    std::vector<DetItem> items;
+    for (int bi = 0, t = 0; bi < nb; ++bi)
+      for (int bj = bi; bj < nb; ++bj, ++t)
+        items.push_back({0, d, bi * FT, bj * FT, 0, (int)(t * pieces), (int)((t + 1) * pieces)});
+    void* ws = nullptr;
+    DetItem* d_items = nullptr;
+    if (int rc = det_workspace((size_t)tiles * pieces * FT * FT * sizeof(double), &items, stream, &ws, &d_items)) return rc;
+    auto kernel = vec ? syrk_f64_kernel<T, true, true> : syrk_f64_kernel<T, true, false>;
+    VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    kernel<<<grid, 512, smem, stream>>>(x, rows, d, ldx, seg_rows, seg_stride, static_cast<double*>(ws), 0, nb, rpp);
+    VLM_CUDA(cudaGetLastError());
+    count_launch();
+    if (int rc = det_reduce_launch(d_items, (int)items.size(), FT, true, ws, g, ldg, nullptr, stream)) return rc;
+    VLM_CUDA(cudaFreeAsync(ws, stream));
+    return 0;
+  }
   if (vec) {
-    auto kernel = syrk_f64_kernel<T, true>;
+    auto kernel = syrk_f64_kernel<T, false, true>;
     VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     kernel<<<grid, 512, smem, stream>>>(x, rows, d, ldx, seg_rows, seg_stride, g, ldg, nb, rpp);
   } else {
-    auto kernel = syrk_f64_kernel<T, false>;
+    auto kernel = syrk_f64_kernel<T, false, false>;
     VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     kernel<<<grid, 512, smem, stream>>>(x, rows, d, ldx, seg_rows, seg_stride, g, ldg, nb, rpp);
   }

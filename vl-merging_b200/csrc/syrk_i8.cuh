@@ -88,11 +88,22 @@ __device__ __forceinline__ double i8_pow2(int e) {
 
 // segs: PairSeg with the phase (0: groups 4 and 3, 1: groups 2 and 1, 2: group 0) in bits 16.. of sb; k in 32-row chunks
 // tm_g: G as a 2-D fp64 tensor, box 16 columns x 128 rows (the epilogue's TMA reduce-adds)
+// DET (deterministic mode, syrk_det.cu): segs are BatchSegs with a workspace `slot`, and tm_g describes the slot
+// workspace, fp64 {256 columns, slots * 256 rows}.  The phases a cluster runs on one tile chain into one slot.
+__device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, const void* smem_src, int c0, int c1) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
+                   reinterpret_cast<uint64_t>(tm)),
+               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
+               : "memory");
+}
+template <bool DET>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constant__ CUtensorMap tm_p1,
                  const __grid_constant__ CUtensorMap tm_p2, const __grid_constant__ CUtensorMap tm_g,
-                 const PairSeg* __restrict__ segs,
+                 const void* __restrict__ segs_raw,
                  const int* __restrict__ seg_off, int d, const __grid_constant__ I8Args args) {
+  using Seg = typename std::conditional<DET, BatchSeg, PairSeg>::type;
+  const Seg* __restrict__ segs = static_cast<const Seg*>(segs_raw);
   constexpr int kBlk = kBlockBytes;       // one operand of a stage
   constexpr int kNS = k2Stages;
   constexpr int kStageB = k2StageBytes;   // [A][B]
@@ -142,7 +153,7 @@ syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constan
     const uint64_t pol_x = l2_policy(0);
     const uint32_t full0 = mapa_rank(smem_u32(full), 0);
     for (int s = seg_begin; s < seg_end; ++s) {
-      const PairSeg seg = segs[s];
+      const Seg seg = segs[s];
       const int sb_t = seg.sb & 0xFFFF, ph = seg.sb >> 16;
       const bool diag = seg.sa == sb_t;
       const CUtensorMap* tm = ph == 0 ? &tm_p0 : ph == 1 ? &tm_p1 : &tm_p2;
@@ -173,7 +184,7 @@ syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constan
     constexpr uint32_t idesc = make_idesc_i8(256);
     constexpr uint32_t kP = kI8PlaneBytes >> 4;     // 32 rows of one plane, in descriptor units
     for (int s = seg_begin; s < seg_end; ++s) {
-      const PairSeg seg = segs[s];
+      const Seg seg = segs[s];
       const int sa_t = __shfl_sync(0xffffffffu, seg.sa, 0), sbw = __shfl_sync(0xffffffffu, seg.sb, 0);
       const int k0 = __shfl_sync(0xffffffffu, seg.k0, 0), k1 = __shfl_sync(0xffffffffu, seg.k1, 0);
       const int ph = sbw >> 16;
@@ -241,7 +252,7 @@ syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constan
       const uint32_t tempty0 = mapa_rank(smem_u32(tempty), 0);
       uint32_t slab_counter = 0;            // two slabs: the conversion of one overlaps the TMA engine's read of the other
       for (int s = seg_begin; s < seg_end; ++s) {
-        const PairSeg seg = segs[s];
+        const Seg seg = segs[s];
         const int sb_t = seg.sb & 0xFFFF, ph = seg.sb >> 16;
         const bool diag = seg.sa == sb_t;
         const int n_off = (diag && rank == 1) ? 1 : 0;   // peer on a diagonal tile: only block (2a+1, 2a+1)
@@ -280,7 +291,19 @@ syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constan
           fence_proxy_async_smem();
           named_bar_sync(1, 128);
           if (epi_tid == 0) {
-            tma_reduce_add_2d(&tm_g, buf, c0, row0);
+            if constexpr (DET) {
+              // as in syrk_2sm_kernel: the segment that opens the slot stores, a later one first waits for the
+              // completion (writes included: cp.async.bulk.wait_group without .read) of the earlier ones, then adds
+              const int srow = (seg.slot >> 1) * 256 + (int)rank * 128, scol = n_off * 128 + sl * 16;
+              if (seg.slot & 1) {
+                if (sl == 0) bulk_wait_group<0>();
+                tma_reduce_add_2d(&tm_g, buf, scol, srow);
+              } else {
+                tma_store_2d(&tm_g, buf, scol, srow);
+              }
+            } else {
+              tma_reduce_add_2d(&tm_g, buf, c0, row0);
+            }
             bulk_commit_group();
           }
           ++slab_counter;

@@ -64,11 +64,21 @@ __device__ __forceinline__ void tma_reduce_add_2d_hint(const CUtensorMap* tm, co
       : "memory");
 }
 
+__device__ __forceinline__ void tma_store_2d_hint(const CUtensorMap* tm, const void* smem_src, int c0, int c1,
+                                                  uint64_t pol) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3}], [%1], %4;" ::"l"(
+                   reinterpret_cast<uint64_t>(tm)),
+               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "l"(pol)
+               : "memory");
+}
+
 // One unit of work of a cluster in a BATCHED launch (several independent Gram problems in one grid): as PairSeg,
 // plus which problem it belongs to (index into the tensor-map array) and that problem's column count.
 // cps = chunks per row segment of a segmented activation (0: contiguous rows, 3-D tensor map).
+// slot (deterministic mode only, where single launches use this layout too): workspace slot << 1 | 1 if an earlier
+// segment of the same cluster already wrote that slot (det_slots).
 struct BatchSeg {
-  int32_t sa, sb, k0, k1, pid, d, cps, pad;
+  int32_t sa, sb, k0, k1, pid, d, cps, slot;
 };
 __device__ __forceinline__ void tensormap_acquire(const CUtensorMap* tm) {
   asm volatile("fence.proxy.tensormap::generic.acquire.gpu [%0], 128;" ::"l"(reinterpret_cast<uint64_t>(tm)) : "memory");
@@ -82,22 +92,75 @@ __device__ __forceinline__ void tensormap_acquire(const CUtensorMap* tm) {
 
 namespace vlm {
 namespace {
+// d_segs: PairSegs, or in the deterministic mode BatchSegs with workspace slots, plus the reduction's tile list
 struct DeviceSchedule2 {
   int nclusters = 0;
-  PairSeg* d_segs = nullptr;
+  void* d_segs = nullptr;
   int* d_off = nullptr;
+  DetItem* d_items = nullptr;
+  int nitems = 0, nslots = 0;
 };
 std::mutex g_mu2;
-typedef std::tuple<int, int64_t, int, int, int> ScheduleKey;  // (device, chunks, d, chunk rows or -8 for int8, SMs)
+// (device, chunks, d, chunk rows or -8 for int8, SMs, deterministic)
+typedef std::tuple<int, int64_t, int, int, int, bool> ScheduleKey;
 std::map<ScheduleKey, DeviceSchedule2> g_sched2;
 // schedules evicted from the cache: freed at the NEXT eviction, after a device synchronisation, never while a
 // launch that was handed their pointers may still be pending (the lock is held from lookup to launch)
 std::vector<DeviceSchedule2> g_retired2;
 
+// Deterministic mode: gives every (problem, super-tile, cluster) a workspace slot of its own.  The slots of one tile
+// are numbered consecutively in schedule order (cluster by cluster, each cluster's segments in order), which is the
+// order the reduction adds them in.  Sets seg.slot = slot << 1 | (1 when an earlier segment of the same cluster opened
+// the slot: that one stores, the later ones add); returns the number of slots and one DetItem per tile.  same_g (grouped
+// launches): problem p adds into the G of problem same_g[p] <= p, so that problems sharing a G share its tiles' items.
+int det_slots(std::vector<BatchSeg>* segs, const std::vector<int>& off, std::vector<DetItem>* items,
+              const std::vector<int>* same_g = nullptr) {
+  std::map<std::tuple<int, int, int>, int> tile_of;  // (G, super row, super column) -> index into items
+  std::vector<std::vector<int>> opened;              // per tile: its temporary slot ids, in schedule order
+  std::vector<int> temp(segs->size());
+  int ntemp = 0;
+  items->clear();
+  for (size_t c = 0; c + 1 < off.size(); ++c) {
+    std::map<int, int> mine;  // tile -> temporary slot id of this cluster
+    for (int s = off[c]; s < off[c + 1]; ++s) {
+      BatchSeg& q = (*segs)[s];
+      const int sb = q.sb & 0xFFFF;  // (the int8 schedule keeps the phase in the bits above)
+      const int gp = same_g ? (*same_g)[q.pid] : q.pid;
+      auto t = tile_of.emplace(std::make_tuple(gp, q.sa, sb), (int)items->size());
+      if (t.second) {
+        items->push_back({gp, q.d, q.sa * 256, sb * 256, q.sa == sb ? 1 : 0, 0, 0, 0});
+        opened.emplace_back();
+      }
+      const int tile = t.first->second;
+      auto m = mine.find(tile);
+      if (m == mine.end()) {
+        mine.emplace(tile, ntemp);
+        opened[tile].push_back(ntemp);
+        temp[s] = ntemp++;
+        q.slot = 0;
+      } else {
+        temp[s] = m->second;
+        q.slot = 1;
+      }
+    }
+  }
+  std::vector<int> final_id(ntemp);
+  int next = 0;
+  for (size_t t = 0; t < items->size(); ++t) {
+    (*items)[t].slot_begin = next;
+    for (int id : opened[t]) final_id[id] = next++;
+    (*items)[t].slot_end = next;
+  }
+  for (size_t s = 0; s < segs->size(); ++s) (*segs)[s].slot |= final_id[temp[s]] << 1;
+  return next;
+}
+
 // The device copy of the schedule `build` makes for `key`, built and uploaded on first use.  Call with g_mu2 held
-// until the launch that reads it is enqueued.
+// until the launch that reads it is enqueued.  Deterministic keys: as BatchSegs of one problem of width d (cps chunks
+// per row segment) with their workspace slots.
 template <typename Build>
-int cached_schedule(const ScheduleKey& key, Build build, cudaStream_t stream, const DeviceSchedule2** out) {
+int cached_schedule(const ScheduleKey& key, Build build, cudaStream_t stream, const DeviceSchedule2** out, int d = 0,
+                    int cps = 0) {
   auto it = g_sched2.find(key);
   if (it == g_sched2.end()) {
     if (g_sched2.size() >= 512) {  // ragged workloads (a new row count every call): start over, do not grow forever
@@ -105,6 +168,7 @@ int cached_schedule(const ScheduleKey& key, Build build, cudaStream_t stream, co
       for (auto& ds : g_retired2) {
         cudaFree(ds.d_segs);
         cudaFree(ds.d_off);
+        cudaFree(ds.d_items);
       }
       g_retired2.clear();
       for (auto& kv : g_sched2) g_retired2.push_back(kv.second);
@@ -115,14 +179,42 @@ int cached_schedule(const ScheduleKey& key, Build build, cudaStream_t stream, co
     build(&segs, &off);
     DeviceSchedule2 ds;
     ds.nclusters = (int)off.size() - 1;
-    VLM_CUDA(cudaMalloc(&ds.d_segs, std::max<size_t>(1, segs.size()) * sizeof(PairSeg)));
+    const void* seg_src = segs.data();
+    size_t seg_bytes = segs.size() * sizeof(PairSeg);
+    std::vector<BatchSeg> bsegs;
+    std::vector<DetItem> items;
+    if (std::get<5>(key)) {
+      for (const PairSeg& s : segs) bsegs.push_back({s.sa, s.sb, s.k0, s.k1, 0, d, cps, 0});
+      ds.nslots = det_slots(&bsegs, off, &items);
+      ds.nitems = (int)items.size();
+      seg_src = bsegs.data();
+      seg_bytes = bsegs.size() * sizeof(BatchSeg);
+      VLM_CUDA(cudaMalloc(&ds.d_items, std::max<size_t>(1, items.size()) * sizeof(DetItem)));
+      VLM_CUDA(cudaMemcpyAsync(ds.d_items, items.data(), items.size() * sizeof(DetItem), cudaMemcpyHostToDevice, stream));
+    }
+    VLM_CUDA(cudaMalloc(&ds.d_segs, std::max<size_t>(1, seg_bytes)));
     VLM_CUDA(cudaMalloc(&ds.d_off, off.size() * sizeof(int)));
-    VLM_CUDA(cudaMemcpyAsync(ds.d_segs, segs.data(), segs.size() * sizeof(PairSeg), cudaMemcpyHostToDevice, stream));
+    VLM_CUDA(cudaMemcpyAsync(ds.d_segs, seg_src, seg_bytes, cudaMemcpyHostToDevice, stream));
     VLM_CUDA(cudaMemcpyAsync(ds.d_off, off.data(), off.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
     VLM_CUDA(cudaStreamSynchronize(stream));
     it = g_sched2.emplace(key, ds).first;
   }
   *out = &it->second;
+  return 0;
+}
+
+// The slot workspace of the deterministic mode as a 2-D TMA tensor {256 columns, slots * 256 rows}, with the box and
+// swizzle of the G map it stands in for (fp32: 32 x 128, fp64: 16 x 128)
+int encode_slot_map(EncodeTiledFn encode, void* ws, int nslots, bool f64, CUtensorMap* tm) {
+  const int elem = f64 ? 8 : 4;
+  cuuint64_t gdim[2] = {256, (cuuint64_t)nslots * 256};
+  cuuint64_t gstr[1] = {(cuuint64_t)256 * elem};
+  cuuint32_t box[2] = {(cuuint32_t)(128 / elem), 128};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = encode(tm, f64 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, ws, gdim, gstr, box,
+                      estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  VLM_REQUIRE(r == CUDA_SUCCESS, VLM_ERR_DRIVER, "cuTensorMapEncodeTiled(slot workspace) failed: CUresult %d", (int)r);
   return 0;
 }
 
@@ -192,12 +284,12 @@ int l2_hints() {
 
 typedef void (*PairKernel)(const CUtensorMap, const CUtensorMap, const CUtensorMap*, const void*, const int*, int, int,
                            int);
-template <bool BATCH>
+template <bool BATCH, bool DET>
 PairKernel pick_kernel(int dtype) {
-  if (dtype == VLM_TF32X2) return syrk_2sm_kernel<4, 2, BATCH, true>;
-  if (dtype == VLM_F32) return syrk_2sm_kernel<4, 2, BATCH, false>;
-  if (dtype == VLM_BF16) return syrk_2sm_kernel<2, 1, BATCH, false>;
-  return syrk_2sm_kernel<2, 0, BATCH, false>;
+  if (dtype == VLM_TF32X2) return syrk_2sm_kernel<4, 2, BATCH, true, DET>;
+  if (dtype == VLM_F32) return syrk_2sm_kernel<4, 2, BATCH, false, DET>;
+  if (dtype == VLM_BF16) return syrk_2sm_kernel<2, 1, BATCH, false, DET>;
+  return syrk_2sm_kernel<2, 0, BATCH, false, DET>;
 }
 
 }  // namespace
@@ -376,22 +468,35 @@ int syrk_pair_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
   CUtensorMap tm_x, tm_g;
   if (int rc = encode_maps(encode, x, dtype, rows, d, ldx, seg_rows, seg_stride, g, ldg, &tm_x, &tm_g)) return rc;
   const int smem = k2SmemBytes;
-  PairKernel kernel = pick_kernel<false>(dtype);
+  const bool det = deterministic_mode();
+  PairKernel kernel = det ? pick_kernel<false, true>(dtype) : pick_kernel<false, false>(dtype);
 
   // lookup and launch under one lock: an eviction by another host thread cannot free a schedule between the two
   std::lock_guard<std::mutex> lk(g_mu2);
   const DeviceSchedule2* sched = nullptr;
-  if (int rc = cached_schedule(std::make_tuple(dev, kc, d, bk, nsm),
+  if (int rc = cached_schedule(std::make_tuple(dev, kc, d, bk, nsm, det),
                                [&](std::vector<PairSeg>* segs, std::vector<int>* off) {
                                  build_pair_schedule(kc, d, nsm / 2, segs, off);
                                },
-                               stream, &sched))
+                               stream, &sched, d, (int)cps))
     return rc;
   VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  void* ws = nullptr;
+  if (det) {
+    if (int rc = det_workspace((size_t)sched->nslots * 256 * 256 * 4, nullptr, stream, &ws, nullptr)) return rc;
+    if (int rc = encode_slot_map(encode, ws, sched->nslots, false, &tm_g)) {
+      cudaFreeAsync(ws, stream);
+      return rc;
+    }
+  }
   kernel<<<2 * sched->nclusters, kThreads, smem, stream>>>(tm_x, tm_g, nullptr, sched->d_segs, sched->d_off, d, (int)cps,
                                                            l2_hints());
   VLM_CUDA(cudaGetLastError());
   count_launch();
+  if (det) {
+    if (int rc = det_reduce_launch(sched->d_items, sched->nitems, 256, false, ws, g, ldg, nullptr, stream)) return rc;
+    VLM_CUDA(cudaFreeAsync(ws, stream));
+  }
   return 0;
 }
 
@@ -531,21 +636,35 @@ int syrk_i8x4_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
   }
   const int64_t kc = (rows + 31) / 32;
   VLM_REQUIRE(kc < (int64_t)1 << 30, VLM_ERR_INVALID_ARG, "vlm_syrk_accum_i8x4: too many row chunks");
+  const bool det = deterministic_mode();
   std::lock_guard<std::mutex> lk(g_mu2);
   const DeviceSchedule2* sched = nullptr;
-  if (int rc = cached_schedule(std::make_tuple(dev, kc, d, -8, nsm),  // chunk rows -8: the int8 schedule
+  if (int rc = cached_schedule(std::make_tuple(dev, kc, d, -8, nsm, det),  // chunk rows -8: the int8 schedule
                                [&](std::vector<PairSeg>* segs, std::vector<int>* off) {
                                  build_i8_schedule(kc, d, nsm / 2, segs, off);
                                },
-                               stream, &sched))
+                               stream, &sched, d))
     return rc;
   const int smem = kI8SmemBytes;
-  VLM_CUDA(cudaFuncSetAttribute(syrk_i8x4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  auto kernel = det ? syrk_i8x4_kernel<true> : syrk_i8x4_kernel<false>;
+  VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  void* ws = nullptr;
+  if (det) {
+    if (int rc = det_workspace((size_t)sched->nslots * 256 * 256 * 8, nullptr, stream, &ws, nullptr)) return rc;
+    if (int rc = encode_slot_map(encode, ws, sched->nslots, true, &tm_g)) {
+      cudaFreeAsync(ws, stream);
+      return rc;
+    }
+  }
   I8Args args{g, ldg, exps};
-  syrk_i8x4_kernel<<<2 * sched->nclusters, kThreads, smem, stream>>>(tm_p[0], tm_p[1], tm_p[2], tm_g, sched->d_segs,
-                                                                     sched->d_off, d, args);
+  kernel<<<2 * sched->nclusters, kThreads, smem, stream>>>(tm_p[0], tm_p[1], tm_p[2], tm_g, sched->d_segs, sched->d_off, d,
+                                                           args);
   VLM_CUDA(cudaGetLastError());
   count_launch();
+  if (det) {
+    if (int rc = det_reduce_launch(sched->d_items, sched->nitems, 256, true, ws, g, ldg, nullptr, stream)) return rc;
+    VLM_CUDA(cudaFreeAsync(ws, stream));
+  }
   return 0;
 }
 
@@ -622,14 +741,45 @@ int syrk_pair_batch_launch(const vlm_syrk_problem* probs, int n, int dtype, cuda
     foff.push_back((int)flat.size());
   }
   if (flat.empty()) return 0;
+  // deterministic mode: every problem's G map is replaced by the map of the one slot workspace, and the reduction's
+  // tile list and the problems' G pointers follow the segments in the table
+  const bool det = deterministic_mode();
+  std::vector<DetItem> items;
+  std::vector<DetGram> grams;
+  void* ws = nullptr;
+  if (det) {
+    std::vector<int> same_g(n);
+    for (int p = 0; p < n; ++p) {
+      same_g[p] = p;
+      for (int q = 0; q < p; ++q)
+        if (probs[q].g == probs[p].g && probs[q].ldg == probs[p].ldg) {
+          same_g[p] = q;
+          break;
+        }
+      grams.push_back({probs[p].g, probs[p].ldg});
+    }
+    const int nslots = det_slots(&flat, foff, &items, &same_g);
+    if (int rc = det_workspace((size_t)nslots * 256 * 256 * 4, nullptr, stream, &ws, nullptr)) return rc;
+    CUtensorMap tm_ws;
+    if (int rc = encode_slot_map(encode, ws, nslots, false, &tm_ws)) {
+      cudaFreeAsync(ws, stream);
+      return rc;
+    }
+    for (int p = 0; p < n; ++p) maps[2 * p + 1] = tm_ws;
+  }
   const size_t maps_bytes = maps.size() * sizeof(CUtensorMap);
   const size_t off_bytes = ((foff.size() * sizeof(int)) + 127) / 128 * 128;
   const size_t seg_bytes = flat.size() * sizeof(BatchSeg);
-  const size_t total = maps_bytes + off_bytes + seg_bytes;
+  const size_t item_bytes = items.size() * sizeof(DetItem), gram_bytes = grams.size() * sizeof(DetGram);
+  const size_t total = maps_bytes + off_bytes + seg_bytes + item_bytes + gram_bytes;
   std::vector<uint8_t> host(total);
   memcpy(host.data(), maps.data(), maps_bytes);
   memcpy(host.data() + maps_bytes, foff.data(), foff.size() * sizeof(int));
   memcpy(host.data() + maps_bytes + off_bytes, flat.data(), seg_bytes);
+  if (det) {
+    memcpy(host.data() + maps_bytes + off_bytes + seg_bytes, items.data(), item_bytes);
+    memcpy(host.data() + maps_bytes + off_bytes + seg_bytes + item_bytes, grams.data(), gram_bytes);
+  }
   uint8_t* dptr = nullptr;
   {
     std::lock_guard<std::mutex> lk(g_mu2);
@@ -646,13 +796,20 @@ int syrk_pair_batch_launch(const vlm_syrk_problem* probs, int n, int dtype, cuda
   // pageable source: staged before the call returns; ordered on `stream` before the kernel below
   VLM_CUDA(cudaMemcpyAsync(dptr, host.data(), total, cudaMemcpyHostToDevice, stream));
   const int smem = k2SmemBytes;
-  PairKernel kernel = pick_kernel<true>(dtype);
+  PairKernel kernel = det ? pick_kernel<true, true>(dtype) : pick_kernel<true, false>(dtype);
   VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   kernel<<<2 * ncl, kThreads, smem, stream>>>(maps[0], maps[1], reinterpret_cast<const CUtensorMap*>(dptr),
                                               dptr + maps_bytes + off_bytes,
                                               reinterpret_cast<const int*>(dptr + maps_bytes), 0, 0, l2_hints());
   VLM_CUDA(cudaGetLastError());
   count_launch();
+  if (det) {
+    const uint8_t* d_items = dptr + maps_bytes + off_bytes + seg_bytes;
+    if (int rc = det_reduce_launch(reinterpret_cast<const DetItem*>(d_items), (int)items.size(), 256, false, ws, nullptr,
+                                   0, reinterpret_cast<const DetGram*>(d_items + item_bytes), stream))
+      return rc;
+    VLM_CUDA(cudaFreeAsync(ws, stream));
+  }
   return 0;
 }
 

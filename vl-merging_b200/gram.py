@@ -13,6 +13,7 @@ torch.save(middle_representations, path)     GramCache.save(path): {name: fp64 C
                                              regmean() loads (vilt_module.py:386)
 (absent: every DDP rank writes its own sums) GramCache.all_reduce(): ONE NCCL all-reduce of the packed upper triangles
 """
+import contextlib
 from collections import defaultdict
 
 import torch
@@ -132,7 +133,7 @@ class GramCache:
     """
 
     def __init__(self, device=None, use_simt=False, defer_bytes=0, max_pending=256, max_pending_bytes=1 << 30,
-                 side_stream=False, precision="tf32", symmetric=False):
+                 side_stream=False, precision="tf32", symmetric=False, deterministic=None):
         """precision: how fp32 activations reach the tensor cores.  "tf32" (default): one TF32 pass, operands rounded
         by TMA — Gram within ~3e-5 of the reference's fp64 Gram (cache_gram_matrices.py:251-252), inside the 1e-3
         tolerance, but its 2^-11 operand rounding noise is amplified by the inverse in regmean
@@ -168,7 +169,12 @@ class GramCache:
         phases leave the tensor pipes idle; flush() joins the two streams.  Like deferral it holds a reference to
         every hooked activation until the next flush() and assumes nothing modifies them in place; register()
         flushes after every forward of the registered model.  Not for precision="int8x4": its persistent 148-CTA kernels
-        and the forward's GEMMs do not share SMs well (measured 649 vs 834 samples/s)."""
+        and the forward's GEMMs do not share SMs well (measured 649 vs 834 samples/s).
+        deterministic: every Gram launch of this cache (immediate, deferred or grouped, side stream, every precision)
+        runs in the library's deterministic mode (vlm_set_deterministic): the same activations give the same Gram bits
+        in every run on the same GPU model and library build, at the cost of a slot workspace and one reduction launch
+        per call.  None (default): torch.are_deterministic_algorithms_enabled() at construction.  The library's
+        thread-local flag is set only around this cache's own calls."""
         self.device = torch.device(device if device is not None else "cuda")
         if self.device.type != "cuda":
             raise RuntimeError("GramCache needs a CUDA device: the Gram hot path has no CPU fallback")
@@ -195,6 +201,21 @@ class GramCache:
         self.symmetric, self._symm = bool(symmetric), None   # symmetric-memory arena and its rendezvous handle
         self._side = torch.cuda.Stream(self.device) if side_stream else None
         self._side_keep = []   # activations a side-stream launch may still be reading
+        self.deterministic = bool(torch.are_deterministic_algorithms_enabled() if deterministic is None else deterministic)
+
+    @contextlib.contextmanager
+    def _mode(self):
+        """The library's thread-local deterministic flag at this cache's mode for the cache's own launches, restored
+        after them."""
+        prev = self._lib.vlm_get_deterministic()
+        if prev == self.deterministic:
+            yield
+            return
+        self._lib.vlm_set_deterministic(int(self.deterministic))
+        try:
+            yield
+        finally:
+            self._lib.vlm_set_deterministic(prev)
 
     # ---- the hook -------------------------------------------------------------------------------
     def hook_gram_input(self, module, input, output):
@@ -208,6 +229,10 @@ class GramCache:
     __call__ = hook_gram_input
 
     def accumulate(self, name, x):
+        with self._mode():
+            self._accumulate(name, x)
+
+    def _accumulate(self, name, x):
         d = x.shape[-1]
         if x.device != self.device:
             raise RuntimeError(f"activation for {name} is on {x.device}, GramCache is on {self.device}")
@@ -318,6 +343,10 @@ class GramCache:
     def flush(self):
         """Issue every deferred activation (one grouped launch per dtype) and, in side-stream mode, make the
         current stream wait for the Gram launches."""
+        with self._mode():
+            self._flush()
+
+    def _flush(self):
         if not self._pending:
             return self._join()
         pending, self._pending, self._pending_bytes = self._pending, [], 0
