@@ -47,17 +47,17 @@ int device_sm_count(int* out) {
 }
 
 int tensor_map_encoder(EncodeTiledFn* out) {
-  static EncodeTiledFn encode = nullptr;
-  std::lock_guard<std::mutex> lk(g_dev_mu);
-  if (!encode) {
+  // the driver's entry point, the same for every thread: a race between two first lookups stores it twice
+  static std::atomic<EncodeTiledFn> encode{nullptr};
+  if (!encode.load(std::memory_order_acquire)) {
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
     VLM_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
     VLM_REQUIRE(fn != nullptr && qres == cudaDriverEntryPointSuccess, VLM_ERR_DRIVER,
                 "cuTensorMapEncodeTiled not available from the driver");
-    encode = reinterpret_cast<EncodeTiledFn>(fn);
+    encode.store(reinterpret_cast<EncodeTiledFn>(fn), std::memory_order_release);
   }
-  *out = encode;
+  *out = encode.load(std::memory_order_acquire);
   return 0;
 }
 
@@ -120,79 +120,99 @@ extern "C" int vlm_set_deterministic(int on) {
 }
 extern "C" int vlm_get_deterministic(void) { return t_deterministic ? 1 : 0; }
 
-extern "C" int vlm_syrk_accum(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
-                              void* stream) {
-  if (int rc = check_syrk_args("vlm_syrk_accum", x, dtype, rows, d, ldx, g, ldg)) return rc;
-  if (rows == 0) return 0;
-  if (int rc = require_sm100()) return rc;
-  const bool pair = syrk_pair_supported(dtype, x, d, ldx, 0, g, ldg);
-  if (dtype == VLM_TF32X2) {  // the planes exist only for the CTA-pair kernel
-    VLM_REQUIRE(d % 32 == 0, VLM_ERR_UNSUPPORTED,
-                "vlm_syrk_accum: VLM_TF32X2 needs d %% 32 == 0 (got %d); use vlm_syrk_accum_simt on the fp32 activation", d);
-    VLM_REQUIRE(pair, VLM_ERR_ALIGNMENT,
-                "vlm_syrk_accum: VLM_TF32X2 planes and g must be 16-byte aligned with ldx and ldg multiples of 4");
-  }
-  if (pair) return syrk_pair_launch(x, dtype, rows, d, ldx, 0, 0, g, ldg, static_cast<cudaStream_t>(stream));
-  return syrk_simt_launch(x, dtype, rows, d, ldx, g, ldg, static_cast<cudaStream_t>(stream));
-}
-
 namespace {
-int check_segments(const char* who, int dtype, int64_t rows, int64_t seg_rows, int64_t seg_stride) {
+int check_segments(const char* who, int64_t rows, int64_t seg_rows, int64_t seg_stride) {
   VLM_REQUIRE(seg_rows > 0 && rows % seg_rows == 0, VLM_ERR_INVALID_ARG,
               "%s: rows (%lld) must be a multiple of seg_rows (%lld)", who, (long long)rows, (long long)seg_rows);
   VLM_REQUIRE(seg_stride >= 0, VLM_ERR_INVALID_ARG, "%s: seg_stride < 0", who);
-  (void)dtype;
   return 0;
+}
+
+// The fp32-accumulating Gram entry points, and how a Gram of theirs runs
+enum class Entry { kAccum, kStrided, kBatch };
+enum class GramPath { kNone, kPair, kPerSegment, kSimt };
+
+// The one router of vlm_syrk_accum, _strided and _batch.  Validates every problem, normalises its row segments
+// (afterwards seg_rows > 0 only for two or more segments, never for VLM_TF32X2) and picks its path: the CTA-pair
+// kernel, one launch per segment where that kernel cannot read the segments in one launch, or the CUDA-core kernel.
+// Only then does anything run.  vlm_syrk_accum_strided asks for its segments, which must divide the rows; a vlm_syrk_problem
+// with seg_rows outside (0, rows), or of VLM_TF32X2 planes, is one run of rows.  kBatch: the Grams for the CTA-pair
+// kernel share one grouped launch.
+int syrk_route(Entry entry, const vlm_syrk_problem* probs, int n, int dtype, cudaStream_t stream) {
+  static const char* const kWho[] = {"vlm_syrk_accum", "vlm_syrk_accum_strided", "vlm_syrk_accum_batch"};
+  const char* who = kWho[(int)entry];
+  std::vector<vlm_syrk_problem> qs(probs, probs + n);
+  std::vector<GramPath> paths(n, GramPath::kNone);
+  bool any = false;
+  for (int p = 0; p < n; ++p) {
+    vlm_syrk_problem& q = qs[p];
+    if (int rc = check_syrk_args(who, q.x, dtype, q.rows, q.d, q.ldx, q.g, q.ldg)) return rc;
+    if (q.rows == 0) continue;
+    const bool strided = entry == Entry::kStrided;
+    bool segmented = q.seg_rows > 0 && q.seg_rows < q.rows && (strided || dtype != VLM_TF32X2);
+    if (strided || segmented) {
+      if (int rc = check_segments(who, q.rows, q.seg_rows, q.seg_stride)) return rc;
+    }
+    VLM_REQUIRE(!segmented || dtype != VLM_TF32X2, VLM_ERR_INVALID_ARG,
+                "%s: VLM_TF32X2 planes are packed by vlm_tf32_split, they have no row segments", who);
+    if (!segmented) q.seg_rows = q.seg_stride = 0;
+    const bool pair = syrk_pair_supported(dtype, q.x, q.d, q.ldx, q.seg_stride, q.g, q.ldg);
+    if (dtype == VLM_TF32X2) {  // the planes exist only for the CTA-pair kernel
+      VLM_REQUIRE(pair || entry != Entry::kBatch, VLM_ERR_UNSUPPORTED,
+                  "%s: VLM_TF32X2 needs d %% 32 == 0 and 16-byte aligned planes", who);
+      VLM_REQUIRE(q.d % 32 == 0, VLM_ERR_UNSUPPORTED,
+                  "%s: VLM_TF32X2 needs d %% 32 == 0 (got %d); use vlm_syrk_accum_simt on the fp32 activation", who,
+                  q.d);
+      VLM_REQUIRE(pair, VLM_ERR_ALIGNMENT,
+                  "%s: VLM_TF32X2 planes and g must be 16-byte aligned with ldx and ldg multiples of 4", who);
+    }
+    paths[p] = pair ? GramPath::kPair : segmented ? GramPath::kPerSegment : GramPath::kSimt;
+    any = true;
+  }
+  if (!any) return 0;
+  if (int rc = require_sm100()) return rc;
+  std::vector<vlm_syrk_problem> grouped;
+  for (int p = 0; p < n; ++p) {
+    const vlm_syrk_problem& q = qs[p];
+    int rc = 0;
+    if (paths[p] == GramPath::kPair && entry == Entry::kBatch) {
+      grouped.push_back(q);
+    } else if (paths[p] == GramPath::kPair) {
+      rc = syrk_pair_launch(q.x, dtype, q.rows, q.d, q.ldx, q.seg_rows, q.seg_stride, q.g, q.ldg, stream);
+    } else if (paths[p] == GramPath::kSimt) {
+      rc = syrk_simt_launch(q.x, dtype, q.rows, q.d, q.ldx, q.g, q.ldg, stream);
+    } else if (paths[p] == GramPath::kPerSegment) {
+      // row segments the CTA-pair kernel cannot read in one launch: each segment is a Gram of its own
+      const int elem = dtype == VLM_F32 ? 4 : 2;
+      for (int64_t s = 0; s < q.rows / q.seg_rows && rc == 0; ++s) {
+        const char* xs = static_cast<const char*>(q.x) + (size_t)s * q.seg_stride * elem;
+        rc = syrk_pair_supported(dtype, xs, q.d, q.ldx, 0, q.g, q.ldg)
+                 ? syrk_pair_launch(xs, dtype, q.seg_rows, q.d, q.ldx, 0, 0, q.g, q.ldg, stream)
+                 : syrk_simt_launch(xs, dtype, q.seg_rows, q.d, q.ldx, q.g, q.ldg, stream);
+      }
+    }
+    if (rc) return rc;
+  }
+  if (grouped.empty()) return 0;
+  return syrk_pair_batch_launch(grouped.data(), (int)grouped.size(), dtype, stream);
 }
 }  // namespace
 
+extern "C" int vlm_syrk_accum(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
+                              void* stream) {
+  const vlm_syrk_problem q{x, rows, ldx, g, ldg, d, 0, 0, 0};
+  return syrk_route(Entry::kAccum, &q, 1, dtype, static_cast<cudaStream_t>(stream));
+}
+
 extern "C" int vlm_syrk_accum_strided(const void* x, int dtype, int64_t rows, int d, int64_t ldx, int64_t seg_rows,
                                       int64_t seg_stride, float* g, int64_t ldg, void* stream) {
-  if (int rc = check_syrk_args("vlm_syrk_accum_strided", x, dtype, rows, d, ldx, g, ldg)) return rc;
-  if (rows == 0) return 0;
-  if (int rc = check_segments("vlm_syrk_accum_strided", dtype, rows, seg_rows, seg_stride)) return rc;
-  if (seg_rows == rows) return vlm_syrk_accum(x, dtype, rows, d, ldx, g, ldg, stream);
-  VLM_REQUIRE(dtype != VLM_TF32X2, VLM_ERR_INVALID_ARG,
-              "vlm_syrk_accum_strided: VLM_TF32X2 planes are packed by vlm_tf32_split, they have no row segments");
-  if (int rc = require_sm100()) return rc;
-  if (syrk_pair_supported(dtype, x, d, ldx, seg_stride, g, ldg))
-    return syrk_pair_launch(x, dtype, rows, d, ldx, seg_rows, seg_stride, g, ldg, static_cast<cudaStream_t>(stream));
-  // row segments the CTA-pair kernel cannot read in one launch: one vlm_syrk_accum per segment
-  const int elem = dtype == VLM_F32 ? 4 : 2;
-  for (int64_t s = 0; s < rows / seg_rows; ++s) {
-    const char* xs = static_cast<const char*>(x) + (size_t)s * seg_stride * elem;
-    if (int rc = vlm_syrk_accum(xs, dtype, seg_rows, d, ldx, g, ldg, stream)) return rc;
-  }
-  return 0;
+  const vlm_syrk_problem q{x, rows, ldx, g, ldg, d, 0, seg_rows, seg_stride};
+  return syrk_route(Entry::kStrided, &q, 1, dtype, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int vlm_syrk_accum_batch(const vlm_syrk_problem* probs, int n, int dtype, void* stream) {
   VLM_REQUIRE(n >= 0 && (probs != nullptr || n == 0), VLM_ERR_INVALID_ARG, "vlm_syrk_accum_batch: bad arguments");
-  if (n == 0) return 0;
-  if (int rc = require_sm100()) return rc;
-  std::vector<vlm_syrk_problem> grouped;
-  for (int p = 0; p < n; ++p) {
-    const vlm_syrk_problem& q = probs[p];
-    if (int rc = check_syrk_args("vlm_syrk_accum_batch", q.x, dtype, q.rows, q.d, q.ldx, q.g, q.ldg)) return rc;
-    if (q.rows == 0) continue;
-    const bool segmented = dtype != VLM_TF32X2 && q.seg_rows > 0 && q.seg_rows < q.rows;
-    const bool pair = syrk_pair_supported(dtype, q.x, q.d, q.ldx, segmented ? q.seg_stride : 0, q.g, q.ldg);
-    VLM_REQUIRE(dtype != VLM_TF32X2 || pair, VLM_ERR_UNSUPPORTED,
-                "vlm_syrk_accum_batch: VLM_TF32X2 needs d %% 32 == 0 and 16-byte aligned planes");
-    if (segmented) {
-      if (int rc = check_segments("vlm_syrk_accum_batch", dtype, q.rows, q.seg_rows, q.seg_stride)) return rc;
-    }
-    if (pair) {
-      grouped.push_back(q);
-    } else if (segmented) {
-      if (int rc = vlm_syrk_accum_strided(q.x, dtype, q.rows, q.d, q.ldx, q.seg_rows, q.seg_stride, q.g, q.ldg, stream))
-        return rc;
-    } else if (int rc = vlm_syrk_accum(q.x, dtype, q.rows, q.d, q.ldx, q.g, q.ldg, stream)) {
-      return rc;
-    }
-  }
-  if (grouped.empty()) return 0;
-  return syrk_pair_batch_launch(grouped.data(), (int)grouped.size(), dtype, static_cast<cudaStream_t>(stream));
+  return syrk_route(Entry::kBatch, probs, n, dtype, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int vlm_syrk_accum_simt(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
@@ -249,13 +269,10 @@ extern "C" int vlm_syrk_pair_schedule_host(int64_t rows, int d, int elem_bytes, 
                                            int32_t* off_out, int off_cap, int* ncluster_out) {
   VLM_REQUIRE(rows > 0 && d > 0 && (elem_bytes == 1 || elem_bytes == 2 || elem_bytes == 4) && nsm > 1 && ncluster_out,
               VLM_ERR_INVALID_ARG, "vlm_syrk_pair_schedule_host: bad arguments");
-  const int bk = 128 / elem_bytes;
+  const int bk = elem_bytes == 1 ? 32 : 128 / elem_bytes;  // int8: the 32-row chunks of the int8 schedule
   std::vector<int32_t> flat;
   std::vector<int> off;
-  if (elem_bytes == 1)
-    build_syrk_i8_schedule_host((rows + 31) / 32, d, nsm, &flat, &off);
-  else
-    build_syrk_pair_schedule_host((rows + bk - 1) / bk, d, nsm, &flat, &off);
+  syrk_schedule_host((rows + bk - 1) / bk, d, nsm, elem_bytes == 1, &flat, &off);
   *ncluster_out = (int)off.size() - 1;
   VLM_REQUIRE((int)flat.size() <= 4 * cap && (int)off.size() <= off_cap, VLM_ERR_INVALID_ARG,
               "vlm_syrk_pair_schedule_host: output capacity too small (%d segments)", (int)flat.size() / 4);

@@ -93,11 +93,35 @@ __device__ __forceinline__ void tma_load_2d(const CUtensorMap* tm, uint64_t* bar
       ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
-__device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* tm, const void* smem_src, int c0, int c1) {
-  asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(tm)),
-               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
-               : "memory");
+// Bulk-tensor store / reduce-add (.add) of a 2-D box from shared memory, completed as a bulk group.  HINT: the writes
+// carry the L2 cache policy `pol` (createpolicy).
+template <bool HINT = false>
+__device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, const void* smem_src, int c0, int c1,
+                                             uint64_t pol = 0) {
+  if constexpr (HINT)
+    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3}], [%1], %4;" ::"l"(
+                     reinterpret_cast<uint64_t>(tm)),
+                 "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "l"(pol)
+                 : "memory");
+  else
+    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
+                     reinterpret_cast<uint64_t>(tm)),
+                 "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
+                 : "memory");
+}
+template <bool HINT = false>
+__device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* tm, const void* smem_src, int c0, int c1,
+                                                  uint64_t pol = 0) {
+  if constexpr (HINT)
+    asm volatile(
+        "cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group.L2::cache_hint [%0, {%2, %3}], [%1], %4;"
+        ::"l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "l"(pol)
+        : "memory");
+  else
+    asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
+                     reinterpret_cast<uint64_t>(tm)),
+                 "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
+                 : "memory");
 }
 __device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>

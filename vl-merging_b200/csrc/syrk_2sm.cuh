@@ -117,30 +117,48 @@ __device__ __forceinline__ void umma2(uint32_t d_tmem, uint64_t adesc, uint64_t 
   }
 }
 
+// Epilogue of the CTA-pair kernels: one slab of this CTA's rows of segment seg's tile, staged in shared memory at buf,
+// leaves for G at (col, row).  DET (deterministic mode, syrk_det.cu): tm describes the slot workspace instead, where
+// the tile's origin (256 sa, 256 sb) lies at row 256 * slot, column 0.  The segment that opens the slot stores, later
+// segments of this cluster on the same tile add.  Before adding, wait for COMPLETION (not just the source reads) of
+// every earlier bulk operation of this thread, the previous store / reduce-add into this slot among them: PTX ISA,
+// cp.async.bulk.wait_group — without .read, the wait lasts until the bulk async-groups are complete, writes to their
+// destinations included.  The adds into a slot are then in segment order.  HINT: the writes carry the L2 policy pol.
+template <bool DET, bool HINT>
+__device__ __forceinline__ void emit_slab(const CUtensorMap* tm, const void* buf, const PairSeg& seg, int col, int row,
+                                          bool first_slab, uint64_t pol) {
+  if constexpr (DET) {
+    col -= 256 * seg.sb;
+    row += 256 * ((seg.slot >> 1) - seg.sa);
+    if (seg.slot & 1) {
+      if (first_slab) bulk_wait_group<0>();
+      tma_reduce_add_2d<HINT>(tm, buf, col, row, pol);
+    } else {
+      tma_store_2d<HINT>(tm, buf, col, row, pol);
+    }
+  } else {
+    tma_reduce_add_2d<HINT>(tm, buf, col, row, pol);
+  }
+  bulk_commit_group();
+}
+
 // BATCH = false: one problem, tensor maps in kernel parameters.  BATCH = true: the segments of several problems
 // (e.g. all Grams of the text tower of one forward) share the grid; tensor maps live in global memory (`maps`:
-// [2*pid] = X, [2*pid+1] = G), written by the host before the launch.  SPLIT: tm_x is the 4-D {hi, lo} map (see header); cps is ignored.
+// [2*pid] = X, [2*pid+1] = G), written by the host before the launch.  Either way every segment names its problem's
+// width and chunks per row segment.  SPLIT: tm_x is the 4-D {hi, lo} map (see header), which has no row segments.
 // DET (deterministic mode, syrk_det.cu): the G map (tm_g1, or every maps[2*pid+1]) describes the slot workspace, fp32
-// {256 columns, slots * 256 rows}, and the segments are BatchSegs whose `slot` says where the partial goes.
+// {256 columns, slots * 256 rows}, and each segment's `slot` says where its partial goes (emit_slab).
 template <int ELEM_BYTES, int FMT, bool BATCH, bool SPLIT, bool DET>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 syrk_2sm_kernel(const __grid_constant__ CUtensorMap tm_x1, const __grid_constant__ CUtensorMap tm_g1,
-                const CUtensorMap* __restrict__ maps, const void* __restrict__ segs_raw,
-                const int* __restrict__ seg_off, int d1, int cps1, int l2_hints) {
+                const CUtensorMap* __restrict__ maps, const PairSeg* __restrict__ segs,
+                const int* __restrict__ seg_off) {
   using G = Geo2<ELEM_BYTES, SPLIT>;
-  using Seg = typename std::conditional<BATCH || DET, BatchSeg, PairSeg>::type;
-  const Seg* __restrict__ segs = static_cast<const Seg*>(segs_raw);
-  auto map_x = [&](const Seg& sg) -> const CUtensorMap* {
+  auto map_x = [&](const PairSeg& sg) -> const CUtensorMap* {
     if constexpr (BATCH) return maps + 2 * sg.pid; else return &tm_x1;
   };
-  auto map_g = [&](const Seg& sg) -> const CUtensorMap* {
+  auto map_g = [&](const PairSeg& sg) -> const CUtensorMap* {
     if constexpr (BATCH) return maps + 2 * sg.pid + 1; else return &tm_g1;
-  };
-  auto cols_of = [&](const Seg& sg) -> int {
-    if constexpr (BATCH) return sg.d; else return d1;
-  };
-  auto cps_of = [&](const Seg& sg) -> int {
-    if constexpr (SPLIT) return 0; else if constexpr (BATCH) return sg.cps; else return cps1;
   };
   constexpr int kRows = G::BK;
   constexpr int kBlk = kBlockBytes;
@@ -190,10 +208,10 @@ syrk_2sm_kernel(const __grid_constant__ CUtensorMap tm_x1, const __grid_constant
     int stage = 0;
     uint32_t phase = 0;
     int cur_pid = -1;
-    const uint64_t pol_x = l2_policy(l2_hints & 3);
+    const uint64_t pol_x = l2_evict_normal();
     const uint32_t full0 = mapa_rank(smem_u32(full), 0);
     for (int s = seg_begin; s < seg_end; ++s) {
-      const Seg seg = segs[s];
+      const PairSeg seg = segs[s];
       const CUtensorMap* tm_x = map_x(seg);
       if constexpr (BATCH) {
         if (seg.pid != cur_pid) {
@@ -205,7 +223,7 @@ syrk_2sm_kernel(const __grid_constant__ CUtensorMap tm_x1, const __grid_constant
       const int a_group = (2 * seg.sa + (int)rank) * G::GB;
       const int b_group = (2 * seg.sb + (int)rank) * G::GB;
       const uint32_t bytes_pair = (diag ? 2u : 4u) * kBlk;   // both CTAs: B (+ A) block each
-      const int cps = cps_of(seg);
+      const int cps = SPLIT ? 0 : seg.cps;
       int xseg = cps > 0 ? seg.k0 / cps : 0;
       int kin = seg.k0 - xseg * cps;
       for (int k = seg.k0; k < seg.k1; ++k) {
@@ -242,7 +260,7 @@ syrk_2sm_kernel(const __grid_constant__ CUtensorMap tm_x1, const __grid_constant
     constexpr uint32_t kDescLo = (uint32_t)((G::BOX_BYTES >> 4) & 0x3FFF) << 16;
     constexpr uint32_t idesc = make_idesc2(FMT, 256);
     for (int s = seg_begin; s < seg_end; ++s) {
-      const Seg seg = segs[s];
+      const PairSeg seg = segs[s];
       const int sa_t = __shfl_sync(0xffffffffu, seg.sa, 0), sb_t = __shfl_sync(0xffffffffu, seg.sb, 0);
       const int k0 = __shfl_sync(0xffffffffu, seg.k0, 0), k1 = __shfl_sync(0xffffffffu, seg.k1, 0);
       // diagonal super-tile: each CTA's A block IS its B block (one load); the pair forms all four blocks
@@ -293,12 +311,12 @@ syrk_2sm_kernel(const __grid_constant__ CUtensorMap tm_x1, const __grid_constant
     uint32_t acc_phase = 0;
     uint32_t slab_counter = 0;
     int cur_pid = -1;
-    const uint64_t pol_g = l2_policy((l2_hints >> 2) & 3);
+    const uint64_t pol_g = l2_evict_last();
     const uint32_t tempty0 = mapa_rank(smem_u32(tempty), 0);
     for (int s = seg_begin; s < seg_end; ++s) {
-      const Seg seg = segs[s];
+      const PairSeg seg = segs[s];
       const CUtensorMap* tm_g = map_g(seg);
-      const int d = cols_of(seg);
+      const int d = seg.d;
       if constexpr (BATCH) {
         if (epi_tid == 0 && seg.pid != cur_pid) {
           tensormap_acquire(tm_g);
@@ -332,25 +350,7 @@ syrk_2sm_kernel(const __grid_constant__ CUtensorMap tm_x1, const __grid_constant
         }
         fence_proxy_async_smem();
         named_bar_sync(1, 128);
-        if (epi_tid == 0) {
-          if constexpr (DET) {
-            // this CTA's 128 rows of the slot: the segment that opens the slot stores, later segments of this
-            // cluster on the same tile add.  Before adding, wait for COMPLETION (not just the source reads) of every
-            // earlier bulk operation of this thread, the previous store / reduce-add into this slot among them: PTX
-            // ISA, cp.async.bulk.wait_group — without .read, the wait lasts until the bulk async-groups are complete,
-            // writes to their destinations included.  The adds into a slot are then in segment order.
-            const int srow = (seg.slot >> 1) * 256 + (int)rank * 128, scol = n_off * 128 + sl * 32;
-            if (seg.slot & 1) {
-              if (sl == 0) bulk_wait_group<0>();
-              tma_reduce_add_2d_hint(tm_g, buf, scol, srow, pol_g);
-            } else {
-              tma_store_2d_hint(tm_g, buf, scol, srow, pol_g);
-            }
-          } else {
-            tma_reduce_add_2d_hint(tm_g, buf, col0 + sl * 32, row0, pol_g);
-          }
-          bulk_commit_group();
-        }
+        if (epi_tid == 0) emit_slab<DET, true>(tm_g, buf, seg, col0 + sl * 32, row0, sl == 0, pol_g);
         ++slab_counter;
       }
       tc_fence_before();

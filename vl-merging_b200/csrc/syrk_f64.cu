@@ -16,7 +16,6 @@
 // small Grams fill the GPU; every CTA adds its tile with red.global.add.f64 — the split-K reduction and the `+=`
 // across hook calls in one mechanism, like the TMA reduce-add of the tcgen05 kernels.
 #include <algorithm>
-#include <vector>
 
 #include "common.cuh"
 #include "syrk.h"
@@ -174,36 +173,20 @@ int launch_f64(const T* x, int64_t rows, int d, int64_t ldx, int64_t seg_rows, i
   const bool vec = (reinterpret_cast<uintptr_t>(x) & 15) == 0 && ldx % ev == 0 && seg_stride % ev == 0 && d % ev == 0;
   dim3 grid((unsigned)tiles, (unsigned)pieces);
   const int smem = (int)sizeof(F64Smem<T>);
-  if (deterministic_mode()) {
-    // tile t (row-major over the block-upper triangle, as the kernel numbers them): slots t * pieces .. + pieces
-    std::vector<DetItem> items;
-    for (int bi = 0, t = 0; bi < nb; ++bi)
-      for (int bj = bi; bj < nb; ++bj, ++t)
-        items.push_back({0, d, bi * FT, bj * FT, 0, (int)(t * pieces), (int)((t + 1) * pieces)});
-    void* ws = nullptr;
-    DetItem* d_items = nullptr;
-    if (int rc = det_workspace((size_t)tiles * pieces * FT * FT * sizeof(double), &items, stream, &ws, &d_items)) return rc;
-    auto kernel = vec ? syrk_f64_kernel<T, true, true> : syrk_f64_kernel<T, true, false>;
-    VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    kernel<<<grid, 512, smem, stream>>>(x, rows, d, ldx, seg_rows, seg_stride, static_cast<double*>(ws), 0, nb, rpp);
+  const bool det = deterministic_mode();
+  auto kernel = det ? (vec ? syrk_f64_kernel<T, true, true> : syrk_f64_kernel<T, true, false>)
+                    : (vec ? syrk_f64_kernel<T, false, true> : syrk_f64_kernel<T, false, false>);
+  VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  auto launch = [&](void* ws) -> int {
+    kernel<<<grid, 512, smem, stream>>>(x, rows, d, ldx, seg_rows, seg_stride, ws ? static_cast<double*>(ws) : g,
+                                        ws ? 0 : ldg, nb, rpp);
     VLM_CUDA(cudaGetLastError());
     count_launch();
-    if (int rc = det_reduce_launch(d_items, (int)items.size(), FT, true, ws, g, ldg, nullptr, stream)) return rc;
-    VLM_CUDA(cudaFreeAsync(ws, stream));
     return 0;
-  }
-  if (vec) {
-    auto kernel = syrk_f64_kernel<T, false, true>;
-    VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    kernel<<<grid, 512, smem, stream>>>(x, rows, d, ldx, seg_rows, seg_stride, g, ldg, nb, rpp);
-  } else {
-    auto kernel = syrk_f64_kernel<T, false, false>;
-    VLM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    kernel<<<grid, 512, smem, stream>>>(x, rows, d, ldx, seg_rows, seg_stride, g, ldg, nb, rpp);
-  }
-  VLM_CUDA(cudaGetLastError());
-  count_launch();
-  return 0;
+  };
+  if (!det) return launch(nullptr);
+  // tile t (row-major over the block-upper triangle, as the kernel numbers them): slots t * pieces .. + pieces
+  return det_grid_launch(d, FT, (int)pieces, 0, true, g, ldg, stream, launch);
 }
 
 }  // namespace

@@ -74,36 +74,23 @@ __device__ __forceinline__ void tmem_ld_32x32b_x16(uint32_t taddr, uint32_t (&v)
       : "r"(taddr)
       : "memory");
 }
-__device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* tm, const void* smem_src, int c0, int c1) {
-  asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(tm)),
-               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
-               : "memory");
-}
 // 2^e as a double, from its exponent bits (|e| < 1022: column exponents come from fp32 maxima); NaN for a poisoned
 // column (exponent kI8Poison, minus whatever the caller subtracted from it)
 __device__ __forceinline__ double i8_pow2(int e) {
   return e < -(1 << 19) ? __longlong_as_double(0x7ff8000000000000ll) : __hiloint2double((1023 + e) << 20, 0);
 }
 
-// segs: PairSeg with the phase (0: groups 4 and 3, 1: groups 2 and 1, 2: group 0) in bits 16.. of sb; k in 32-row chunks
+// segs: k in 32-row chunks, phase 0 (groups 4 and 3), 1 (groups 2 and 1) or 2 (group 0), width d; cps is always 0
 // tm_g: G as a 2-D fp64 tensor, box 16 columns x 128 rows (the epilogue's TMA reduce-adds)
-// DET (deterministic mode, syrk_det.cu): segs are BatchSegs with a workspace `slot`, and tm_g describes the slot
-// workspace, fp64 {256 columns, slots * 256 rows}.  The phases a cluster runs on one tile chain into one slot.
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, const void* smem_src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(tm)),
-               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
-               : "memory");
-}
+// DET (deterministic mode, syrk_det.cu): tm_g describes the slot workspace, fp64 {256 columns, slots * 256 rows}, and
+// each segment's `slot` says where its partial goes (emit_slab).  The phases a cluster runs on one tile chain into one
+// slot.
 template <bool DET>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constant__ CUtensorMap tm_p1,
                  const __grid_constant__ CUtensorMap tm_p2, const __grid_constant__ CUtensorMap tm_g,
-                 const void* __restrict__ segs_raw,
-                 const int* __restrict__ seg_off, int d, const __grid_constant__ I8Args args) {
-  using Seg = typename std::conditional<DET, BatchSeg, PairSeg>::type;
-  const Seg* __restrict__ segs = static_cast<const Seg*>(segs_raw);
+                 const PairSeg* __restrict__ segs, const int* __restrict__ seg_off,
+                 const __grid_constant__ I8Args args) {
   constexpr int kBlk = kBlockBytes;       // one operand of a stage
   constexpr int kNS = k2Stages;
   constexpr int kStageB = k2StageBytes;   // [A][B]
@@ -150,15 +137,15 @@ syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constan
     // ===== TMA producer (both CTAs): one box for its own A block, one for its own half of B =====
     int stage = 0;
     uint32_t phase = 0;
-    const uint64_t pol_x = l2_policy(0);
+    const uint64_t pol_x = l2_evict_normal();
     const uint32_t full0 = mapa_rank(smem_u32(full), 0);
     for (int s = seg_begin; s < seg_end; ++s) {
-      const Seg seg = segs[s];
-      const int sb_t = seg.sb & 0xFFFF, ph = seg.sb >> 16;
-      const bool diag = seg.sa == sb_t;
+      const PairSeg seg = segs[s];
+      const int ph = seg.phase;
+      const bool diag = seg.sa == seg.sb;
       const CUtensorMap* tm = ph == 0 ? &tm_p0 : ph == 1 ? &tm_p1 : &tm_p2;
       const int a_group = 2 * seg.sa + (int)rank;
-      const int b_group = 2 * sb_t + (int)rank;
+      const int b_group = 2 * seg.sb + (int)rank;
       const uint32_t bytes_pair = (diag ? 2u : 4u) * (ph == 1 ? 3u * kI8PlaneBytes : (uint32_t)kBlk);
       for (int k = seg.k0; k < seg.k1; k += ph == 2 ? 4 : 1) {
         mbar_wait(&empty[stage], phase ^ 1);
@@ -184,11 +171,11 @@ syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constan
     constexpr uint32_t idesc = make_idesc_i8(256);
     constexpr uint32_t kP = kI8PlaneBytes >> 4;     // 32 rows of one plane, in descriptor units
     for (int s = seg_begin; s < seg_end; ++s) {
-      const Seg seg = segs[s];
-      const int sa_t = __shfl_sync(0xffffffffu, seg.sa, 0), sbw = __shfl_sync(0xffffffffu, seg.sb, 0);
+      const PairSeg seg = segs[s];
+      const int sa_t = __shfl_sync(0xffffffffu, seg.sa, 0), sb_t = __shfl_sync(0xffffffffu, seg.sb, 0);
       const int k0 = __shfl_sync(0xffffffffu, seg.k0, 0), k1 = __shfl_sync(0xffffffffu, seg.k1, 0);
-      const int ph = sbw >> 16;
-      const uint32_t a_off = (sa_t == (sbw & 0xFFFF)) ? kBlk : 0u;
+      const int ph = __shfl_sync(0xffffffffu, seg.phase, 0);
+      const uint32_t a_off = (sa_t == sb_t) ? kBlk : 0u;
       const uint32_t d_hi = tmem_base, d_lo = tmem_base + kAccCols;   // the higher / lower group of this phase
       mbar_wait(tempty, acc_phase ^ 1);
       tc_fence_after();
@@ -252,12 +239,12 @@ syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constan
       const uint32_t tempty0 = mapa_rank(smem_u32(tempty), 0);
       uint32_t slab_counter = 0;            // two slabs: the conversion of one overlaps the TMA engine's read of the other
       for (int s = seg_begin; s < seg_end; ++s) {
-        const Seg seg = segs[s];
-        const int sb_t = seg.sb & 0xFFFF, ph = seg.sb >> 16;
-        const bool diag = seg.sa == sb_t;
+        const PairSeg seg = segs[s];
+        const int ph = seg.phase, d = seg.d;
+        const bool diag = seg.sa == seg.sb;
         const int n_off = (diag && rank == 1) ? 1 : 0;   // peer on a diagonal tile: only block (2a+1, 2a+1)
         const int row0 = (2 * seg.sa + (int)rank) * 128;
-        const int col0 = (2 * sb_t + n_off) * 128;
+        const int col0 = (2 * seg.sb + n_off) * 128;
         const int grp = 4 - 2 * ph;                      // the group in accumulator 0 (the smaller scale of the phase)
         const bool two = ph != 2;
         mbar_wait(tfull, acc_phase);
@@ -290,22 +277,7 @@ syrk_i8x4_kernel(const __grid_constant__ CUtensorMap tm_p0, const __grid_constan
           }
           fence_proxy_async_smem();
           named_bar_sync(1, 128);
-          if (epi_tid == 0) {
-            if constexpr (DET) {
-              // as in syrk_2sm_kernel: the segment that opens the slot stores, a later one first waits for the
-              // completion (writes included: cp.async.bulk.wait_group without .read) of the earlier ones, then adds
-              const int srow = (seg.slot >> 1) * 256 + (int)rank * 128, scol = n_off * 128 + sl * 16;
-              if (seg.slot & 1) {
-                if (sl == 0) bulk_wait_group<0>();
-                tma_reduce_add_2d(&tm_g, buf, scol, srow);
-              } else {
-                tma_store_2d(&tm_g, buf, scol, srow);
-              }
-            } else {
-              tma_reduce_add_2d(&tm_g, buf, c0, row0);
-            }
-            bulk_commit_group();
-          }
+          if (epi_tid == 0) emit_slab<DET, false>(&tm_g, buf, seg, c0, row0, sl == 0, 0);
           ++slab_counter;
         }
         tc_fence_before();

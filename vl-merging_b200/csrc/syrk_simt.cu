@@ -2,8 +2,6 @@
 // cannot address).
 // Same contract as the tensor-core kernel: G[r][c] += sum_k X[k][r]*X[k][c] for c >= r
 // (src/cache_gram_matrices.py:246-254 of the reference computes the full fp64 matrix).
-#include <vector>
-
 #include "common.cuh"
 #include "syrk.h"
 
@@ -80,6 +78,18 @@ syrk_simt_kernel(const T* __restrict__ x, int64_t rows, int d, int64_t ldx, floa
     }
 }
 
+template <bool DET>
+void launch_simt(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg, dim3 grid,
+                 cudaStream_t stream) {
+  if (dtype == VLM_F32)
+    syrk_simt_kernel<float, DET><<<grid, 256, 0, stream>>>(static_cast<const float*>(x), rows, d, ldx, g, ldg);
+  else if (dtype == VLM_BF16)
+    syrk_simt_kernel<__nv_bfloat16, DET>
+        <<<grid, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(x), rows, d, ldx, g, ldg);
+  else
+    syrk_simt_kernel<__half, DET><<<grid, 256, 0, stream>>>(static_cast<const __half*>(x), rows, d, ldx, g, ldg);
+}
+
 }  // namespace
 
 int syrk_simt_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx, float* g, int64_t ldg,
@@ -88,38 +98,18 @@ int syrk_simt_launch(const void* x, int dtype, int64_t rows, int d, int64_t ldx,
   const int nz = (int)((rows + kSplit - 1) / kSplit);
   VLM_REQUIRE(nz <= 65535, VLM_ERR_INVALID_ARG, "vlm_syrk_accum_simt: rows too large");
   dim3 grid(nt, nt, nz);
-  if (deterministic_mode()) {
-    // upper tile t (row-major): slots t * nz .. + nz
-    std::vector<DetItem> items;
-    for (int bi = 0, t = 0; bi < nt; ++bi)
-      for (int bj = bi; bj < nt; ++bj, ++t) items.push_back({0, d, bi * kTile, bj * kTile, 2, t * nz, (t + 1) * nz});
-    void* ws = nullptr;
-    DetItem* d_items = nullptr;
-    if (int rc = det_workspace(items.size() * nz * kTile * kTile * sizeof(float), &items, stream, &ws, &d_items)) return rc;
-    float* slots = static_cast<float*>(ws);
-    if (dtype == VLM_F32)
-      syrk_simt_kernel<float, true><<<grid, 256, 0, stream>>>(static_cast<const float*>(x), rows, d, ldx, slots, 0);
-    else if (dtype == VLM_BF16)
-      syrk_simt_kernel<__nv_bfloat16, true>
-          <<<grid, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(x), rows, d, ldx, slots, 0);
+  auto launch = [&](void* ws) -> int {
+    if (ws)
+      launch_simt<true>(x, dtype, rows, d, ldx, static_cast<float*>(ws), 0, grid, stream);
     else
-      syrk_simt_kernel<__half, true><<<grid, 256, 0, stream>>>(static_cast<const __half*>(x), rows, d, ldx, slots, 0);
+      launch_simt<false>(x, dtype, rows, d, ldx, g, ldg, grid, stream);
     VLM_CUDA(cudaGetLastError());
     count_launch();
-    if (int rc = det_reduce_launch(d_items, (int)items.size(), kTile, false, ws, g, ldg, nullptr, stream)) return rc;
-    VLM_CUDA(cudaFreeAsync(ws, stream));
     return 0;
-  }
-  if (dtype == VLM_F32)
-    syrk_simt_kernel<float, false><<<grid, 256, 0, stream>>>(static_cast<const float*>(x), rows, d, ldx, g, ldg);
-  else if (dtype == VLM_BF16)
-    syrk_simt_kernel<__nv_bfloat16, false>
-        <<<grid, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(x), rows, d, ldx, g, ldg);
-  else
-    syrk_simt_kernel<__half, false><<<grid, 256, 0, stream>>>(static_cast<const __half*>(x), rows, d, ldx, g, ldg);
-  VLM_CUDA(cudaGetLastError());
-  count_launch();
-  return 0;
+  };
+  if (!deterministic_mode()) return launch(nullptr);
+  // upper tile t (row-major): slots t * nz .. + nz
+  return det_grid_launch(d, kTile, nz, 2, false, g, ldg, stream, launch);
 }
 
 }  // namespace vlm
