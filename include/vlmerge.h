@@ -185,6 +185,12 @@ typedef struct vlm_sym_span {
 } vlm_sym_span;
 int vlm_sym_allreduce_multimem(void* multicast_base, const vlm_sym_span* spans, int n, int dtype, int rank, int world,
                                void* stream);
+/* The reduce-scatter form of the same exchange: each rank passes only the spans it owns (every span on exactly one
+ * rank), reads them with multimem.ld_reduce.add and stores the sums with plain stores into its own copy at
+ * local_base + offset_bytes (16-byte aligned); nothing is broadcast, and the other ranks' copies are left as they
+ * were.  Same alignment rules and barriers as vlm_sym_allreduce_multimem; the lower triangles follow locally. */
+int vlm_sym_reduce_multimem(void* multicast_base, void* local_base, const vlm_sym_span* spans, int n, int dtype,
+                            void* stream);
 
 /* Host-only view of the work decomposition of vlm_syrk_accum's CTA-pair kernel for (rows, d) on a device with nsm SMs
  * (elem_bytes 4 = f32, 2 = bf16/f16): writes segments as 4 int32 each {super_row, super_col (256-column units),

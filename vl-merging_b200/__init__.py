@@ -15,7 +15,7 @@ from ._lib import VlmError, build  # noqa: F401
 from .checkpoint import load_checkpoint, modify_checkpoint_vlmo, save_checkpoint  # noqa: F401
 from .gram import GramCache, cache_gram_matrices  # noqa: F401
 from .irtr import irtr_features, irtr_recall, irtr_recall_fused, sim_topk  # noqa: F401
-from .merge import Merger, independent, merge_weights, regmean, sum_task_vectors  # noqa: F401
+from .merge import Merger, independent, merge_weights, regmean, regmean_gram_owners, sum_task_vectors  # noqa: F401
 from .model import VLMo, init_synthetic_, synthetic_batch, vlmo_config  # noqa: F401
 
 __version__ = "0.1.0"

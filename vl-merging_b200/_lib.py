@@ -96,6 +96,7 @@ SIGNATURES = {
     "vlm_sym_pack_upper_batch": (c_int, [POINTER(SymItem), c_int, c_int, c_void_p]),
     "vlm_sym_unpack_batch": (c_int, [POINTER(SymItem), c_int, c_int, c_void_p]),
     "vlm_sym_allreduce_multimem": (c_int, [c_void_p, POINTER(SymSpan), c_int, c_int, c_int, c_int, c_void_p]),
+    "vlm_sym_reduce_multimem": (c_int, [c_void_p, c_void_p, POINTER(SymSpan), c_int, c_int, c_void_p]),
     "vlm_sym_mirror_batch": (c_int, [POINTER(SymItem), c_int, c_int, c_void_p]),
     "vlm_syrk_pair_schedule_host": (c_int, [c_int64, c_int, c_int, c_int, POINTER(c_int32), c_int, POINTER(c_int32),
                                             c_int, POINTER(c_int)]),

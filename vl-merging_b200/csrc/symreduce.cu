@@ -14,6 +14,9 @@
 // pack + reduce-scatter + all-gather + unpack in one launch; every element of the upper triangles crosses NVLink once
 // in each direction, and every rank ends up with bit-identical Grams (one owner computes each value).  The launch must be bracketed by cross-rank barriers (GramCache does that with the
 // symmetric-memory handle's barrier): all ranks' SYRK launches before, nobody reads a Gram until all stores landed.
+//
+// vlm_sym_reduce_multimem is the reduce-scatter form (GramCache.reduce_scatter): every Gram has one owner rank, which
+// reads it the same way and keeps the sum in its own arena only (plain stores, no broadcast).
 #include <vector>
 
 #include "common.cuh"
@@ -69,28 +72,38 @@ __device__ __forceinline__ SpanDev locate_band(const SpanDev* __restrict__ spans
 // switch; the lower triangles are mirrored locally afterwards (vlm_sym_mirror_batch), so every element of the
 // upper triangles crosses NVLink once in each direction.  (A first version dealt 32 x 32 tiles to the ranks: 128-byte
 // runs, 1.9 ms for the 538 MB of VLMo-base at N = 2.)
-template <typename T, typename V, int VE>   // V: the access type (float4 / double), VE elements each
+//
+// kLocal (vlm_sym_reduce_multimem, the reduce-scatter form): the caller passes only the spans it owns, so every band is
+// its own; the sums go to local_base + offset with plain stores instead of the multimem.st broadcast.
+template <typename T, typename V, int VE, bool kLocal>   // V: the access type (float4 / double), VE elements each
 __global__ void __launch_bounds__(256) sym_allreduce_mc_kernel(uint8_t* __restrict__ mc_base, const SpanDev* __restrict__ spans,
-                                                                int n, int rank, int world) {
+                                                                int n, int rank, int world, uint8_t* __restrict__ local_base) {
   int item, bi;
   const SpanDev sp = locate_band(spans, n, blockIdx.x, &item, &bi);
-  if ((item + bi) % world != rank) return;
+  if (!kLocal && (item + bi) % world != rank) return;
   const int d = sp.d;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   T* g = reinterpret_cast<T*>(mc_base + sp.offset_bytes);
+  T* out = kLocal ? reinterpret_cast<T*>(local_base + sp.offset_bytes) : g;
   constexpr int kStep = 32 * VE;            // elements per warp instruction
   for (int rr = warp; rr < 32; rr += 8) {
     const int r = bi * 32 + rr;
     if (r >= d) break;
     T* row = g + (int64_t)r * sp.ld;
+    T* out_row = out + (int64_t)r * sp.ld;
     for (int c = bi * 32 + lane * VE; c < d; c += 4 * kStep) {
       V s[4];
 #pragma unroll
       for (int u = 0; u < 4; ++u)
         if (c + u * kStep < d) s[u] = mc_ld_reduce(row + c + u * kStep);   // d % VE == 0 (host): a vector is in or out
 #pragma unroll
-      for (int u = 0; u < 4; ++u)
-        if (c + u * kStep < d) mc_st(row + c + u * kStep, s[u]);
+      for (int u = 0; u < 4; ++u) {
+        if (c + u * kStep >= d) continue;
+        if (kLocal)
+          *reinterpret_cast<V*>(out_row + c + u * kStep) = s[u];
+        else
+          mc_st(row + c + u * kStep, s[u]);
+      }
     }
   }
 }
@@ -119,24 +132,43 @@ int upload_spans(const vlm_sym_span* spans, int n, int dtype, const char* who, c
 
 using namespace vlm;
 
-extern "C" int vlm_sym_allreduce_multimem(void* multicast_base, const vlm_sym_span* spans, int n, int dtype, int rank,
-                                          int world, void* stream) {
-  VLM_REQUIRE(multicast_base != nullptr && spans != nullptr && n >= 0 && world >= 1 && rank >= 0 && rank < world,
-              VLM_ERR_INVALID_ARG, "vlm_sym_allreduce_multimem: bad arguments");
-  VLM_REQUIRE(dtype == VLM_F32 || dtype == VLM_F64, VLM_ERR_INVALID_ARG,
-              "vlm_sym_allreduce_multimem: dtype must be VLM_F32 or VLM_F64 (got %d)", dtype);
+// Both entry points: argument checks, span upload, one launch.  kLocal: see sym_allreduce_mc_kernel.
+template <bool kLocal>
+static int launch_mc(const char* who, void* multicast_base, void* local_base, const vlm_sym_span* spans, int n, int dtype,
+                     int rank, int world, void* stream) {
+  VLM_REQUIRE(dtype == VLM_F32 || dtype == VLM_F64, VLM_ERR_INVALID_ARG, "%s: dtype must be VLM_F32 or VLM_F64 (got %d)",
+              who, dtype);
   if (n == 0) return 0;
   if (int rc = require_sm100()) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   SpanDev* dev = nullptr;
   int64_t bands = 0;
-  if (int rc = upload_spans(spans, n, dtype, "vlm_sym_allreduce_multimem", s, &dev, &bands)) return rc;
+  if (int rc = upload_spans(spans, n, dtype, who, s, &dev, &bands)) return rc;
+  uint8_t* mc = static_cast<uint8_t*>(multicast_base);
+  uint8_t* local = static_cast<uint8_t*>(local_base);
   if (dtype == VLM_F32)
-    sym_allreduce_mc_kernel<float, float4, 4><<<(unsigned)bands, 256, 0, s>>>(static_cast<uint8_t*>(multicast_base), dev, n, rank, world);
+    sym_allreduce_mc_kernel<float, float4, 4, kLocal><<<(unsigned)bands, 256, 0, s>>>(mc, dev, n, rank, world, local);
   else
-    sym_allreduce_mc_kernel<double, double, 1><<<(unsigned)bands, 256, 0, s>>>(static_cast<uint8_t*>(multicast_base), dev, n, rank, world);
+    sym_allreduce_mc_kernel<double, double, 1, kLocal><<<(unsigned)bands, 256, 0, s>>>(mc, dev, n, rank, world, local);
   VLM_CUDA(cudaGetLastError());
   VLM_CUDA(cudaFreeAsync(dev, s));
   count_launch();
   return 0;
+}
+
+extern "C" int vlm_sym_allreduce_multimem(void* multicast_base, const vlm_sym_span* spans, int n, int dtype, int rank,
+                                          int world, void* stream) {
+  VLM_REQUIRE(multicast_base != nullptr && spans != nullptr && n >= 0 && world >= 1 && rank >= 0 && rank < world,
+              VLM_ERR_INVALID_ARG, "vlm_sym_allreduce_multimem: bad arguments");
+  return launch_mc<false>("vlm_sym_allreduce_multimem", multicast_base, nullptr, spans, n, dtype, rank, world, stream);
+}
+
+extern "C" int vlm_sym_reduce_multimem(void* multicast_base, void* local_base, const vlm_sym_span* spans, int n, int dtype,
+                                       void* stream) {
+  VLM_REQUIRE(multicast_base != nullptr && local_base != nullptr && spans != nullptr && n >= 0, VLM_ERR_INVALID_ARG,
+              "vlm_sym_reduce_multimem: bad arguments");
+  // the plain stores are as wide as the multimem loads: the local arena needs the same alignment as the multicast one
+  VLM_REQUIRE(reinterpret_cast<uintptr_t>(local_base) % 16 == 0, VLM_ERR_ALIGNMENT,
+              "vlm_sym_reduce_multimem: local_base must be 16-byte aligned");
+  return launch_mc<true>("vlm_sym_reduce_multimem", multicast_base, local_base, spans, n, dtype, 0, 1, stream);
 }

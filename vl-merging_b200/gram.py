@@ -11,7 +11,9 @@ hook_gram_input(module, input, output)       GramCache.hook_gram_input — same 
 registration loop (:278-281)                 GramCache.register(model, use_moe)
 torch.save(middle_representations, path)     GramCache.save(path): {name: fp64 CPU (d,d)} — the file
                                              regmean() loads (vilt_module.py:386)
-(absent: every DDP rank writes its own sums) GramCache.all_reduce(): ONE NCCL all-reduce of the packed upper triangles
+(absent: every DDP rank writes its own sums) GramCache.all_reduce(): ONE NCCL all-reduce of the packed upper triangles;
+                                             GramCache.reduce_scatter(owners): each Gram's sum on the rank whose
+                                             regmean(..., group=g) solves it only (ONE NCCL reduce-scatter)
 """
 import contextlib
 from collections import defaultdict
@@ -55,28 +57,36 @@ def select_hooked_modules(model, use_moe=True, all_keys=None):
             if any(name.endswith(k) for k in keys) and ".bias" not in name]
 
 
+def _same_everywhere(obj, group, device):
+    """Whether every rank of `group` passed an object with the same repr: one 16-byte all-reduce of a 56-bit digest (the
+    max of the digest and of its negation agree only if all digests are equal); the same answer on every rank."""
+    import hashlib
+
+    import torch.distributed as dist
+
+    if dist.get_backend(group) == "nccl" and torch.device(device).type != "cuda":
+        device = torch.device("cuda", torch.cuda.current_device())
+    elif dist.get_backend(group) != "nccl":
+        device = torch.device("cpu")
+    digest = int.from_bytes(hashlib.sha256(repr(obj).encode()).digest()[:7], "little")      # 56 bits: exact in int64
+    t = torch.tensor([digest, -digest], dtype=torch.int64, device=device)
+    dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
+    hi, neg_lo = t.tolist()
+    return hi == -neg_lo
+
+
 def agree_on_buffers(buffers, group=None, make=None, device=None):
     """Ranks may hold different sets of lazily created buffers (a module whose width was unknown at register() fires on
     some ranks only): agree on the union of (name, width) first and create zero buffers for the names missing
     locally, so every rank issues the same collectives on the same shapes.  Raises if two ranks disagree on a width.
     The common case — every rank holds the same set — costs one 16-byte all-reduce of a digest (max of the digest and
     of its complement agree only if all digests are equal); only a mismatch pays for the all_gather_object."""
-    import hashlib
-
     import torch.distributed as dist
 
     mine = sorted((n, int(g.shape[0])) for n, g in buffers.items())
     if device is None:
         device = next(iter(buffers.values())).device if buffers else torch.device("cpu")
-    if dist.get_backend(group) == "nccl" and torch.device(device).type != "cuda":
-        device = torch.device("cuda", torch.cuda.current_device())
-    elif dist.get_backend(group) != "nccl":
-        device = torch.device("cpu")
-    digest = int.from_bytes(hashlib.sha256(repr(mine).encode()).digest()[:7], "little")      # 56 bits: exact in int64
-    t = torch.tensor([digest, -digest], dtype=torch.int64, device=device)
-    dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)    # every rank takes part, with or without buffers
-    hi, neg_lo = t.tolist()
-    if hi == -neg_lo:                                         # max == min: the same set everywhere (same test on every rank)
+    if _same_everywhere(mine, group, device):    # every rank takes part, with or without buffers
         return [n for n, _ in mine]
     everyone = [None] * dist.get_world_size(group)
     dist.all_gather_object(everyone, mine, group=group)
@@ -202,6 +212,8 @@ class GramCache:
         self._side = torch.cuda.Stream(self.device) if side_stream else None
         self._side_keep = []   # activations a side-stream launch may still be reading
         self.deterministic = bool(torch.are_deterministic_algorithms_enabled() if deterministic is None else deterministic)
+        self.owners = None     # after reduce_scatter(): {name: rank} of the exchanged Grams; this rank holds its own only
+        self._rank = None      # this cache's rank in the reduce_scatter() group
 
     @contextlib.contextmanager
     def _mode(self):
@@ -229,6 +241,7 @@ class GramCache:
     __call__ = hook_gram_input
 
     def accumulate(self, name, x):
+        self._require_whole("accumulate")
         with self._mode():
             self._accumulate(name, x)
 
@@ -435,6 +448,7 @@ class GramCache:
         whole arena."""
         import torch.distributed as dist
 
+        self._require_whole("all_reduce")
         self.flush()
         if self.symmetric and packed:
             return self._all_reduce_multimem(group)
@@ -452,6 +466,118 @@ class GramCache:
         _lib.check(self._lib.vlm_sym_unpack_batch(items, len(live), self._sym_code, stream))
         self._finalized = True
         self.last_reduce_bytes = flat.numel() * flat.element_size()
+
+    def reduce_scatter(self, owners, group=None):
+        """Data-parallel calibration followed by a sharded regmean(..., group=group): sum each Gram over the ranks of
+        `group` onto its owner only.  owners: {Gram name: rank in group}, normally
+        regmean_gram_owners(state_dict, config, cache.live_names(), world, num_layers) with the arguments regmean will
+        get; it must name live Grams only, and live Grams it leaves out (ones no regmean problem reads) are not summed.
+        Plain caches: the owned upper triangles are packed by owner into [world x width] (width: the largest owner's
+        section; one vlm_sym_pack_upper_batch), ONE NCCL reduce-scatter, and this rank's section unpacked into its
+        Grams (one vlm_sym_unpack_batch): each rank sends (world - 1) / world of the buffer instead of the all-reduce's
+        2 (world - 1) / world, and unpacks only its own Grams.  Symmetric caches: one vlm_sym_reduce_multimem
+        launch over this rank's Grams between two cross-rank barriers, then their local mirror.
+        Afterwards the cache is scattered: `owners` records the map, this rank's own Grams hold the full symmetric
+        sums and gram() returns them; the other Grams, state_dict() / save() / save_packed(), all_reduce() and
+        further accumulation raise until reset().  live_names() is still the full agreed list on every rank."""
+        import torch.distributed as dist
+
+        self._require_whole("reduce_scatter")
+        self.flush()
+        group = group if group is not None else dist.group.WORLD
+        rank, world = dist.get_rank(group), dist.get_world_size(group)
+        names = agree_on_buffers(self.buffers, group,
+                                 lambda d: torch.zeros(d, d, dtype=self.dtype, device=self.device), device=self.device)
+        calls, rows = defaultdict(int, self.calls), defaultdict(int, self.rows)
+        _reduce_counts(self.buffers, names, calls, rows, group)
+        # every check that can fail comes before the cache's own counters change (the same outcome on every rank: the
+        # summed counters, the owner map and the arena are the same everywhere)
+        live = [n for n in names if calls[n] > 0]
+        if not _same_everywhere(sorted(owners.items()), group, self.device):
+            raise ValueError("GramCache.reduce_scatter: the ranks passed different owner maps (build it on every rank "
+                             "from the same state_dict, config and world, and the live names every rank holds)")
+        for n, r in owners.items():
+            if n not in live:
+                raise ValueError(f"GramCache.reduce_scatter: owner map names {n!r}, which is not a live Gram of this cache "
+                                 "(build the map from cache.live_names())")
+            if not isinstance(r, int) or not 0 <= r < world:
+                raise ValueError(f"GramCache.reduce_scatter: owner {r!r} of {n!r} is not a rank of a {world}-rank group")
+        owned = [n for n in live if n in owners]
+        if self.symmetric:
+            mc, spans = self._multicast_spans(owned, [n for n in owned if owners[n] == rank], group)
+        self.calls.update(calls)
+        self.rows.update(rows)
+        self.owners, self._rank = {n: owners[n] for n in owned}, rank
+        self._finalized = True
+        esz = 8 if self.dtype == torch.float64 else 4
+        mine = [n for n in owned if owners[n] == rank]
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        if self.symmetric:
+            with torch.cuda.device(self.device):
+                self._symm.barrier(channel=0)      # every rank's Gram launches have completed
+                _lib.check(self._lib.vlm_sym_reduce_multimem(mc, self._arenas[0].data_ptr(), spans, len(spans),
+                                                             self._sym_code, stream))
+                self._symm.barrier(channel=0)      # nobody reads a rank's arena any more
+                self._mirror(mine, stream)
+            self.last_reduce_bytes = sum(self.buffers[n].shape[0] * (self.buffers[n].shape[0] + 1) // 2 for n in mine) * esz
+            return
+        tri = {n: self.buffers[n].shape[0] * (self.buffers[n].shape[0] + 1) // 2 for n in owned}
+        order = sorted(owned, key=lambda n: self.owners[n])         # stable: live order inside each owner's section
+        section, offsets = [0] * world, []
+        for n in order:
+            offsets.append(section[self.owners[n]])
+            section[self.owners[n]] += tri[n]
+        width = max(section)
+        self.last_reduce_bytes = world * width * esz
+        if width == 0:
+            return
+        flat = torch.empty(world * width, dtype=self.dtype, device=self.device)    # padding is summed, never read
+        items = _lib.sym_items([self.buffers[n] for n in order], flat,
+                               [self.owners[n] * width + off for n, off in zip(order, offsets)])
+        _lib.check(self._lib.vlm_sym_pack_upper_batch(items, len(order), self._sym_code, stream))
+        out = torch.empty(width, dtype=self.dtype, device=self.device)
+        dist.reduce_scatter_tensor(out, flat, op=dist.ReduceOp.SUM, group=group)
+        items = _lib.sym_items([self.buffers[n] for n in mine], out)      # this rank's section, in the same order
+        _lib.check(self._lib.vlm_sym_unpack_batch(items, len(mine), self._sym_code, stream))
+
+    def _require_whole(self, what, name=None):
+        """Raise if this cache was reduce_scatter()ed (and `name`, when given, is not one of this rank's Grams)."""
+        if self.owners is None or (name is not None and self.owners.get(name) == self._rank):
+            return
+        raise RuntimeError(f"GramCache.{what}: this cache was reduce_scatter()ed, so this rank holds the summed Grams it "
+                           "owns only; pass the cache to regmean(..., gram_matrices=cache, group=...) with the same "
+                           "arguments as the owner map, use all_reduce() instead of reduce_scatter() for Gram files and "
+                           "state_dict(), or reset() it to calibrate again")
+
+    def _multicast_spans(self, names, mine, group):
+        """Checks of the multimem exchange and its spans: (multicast address, vlm_sym_span array of `mine`).  Every
+        Gram of `names` must lie in the one symmetric arena and meet the kernel's alignment rules, so every rank
+        raises or none does."""
+        import torch.distributed._symmetric_memory as symm_mem
+
+        if len(self._arenas) != 1:
+            raise RuntimeError("GramCache(symmetric=True): no symmetric arena (register() the model before calibrating)")
+        arena = self._arenas[0]
+        lo, hi = arena.data_ptr(), arena.data_ptr() + arena.numel() * arena.element_size()
+        for n in names:
+            g = self.buffers[n]
+            if not lo <= g.data_ptr() < hi:
+                raise RuntimeError("GramCache(symmetric=True): a Gram buffer lives outside the symmetric arena (a module "
+                                   "whose width was unknown at register()); use a plain cache (NCCL exchange) for this model")
+            if (g.data_ptr() - lo) % 16 or (self.dtype == torch.float32 and (g.shape[0] % 4 or g.stride(0) % 4)):
+                raise RuntimeError(f"GramCache(symmetric=True): Gram {n} of width {g.shape[0]} does not meet the multimem "
+                                   "alignment rules (16-byte offset; fp32 widths a multiple of 4); use a plain cache")
+        if self._symm is None:
+            self._symm = symm_mem.rendezvous(arena, group)          # collective: every rank, same order
+        mc = int(self._symm.multicast_ptr or 0)
+        if mc == 0:
+            raise RuntimeError("GramCache(symmetric=True): this system offers no multicast mapping (NVSwitch + driver "
+                               "support needed); use a plain cache (NCCL exchange)")
+        spans = (_lib.SymSpan * len(mine))()
+        for sp, n in zip(spans, mine):
+            g = self.buffers[n]
+            sp.offset_bytes, sp.d, sp.ld = g.data_ptr() - lo, g.shape[0], g.stride(0)
+        return mc, spans
 
     def _agree_on_live(self, group):
         """The first step of both exchanges: every rank agrees on the buffer set (creating zero buffers for names it
@@ -514,7 +640,8 @@ class GramCache:
         _lib.check(self._lib.vlm_sym_mirror_batch(items, len(names), self._sym_code, stream))
 
     def gram(self, name):
-        """Full symmetric fp32 Gram of one module, on the device."""
+        """Full symmetric fp32 Gram of one module, on the device (of a scattered cache: one this rank owns)."""
+        self._require_whole(f"gram({name!r})", name)
         self.finalize()
         return self.buffers[name]
 
@@ -522,6 +649,7 @@ class GramCache:
         """{module_name: (d,d) tensor} for every module that fired — by default fp64 CPU tensors, the
         format of the reference's Gram file, in the reference's insertion order (first-call order
         there; registration order here, which is the same for a sequential forward)."""
+        self._require_whole("state_dict")
         self.finalize()
         out = defaultdict(float)
         for name in self.live_names():
@@ -532,6 +660,7 @@ class GramCache:
 
     def save(self, path):
         """torch.save of the reference-format dict (src/cache_gram_matrices.py:349)."""
+        self._require_whole("save")
         torch.save(self.state_dict(), path)
 
     def save_packed(self, path):
@@ -549,6 +678,7 @@ class GramCache:
         self.calls.clear()
         self.rows.clear()
         self._finalized = True
+        self.owners = None
 
 
 def hook_gram_input_factory(cache):

@@ -64,6 +64,7 @@ def save_packed(grams, path, rows=None, calls=None, device=None, dtype=None):
         if dtype is None:
             dtype = grams.dtype
         cache = grams
+        cache._require_whole("save_packed")
         cache.flush()
         device = cache.device
         rows, calls = cache.rows, cache.calls

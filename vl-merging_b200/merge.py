@@ -492,10 +492,38 @@ def _regmean_linears(lib, state_dict, grams, lin_ops, mine, cost, alpha, device,
 
 
 def _as_gram_dict(grams):
+    """{name: Gram} of a dict or a GramCache (on its device).  Of a reduce-scattered cache every live name is listed,
+    so that every rank plans the same problems, but only the Grams this rank owns hold sums and may be read."""
     if hasattr(grams, "state_dict") and hasattr(grams, "buffers"):  # a GramCache: stay on the device, fp32
         grams.finalize()
         return {n: grams.buffers[n] for n in grams.live_names()}
     return grams
+
+
+def _regmean_cost(state_dict, op):
+    o, i = state_dict[op.regmean[0][0]].shape
+    return i * i * i // 3 + 2 * len(op.regmean) * o * i * i + 2 * o * i * i
+
+
+def _regmean_sharding(state_dict, config, gram_names, world, num_layers):
+    """regmean()'s plan and the cost-balanced ShardLayout of its linear problems over `world` ranks, plus the owner of
+    every Gram a problem reads: (ops, lin_ops, layout, {gram name: rank})."""
+    ops = plan_regmean(state_dict.keys(), gram_names, config, num_layers)
+    lin_ops = [op for op in ops if not op.passthrough and op.regmean is not None]
+    sizes = [int(state_dict[op.regmean[0][0]].numel()) for op in lin_ops]
+    layout = ShardLayout(sizes, world, cost=lambda i: _regmean_cost(state_dict, lin_ops[i]), align=1)
+    # plan_regmean gives every expert's linear its own Gram: each Gram has exactly one owner
+    owners = {gram: layout.owner[idx] for idx, op in enumerate(lin_ops) for _, gram in op.regmean}
+    return ops, lin_ops, layout, owners
+
+
+def regmean_gram_owners(state_dict, config, gram_names, world, num_layers=12):
+    """{Gram name: rank} — which rank's regmean(..., group=g) with a world of `world` ranks solves the one linear
+    problem that reads each Gram (qkv <- attn.{m}, proj <- attn.{m}.proj, fc1 / fc2 <- mlp.{m}.fc1 / fc2).  Grams
+    that no problem reads (the `v` / `l` Grams of the deep layers under a VQA config, for example) are not in the map.
+    Pass every rank's agreed live names (GramCache.live_names() after calibration) and the arguments regmean() will
+    get; GramCache.reduce_scatter(owners) then leaves each Gram's sum on its owner only."""
+    return _regmean_sharding(state_dict, config, gram_names, int(world), num_layers)[3]
 
 
 def regmean(state_dict, config, device=None, num_layers=12, group=None, stats=None, gram_matrices=None,
@@ -524,28 +552,27 @@ def regmean(state_dict, config, device=None, num_layers=12, group=None, stats=No
                       "calibrate with GramCache(precision='int8x4') (or 'fp64') for the reference's 1e-4",
                       RuntimeWarning, stacklevel=2)
     grams = _as_gram_dict(gram_matrices)
-    ops = plan_regmean(state_dict.keys(), grams.keys(), config, num_layers)
+    world = dist.get_world_size(group) if group is not None else 1
+    rank = dist.get_rank(group) if group is not None else 0
+    ops, lin_ops, lin_layout, owners = _regmean_sharding(state_dict, config, grams.keys(), world, num_layers)
+    scattered = getattr(gram_matrices, "owners", None)
+    if scattered is not None and (scattered != owners or gram_matrices._rank != rank):
+        raise ValueError("regmean: the GramCache was reduce_scatter()ed with a different owner map or rank than this "
+                         f"call's (world {world}, rank {rank}, num_layers {num_layers}, this config): every rank holds only its own Gram "
+                         "sums; scatter it with regmean_gram_owners() of the same arguments, or all_reduce() it")
     todo = [op for op in ops if not op.passthrough]
     mean_ops = [op for op in todo if op.regmean is None]
-    lin_ops = [op for op in todo if op.regmean is not None]
     out_device = _out_device(state_dict, todo, out_device, device)
     with torch.cuda.device(device):
         shapes = {op.dst: state_dict[op.srcs[0]].shape for op in mean_ops}
         computed = _run_elementwise(mean_ops, lambda op, j: state_dict[op.srcs[j]], shapes, device, out_device,
                                     group, stats)
 
-        world = dist.get_world_size(group) if group is not None else 1
-        rank = dist.get_rank(group) if group is not None else 0
-
         def cost(op):
-            o, i = state_dict[op.regmean[0][0]].shape
-            return i * i * i // 3 + 2 * len(op.regmean) * o * i * i + 2 * o * i * i
+            return _regmean_cost(state_dict, op)
 
-        lin_sizes = [int(state_dict[op.regmean[0][0]].numel()) for op in lin_ops]
-        lin_layout = ShardLayout(lin_sizes, world, cost=lambda i: cost(lin_ops[i]), align=1)
-        owner = lin_layout.owner
         results = {}
-        mine_lin = [idx for idx in range(len(lin_ops)) if owner[idx] == rank]
+        mine_lin = lin_layout.mine(rank)
         if mine_lin:
             _regmean_linears(lib, state_dict, grams, lin_ops, mine_lin, cost, alpha, device, solve_streams, results, stats)
 
@@ -608,4 +635,4 @@ def independent(state_dict):
             for k, v in state_dict.items()}
 
 
-__all__ = ["merge_weights", "sum_task_vectors", "regmean", "Merger", "independent", "WSUM", "SEQ_LERP", "MEAN"]
+__all__ = ["merge_weights", "sum_task_vectors", "regmean", "regmean_gram_owners", "Merger", "independent", "WSUM", "SEQ_LERP", "MEAN"]
