@@ -2,7 +2,8 @@
 of caches, all-reduces one of each pair and reduce-scatters the other by regmean_gram_owners, then compares the owned
 Grams and the sharded regmean results.  Pairs: fp32 and int8x4 (fp64 Grams), plain (NCCL) and symmetric=True
 (multimem).  2 ranks: one addition per element either way, so everything must match bit for bit; 4 ranks (where the
-box has them): the reductions may add in a different order.  Skipped with fewer than 2 GPUs."""
+box has them): the reductions may add in a different order.  Also: a symmetric cache's all_reduce() that must refuse
+leaves the cache as it was.  Skipped with fewer than 2 GPUs."""
 import os
 import socket
 import tempfile
@@ -94,6 +95,37 @@ def _compare(whole, scat, sd, rank, world):
     return res
 
 
+def _outside_arena(model, rank):
+    """A symmetric cache with a Gram outside its arena (a name register() did not know): all_reduce() must refuse on
+    every rank before it sums a counter, and all_reduce(packed=False) must then give what a plain cache gives."""
+    import vl_merging_b200 as vlm
+
+    sym, plain = vlm.GramCache(symmetric=True), vlm.GramCache()
+    for c in (sym, plain):
+        c.register(model)
+    gen = torch.Generator(device="cuda").manual_seed(90 + rank)
+    for name in ("transformer.blocks.0.attn.v", "not.registered"):
+        d = sym.buffers[name].shape[0] if name in sym.buffers else 64
+        x = torch.randint(-4, 5, (37, d), generator=gen, device="cuda").float()   # exact Grams, in any summation order
+        for c in (sym, plain):
+            c.accumulate(name, x)
+
+    def counts(c):
+        return {n: v for n, v in c.calls.items() if v}, {n: v for n, v in c.rows.items() if v}
+
+    before, refused = counts(sym), None
+    try:
+        sym.all_reduce()
+    except RuntimeError as e:
+        refused = str(e)
+    res = {"refused": refused, "counters_kept": counts(sym) == before}
+    sym.all_reduce(packed=False)
+    plain.all_reduce()
+    res["counters_equal"] = counts(sym) == counts(plain) and len(before[0]) == 2
+    res["grams_equal"] = all(torch.equal(sym.gram(n), plain.gram(n)) for n in before[0])
+    return res
+
+
 def _worker(rank, world, port, ret):
     import torch.distributed as dist
 
@@ -122,6 +154,7 @@ def _worker(rank, world, port, ret):
                 if not (whole.symmetric and "multicast" in str(e)):
                     raise
                 out[leg] = {"unsupported": str(e)}
+        out["outside_arena"] = _outside_arena(model, rank)
         ret[rank] = out
     finally:
         dist.destroy_process_group()
@@ -171,3 +204,11 @@ def test_nccl_reduce_scatter_matches_all_reduce(ranks, leg):
 @pytest.mark.parametrize("leg", ["fp32_mc", "int8x4_mc"])
 def test_multimem_reduce_scatter_matches_all_reduce(ranks, leg):
     _check(ranks, leg)
+
+
+def test_refused_symmetric_all_reduce_keeps_the_counters(ranks):
+    _, res = ranks
+    for r in (r["outside_arena"] for r in res):
+        assert "outside the symmetric arena" in (r["refused"] or ""), r["refused"]
+        assert r["counters_kept"]
+        assert r["counters_equal"] and r["grams_equal"]

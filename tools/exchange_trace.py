@@ -1,5 +1,7 @@
 """Development helper: where the time of GramCache.all_reduce() goes (host wall clock per phase, GPU drained after each).
 torchrun --nproc-per-node N tools/exchange_trace.py [--symmetric]
+    the phases are the library's own steps: exchange_plan (the buffer-set agreement and the counter all-reduce;
+    agree_on_buffers alone is timed too), the cache's multicast setup and its batched pack / unpack / mirror launches
 torchrun --nproc-per-node N tools/exchange_trace.py --reduce-scatter
     whole-call host time of reduce_scatter() (by regmean_gram_owners) against all_reduce(), for fp32 and fp64 caches,
     NCCL and multimem (symmetric=True), after a barrier and ending in a device synchronise; VLMo-base's 96 Grams."""
@@ -102,37 +104,25 @@ if "--reduce-scatter" in sys.argv:
     dist.destroy_process_group()
     sys.exit(0)
 
+L = vlm._lib.lib()
 for it in range(3):
     if rank == 0:
         print(f"--- iteration {it} ({'multimem' if symmetric else 'NCCL'}, world {world})", flush=True)
     timed("whole all_reduce()", lambda: cache.all_reduce())
-    names = timed("agree_on_buffers", lambda: G.agree_on_buffers(cache.buffers, None, None, device=dev))
-    timed("_reduce_counts", lambda: G._reduce_counts(cache.buffers, names, dict(cache.calls), dict(cache.rows), None))
+    timed("agree_on_buffers", lambda: G.agree_on_buffers(cache.buffers, None, None, device=dev))
+    plan = timed("exchange_plan", lambda: G.exchange_plan(cache.buffers, cache.calls, cache.rows, None,
+                                                          symmetric=symmetric, device=dev))
     x = torch.ones(134_544_384, device=dev)
     timed("NCCL all_reduce of 538 MB", lambda: dist.all_reduce(x))
     if symmetric:
         timed("handle.barrier()", lambda: cache._symm.barrier(channel=0))
-        from vl_merging_b200 import _lib
-        live = cache.live_names()
-        arena = cache._arenas[0]
-        spans = (_lib.SymSpan * len(live))()
-        for sp, n in zip(spans, live):
-            g = cache.buffers[n]
-            sp.offset_bytes, sp.d, sp.ld = g.data_ptr() - arena.data_ptr(), g.shape[0], g.stride(0)
+        mc, spans = cache._multicast_spans(plan.names, plan.mine, dist.group.WORLD)
         st = torch.cuda.current_stream().cuda_stream
-        L = _lib.lib()
-        mc = int(cache._symm.multicast_ptr)
-        timed("multimem kernel alone", lambda: _lib.check(L.vlm_sym_allreduce_multimem(mc, spans, len(live), 0, rank, world, st)))
-        items = _lib.sym_items([cache.buffers[n] for n in live])
-        timed("local mirror alone", lambda: _lib.check(L.vlm_sym_mirror_batch(items, len(live), 0, st)))
+        timed("multimem kernel alone", lambda: vlm._lib.check(L.vlm_sym_allreduce_multimem(
+            mc, spans, len(spans), cache._sym_code, rank, world, st)))
+        timed("local mirror alone", lambda: cache._sym_launch(L.vlm_sym_mirror_batch, plan.mine))
     else:
-        from vl_merging_b200 import _lib
-        live = cache.live_names()
-        grams = [cache.buffers[n] for n in live]
-        flat = torch.empty(sum(g.shape[0] * (g.shape[0] + 1) // 2 for g in grams), device=dev)
-        items = _lib.sym_items(grams, flat)
-        st = torch.cuda.current_stream().cuda_stream
-        L = _lib.lib()
-        timed("pack (one launch)", lambda: _lib.check(L.vlm_sym_pack_upper_batch(items, len(live), 0, st)))
-        timed("unpack (one launch)", lambda: _lib.check(L.vlm_sym_unpack_batch(items, len(live), 0, st)))
+        flat = torch.empty(len(plan.sections) * plan.width, device=dev)
+        timed("pack (one launch)", lambda: cache._sym_launch(L.vlm_sym_pack_upper_batch, plan.names, flat, plan.offsets))
+        timed("unpack (one launch)", lambda: cache._sym_launch(L.vlm_sym_unpack_batch, plan.mine, flat, plan.offsets))
 dist.destroy_process_group()

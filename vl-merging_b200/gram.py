@@ -17,6 +17,7 @@ torch.save(middle_representations, path)     GramCache.save(path): {name: fp64 C
 """
 import contextlib
 from collections import defaultdict
+from typing import NamedTuple
 
 import torch
 import torch.nn as nn
@@ -101,36 +102,92 @@ def agree_on_buffers(buffers, group=None, make=None, device=None):
     return sorted(union)
 
 
+class ExchangePlan(NamedTuple):
+    """What one packed Gram exchange moves (exchange_plan)."""
+    names: list      # the Grams that travel, in packed order
+    offsets: list    # element offset of each one's packed upper triangle in the flat buffer
+    sections: list   # elements per owner rank (all-reduce: one section, every live Gram)
+    width: int       # elements per section in the flat buffer: the largest section
+    mine: list       # the Grams whose sums this rank keeps, in packed order
+    nbytes: int      # last_reduce_bytes
+    calls: dict      # {agreed name: call count summed over the ranks}
+    rows: dict       # {agreed name: row count summed over the ranks}
+    owners: dict     # {name: rank} of the Grams that travel (None for an all-reduce)
+    rank: int
+    world: int
+
+
+def exchange_plan(buffers, calls, rows, group=None, owners=None, symmetric=False, make=None, device=None):
+    """The host side of a Gram exchange, the same for GramCache.all_reduce() and reduce_scatter(); any backend, no
+    CUDA.  Collectives, in this order on every rank: the buffer-set digest (agree_on_buffers, which creates zero
+    buffers with `make` for names missing here), one all-reduce of the call / row counters (none when no rank holds a
+    buffer), and, with `owners`, one digest of the owner map.  The caller's `calls` and `rows` are never written: their
+    sums come back in the plan, to be committed once every check has passed.  Raises ValueError on every rank alike
+    when the ranks passed different owner maps, or the map names a Gram that is not live or a rank outside the group.
+    owners None: every live Gram travels, back to back in live order, and every rank keeps all of them.  owners
+    {name: rank}: the owned Grams travel sorted by owner (stable, so in live order inside each owner's section),
+    section r at element r * width of a [world x width] buffer, and this rank keeps its own.
+    nbytes: what the NCCL transport moves (the whole flat buffer, padding included), or with `symmetric` what the
+    multimem one reduces for this rank (its own triangles)."""
+    import torch.distributed as dist
+
+    if device is None:
+        device = next(iter(buffers.values())).device if buffers else torch.device("cpu")
+    names = agree_on_buffers(buffers, group, make, device)
+    summed = {}
+    if names:
+        counts = torch.tensor([[calls.get(n, 0), rows.get(n, 0)] for n in names], dtype=torch.int64,
+                              device=buffers[names[0]].device)
+        dist.all_reduce(counts, group=group)
+        summed = dict(zip(names, counts.tolist()))
+    live = [n for n in names if summed[n][0] > 0]
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    if owners is None:
+        order, where = live, dict.fromkeys(live, 0)
+    else:
+        if not _same_everywhere(sorted(owners.items()), group, device):
+            raise ValueError("GramCache.reduce_scatter: the ranks passed different owner maps (build it on every rank "
+                             "from the same state_dict, config and world, and the live names every rank holds)")
+        for n, r in owners.items():
+            if n not in live:
+                raise ValueError(f"GramCache.reduce_scatter: owner map names {n!r}, which is not a live Gram of this cache "
+                                 "(build the map from cache.live_names())")
+            if not isinstance(r, int) or not 0 <= r < world:
+                raise ValueError(f"GramCache.reduce_scatter: owner {r!r} of {n!r} is not a rank of a {world}-rank group")
+        where = {n: owners[n] for n in live if n in owners}
+        order = sorted(where, key=where.get)
+    tri = {n: buffers[n].shape[0] * (buffers[n].shape[0] + 1) // 2 for n in order}
+    sections, offsets = [0] * (1 if owners is None else world), []
+    for n in order:
+        offsets.append(sections[where[n]])
+        sections[where[n]] += tri[n]
+    width = max(sections)
+    mine = [n for n in order if owners is None or where[n] == rank]
+    esz = buffers[names[0]].element_size() if names else 0
+    return ExchangePlan(
+        names=order, offsets=[where[n] * width + off for n, off in zip(order, offsets)], sections=sections,
+        width=width, mine=mine, nbytes=esz * (sum(tri[n] for n in mine) if symmetric else len(sections) * width),
+        calls={n: c for n, (c, _) in summed.items()}, rows={n: r for n, (_, r) in summed.items()},
+        owners=None if owners is None else where, rank=rank, world=world)
+
+
 def reduce_gram_buffers(buffers, arenas, calls, rows, group=None):
-    """Sum Gram buffers over the ranks of `group`: one all-reduce per flat arena (normally exactly one)
-    plus one per buffer that lives outside the arenas, then the per-name call / row counters, so every
+    """Sum Gram buffers over the ranks of `group`: the per-name call / row counters (exchange_plan), then one
+    all-reduce per flat arena (normally exactly one) plus one per buffer that lives outside the arenas, so every
     rank ends up with the same keys.  Works on any backend (NCCL on the GPUs, gloo in the CPU tests)."""
     import torch.distributed as dist
 
-    if buffers:
-        ref = next(iter(buffers.values()))
-        names = agree_on_buffers(buffers, group, lambda d: torch.zeros(d, d, dtype=ref.dtype, device=ref.device))
-    else:
-        names = agree_on_buffers(buffers, group, lambda d: torch.zeros(d, d))
+    ref = next(iter(buffers.values()), torch.zeros(0))
+    plan = exchange_plan(buffers, calls, rows, group, make=lambda d: torch.zeros(d, d, dtype=ref.dtype, device=ref.device))
     for arena in arenas:
         dist.all_reduce(arena, op=dist.ReduceOp.SUM, group=group)
     spans = [(a.data_ptr(), a.data_ptr() + a.numel() * a.element_size()) for a in arenas]
-    for name in names:
+    for name in plan.calls:     # every agreed name, live or not
         g = buffers[name]
         if not any(lo <= g.data_ptr() < hi for lo, hi in spans):
             dist.all_reduce(g, op=dist.ReduceOp.SUM, group=group)
-    _reduce_counts(buffers, names, calls, rows, group)
-
-
-def _reduce_counts(buffers, names, calls, rows, group):
-    import torch.distributed as dist
-
-    if names:
-        dev = buffers[names[0]].device
-        counts = torch.tensor([[calls[n], rows[n]] for n in names], dtype=torch.int64, device=dev)
-        dist.all_reduce(counts, group=group)
-        for n, (c, r) in zip(names, counts.tolist()):
-            calls[n], rows[n] = c, r
+    calls.update(plan.calls)
+    rows.update(plan.rows)
 
 
 class GramCache:
@@ -439,106 +496,83 @@ class GramCache:
         return [n for n in self.buffers if self.calls[n] > 0]
 
     def all_reduce(self, group=None, packed=True):
-        """Data-parallel calibration: sum the per-rank Gram buffers (ONE NCCL all-reduce over NVLink).
-        The reference has no such step (every DDP rank writes its own file, SURVEY.md §2.2).
-        packed: only the upper triangles of the Grams that fired travel — vlm_sym_pack_upper_batch (one launch) into one flat
-        buffer, one all-reduce of it (VLMo-base: 0.54 GB instead of the 1.17 GB arena with its lower triangles
-        and never-fired `vl` experts; twice that for the fp64 Grams of the int8x4 / fp64 modes), vlm_sym_unpack_batch
-        back into the full symmetric buffers (which leaves the cache finalized).  packed=False: one all-reduce of the
-        whole arena."""
-        import torch.distributed as dist
-
+        """Data-parallel calibration: sum the per-rank Gram buffers over the ranks of `group` onto every rank (the
+        reference has no such step: every DDP rank writes its own file, SURVEY.md §2.2).
+        packed: only the upper triangles of the Grams that fired travel (VLMo-base: 0.54 GB instead of the 1.17 GB arena
+        with its lower triangles and never-fired `vl` experts; twice that for the fp64 Grams of the int8x4 / fp64
+        modes).  Plain caches: one vlm_sym_pack_upper_batch into one flat buffer, ONE NCCL all-reduce, one
+        vlm_sym_unpack_batch back into the full symmetric buffers; symmetric caches: one vlm_sym_allreduce_multimem
+        launch between two cross-rank barriers, then the local mirror.  Every check that can fail runs, with the same
+        outcome on every rank, before the cache changes, so a refused call can be followed by all_reduce(packed=False):
+        one all-reduce of each whole arena and of each buffer outside them."""
         self._require_whole("all_reduce")
         self.flush()
-        if self.symmetric and packed:
-            return self._all_reduce_multimem(group)
         if not packed:
             return reduce_gram_buffers(self.buffers, self._arenas, self.calls, self.rows, group)
-        live = self._agree_on_live(group)
-        if not live:
-            return
-        grams = [self.buffers[n] for n in live]
-        flat = torch.empty(sum(g.shape[0] * (g.shape[0] + 1) // 2 for g in grams), dtype=self.dtype, device=self.device)
-        stream = torch.cuda.current_stream(self.device).cuda_stream
-        items = _lib.sym_items(grams, flat)
-        _lib.check(self._lib.vlm_sym_pack_upper_batch(items, len(live), self._sym_code, stream))   # one launch for all Grams
-        dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
-        _lib.check(self._lib.vlm_sym_unpack_batch(items, len(live), self._sym_code, stream))
-        self._finalized = True
-        self.last_reduce_bytes = flat.numel() * flat.element_size()
+        self._exchange(group)
 
     def reduce_scatter(self, owners, group=None):
         """Data-parallel calibration followed by a sharded regmean(..., group=group): sum each Gram over the ranks of
         `group` onto its owner only.  owners: {Gram name: rank in group}, normally
         regmean_gram_owners(state_dict, config, cache.live_names(), world, num_layers) with the arguments regmean will
         get; it must name live Grams only, and live Grams it leaves out (ones no regmean problem reads) are not summed.
+        All ranks must pass the same map.
         Plain caches: the owned upper triangles are packed by owner into [world x width] (width: the largest owner's
         section; one vlm_sym_pack_upper_batch), ONE NCCL reduce-scatter, and this rank's section unpacked into its
         Grams (one vlm_sym_unpack_batch): each rank sends (world - 1) / world of the buffer instead of the all-reduce's
         2 (world - 1) / world, and unpacks only its own Grams.  Symmetric caches: one vlm_sym_reduce_multimem
-        launch over this rank's Grams between two cross-rank barriers, then their local mirror.
+        launch over this rank's Grams between two cross-rank barriers, then their local mirror.  Checks as in
+        all_reduce(), the owner map's included, before the cache changes.
         Afterwards the cache is scattered: `owners` records the map, this rank's own Grams hold the full symmetric
         sums and gram() returns them; the other Grams, state_dict() / save() / save_packed(), all_reduce() and
         further accumulation raise until reset().  live_names() is still the full agreed list on every rank."""
-        import torch.distributed as dist
-
         self._require_whole("reduce_scatter")
         self.flush()
+        self._exchange(group, owners)
+
+    def _exchange(self, group, owners=None):
+        """Both packed exchanges: the plan (agreement, counters, owner-map checks), the multicast setup of a symmetric
+        cache (its checks and rendezvous), then the commit and one transport."""
+        import torch.distributed as dist
+
         group = group if group is not None else dist.group.WORLD
-        rank, world = dist.get_rank(group), dist.get_world_size(group)
-        names = agree_on_buffers(self.buffers, group,
-                                 lambda d: torch.zeros(d, d, dtype=self.dtype, device=self.device), device=self.device)
-        calls, rows = defaultdict(int, self.calls), defaultdict(int, self.rows)
-        _reduce_counts(self.buffers, names, calls, rows, group)
-        # every check that can fail comes before the cache's own counters change (the same outcome on every rank: the
-        # summed counters, the owner map and the arena are the same everywhere)
-        live = [n for n in names if calls[n] > 0]
-        if not _same_everywhere(sorted(owners.items()), group, self.device):
-            raise ValueError("GramCache.reduce_scatter: the ranks passed different owner maps (build it on every rank "
-                             "from the same state_dict, config and world, and the live names every rank holds)")
-        for n, r in owners.items():
-            if n not in live:
-                raise ValueError(f"GramCache.reduce_scatter: owner map names {n!r}, which is not a live Gram of this cache "
-                                 "(build the map from cache.live_names())")
-            if not isinstance(r, int) or not 0 <= r < world:
-                raise ValueError(f"GramCache.reduce_scatter: owner {r!r} of {n!r} is not a rank of a {world}-rank group")
-        owned = [n for n in live if n in owners]
+        plan = exchange_plan(self.buffers, self.calls, self.rows, group, owners, self.symmetric,
+                             lambda d: torch.zeros(d, d, dtype=self.dtype, device=self.device), self.device)
+        if owners is None and not plan.names:
+            return                             # no Gram fired on any rank
         if self.symmetric:
-            mc, spans = self._multicast_spans(owned, [n for n in owned if owners[n] == rank], group)
-        self.calls.update(calls)
-        self.rows.update(rows)
-        self.owners, self._rank = {n: owners[n] for n in owned}, rank
+            mc, spans = self._multicast_spans(plan.names, plan.mine, group)
+        self.calls.update(plan.calls)
+        self.rows.update(plan.rows)
+        if owners is not None:
+            self.owners, self._rank = plan.owners, plan.rank
         self._finalized = True
-        esz = 8 if self.dtype == torch.float64 else 4
-        mine = [n for n in owned if owners[n] == rank]
+        self.last_reduce_bytes = plan.nbytes
+        if not plan.names:
+            return
         stream = torch.cuda.current_stream(self.device).cuda_stream
         if self.symmetric:
             with torch.cuda.device(self.device):
-                self._symm.barrier(channel=0)      # every rank's Gram launches have completed
-                _lib.check(self._lib.vlm_sym_reduce_multimem(mc, self._arenas[0].data_ptr(), spans, len(spans),
-                                                             self._sym_code, stream))
-                self._symm.barrier(channel=0)      # nobody reads a rank's arena any more
-                self._mirror(mine, stream)
-            self.last_reduce_bytes = sum(self.buffers[n].shape[0] * (self.buffers[n].shape[0] + 1) // 2 for n in mine) * esz
+                self._symm.barrier(channel=0)  # every rank's Gram launches have completed
+                if owners is None:             # every sum stored into every rank's arena (multimem.st)
+                    _lib.check(self._lib.vlm_sym_allreduce_multimem(mc, spans, len(spans), self._sym_code, plan.rank,
+                                                                    plan.world, stream))
+                else:                          # this rank's sums stored into its own arena only
+                    _lib.check(self._lib.vlm_sym_reduce_multimem(mc, self._arenas[0].data_ptr(), spans, len(spans),
+                                                                 self._sym_code, stream))
+                self._symm.barrier(channel=0)  # every store has landed, and nobody reads a rank's arena any more
+                self._sym_launch(self._lib.vlm_sym_mirror_batch, plan.mine)     # lower triangles, locally
             return
-        tri = {n: self.buffers[n].shape[0] * (self.buffers[n].shape[0] + 1) // 2 for n in owned}
-        order = sorted(owned, key=lambda n: self.owners[n])         # stable: live order inside each owner's section
-        section, offsets = [0] * world, []
-        for n in order:
-            offsets.append(section[self.owners[n]])
-            section[self.owners[n]] += tri[n]
-        width = max(section)
-        self.last_reduce_bytes = world * width * esz
-        if width == 0:
-            return
-        flat = torch.empty(world * width, dtype=self.dtype, device=self.device)    # padding is summed, never read
-        items = _lib.sym_items([self.buffers[n] for n in order], flat,
-                               [self.owners[n] * width + off for n, off in zip(order, offsets)])
-        _lib.check(self._lib.vlm_sym_pack_upper_batch(items, len(order), self._sym_code, stream))
-        out = torch.empty(width, dtype=self.dtype, device=self.device)
-        dist.reduce_scatter_tensor(out, flat, op=dist.ReduceOp.SUM, group=group)
-        items = _lib.sym_items([self.buffers[n] for n in mine], out)      # this rank's section, in the same order
-        _lib.check(self._lib.vlm_sym_unpack_batch(items, len(mine), self._sym_code, stream))
+        flat = torch.empty(len(plan.sections) * plan.width, dtype=self.dtype, device=self.device)  # padding: never read
+        self._sym_launch(self._lib.vlm_sym_pack_upper_batch, plan.names, flat, plan.offsets)
+        if owners is None:
+            dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
+            out, base = flat, 0
+        else:
+            out, base = torch.empty(plan.width, dtype=self.dtype, device=self.device), plan.rank * plan.width
+            dist.reduce_scatter_tensor(out, flat, op=dist.ReduceOp.SUM, group=group)
+        offset = dict(zip(plan.names, plan.offsets))
+        self._sym_launch(self._lib.vlm_sym_unpack_batch, plan.mine, out, [offset[n] - base for n in plan.mine])
 
     def _require_whole(self, what, name=None):
         """Raise if this cache was reduce_scatter()ed (and `name`, when given, is not one of this rank's Grams)."""
@@ -579,65 +613,19 @@ class GramCache:
             sp.offset_bytes, sp.d, sp.ld = g.data_ptr() - lo, g.shape[0], g.stride(0)
         return mc, spans
 
-    def _agree_on_live(self, group):
-        """The first step of both exchanges: every rank agrees on the buffer set (creating zero buffers for names it
-        lacks) and sums the call / row counters; returns the names that fired on some rank, the same list everywhere."""
-        names = agree_on_buffers(self.buffers, group,
-                                 lambda d: torch.zeros(d, d, dtype=self.dtype, device=self.device), device=self.device)
-        _reduce_counts(self.buffers, names, self.calls, self.rows, group)
-        return [n for n in names if self.calls[n] > 0]
-
-    def _all_reduce_multimem(self, group=None):
-        """all_reduce() of a symmetric cache: one kernel over the NVSwitch multicast mapping of the arena, bracketed by
-        two cross-rank barriers on the current stream.  Every rank ends with bit-identical, fully symmetric Grams."""
-        import torch.distributed as dist
-        import torch.distributed._symmetric_memory as symm_mem
-
-        group = group if group is not None else dist.group.WORLD
-        live = self._agree_on_live(group)
-        if not live:
-            return
-        if len(self._arenas) != 1:
-            raise RuntimeError("GramCache(symmetric=True): no symmetric arena (register() the model before calibrating)")
-        arena = self._arenas[0]
-        lo, hi = arena.data_ptr(), arena.data_ptr() + arena.numel() * arena.element_size()
-        if any(not (lo <= self.buffers[n].data_ptr() < hi) for n in live):
-            raise RuntimeError("GramCache(symmetric=True): a Gram buffer lives outside the symmetric arena (a module whose "
-                               "width was unknown at register()); use a plain cache (NCCL exchange) for this model")
-        if self._symm is None:
-            self._symm = symm_mem.rendezvous(arena, group)          # collective: every rank, same order
-        h = self._symm
-        mc = int(h.multicast_ptr or 0)
-        if mc == 0:
-            raise RuntimeError("GramCache(symmetric=True): this system offers no multicast mapping (NVSwitch + driver "
-                               "support needed); use a plain cache (NCCL exchange)")
-        spans = (_lib.SymSpan * len(live))()
-        for sp, n in zip(spans, live):
-            g = self.buffers[n]
-            sp.offset_bytes, sp.d, sp.ld = g.data_ptr() - lo, g.shape[0], g.stride(0)
-        stream = torch.cuda.current_stream(self.device).cuda_stream
-        with torch.cuda.device(self.device):
-            h.barrier(channel=0)               # every rank's Gram launches have completed
-            _lib.check(self._lib.vlm_sym_allreduce_multimem(mc, spans, len(live), self._sym_code, dist.get_rank(group),
-                                                            dist.get_world_size(group), stream))
-            h.barrier(channel=0)               # every rank's stores have landed everywhere
-            self._mirror(live, stream)         # lower triangles, locally
-        self._finalized = True
-        esz = 8 if self.dtype == torch.float64 else 4
-        self.last_reduce_bytes = sum(self.buffers[n].shape[0] * (self.buffers[n].shape[0] + 1) // 2 for n in live) * esz
-
     def finalize(self):
         """Mirror the upper triangles into the lower ones (after the last accumulate / all_reduce)."""
         self.flush()
         if self._finalized:
             return
-        self._mirror(self.live_names(), torch.cuda.current_stream(self.device).cuda_stream)
+        self._sym_launch(self._lib.vlm_sym_mirror_batch, self.live_names())
         self._finalized = True
 
-    def _mirror(self, names, stream):
-        """The lower triangles of the named Grams from their upper ones, in place: one launch."""
-        items = _lib.sym_items([self.buffers[n] for n in names])
-        _lib.check(self._lib.vlm_sym_mirror_batch(items, len(names), self._sym_code, stream))
+    def _sym_launch(self, fn, names, packed=None, offsets=None):
+        """One batched vlm_sym_* launch (pack_upper, unpack or mirror) over the named Grams, on the current stream;
+        packed / offsets as in _lib.sym_items."""
+        items = _lib.sym_items([self.buffers[n] for n in names], packed, offsets)
+        _lib.check(fn(items, len(names), self._sym_code, torch.cuda.current_stream(self.device).cuda_stream))
 
     def gram(self, name):
         """Full symmetric fp32 Gram of one module, on the device (of a scattered cache: one this rank owns)."""
