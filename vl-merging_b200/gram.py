@@ -190,6 +190,41 @@ def reduce_gram_buffers(buffers, arenas, calls, rows, group=None):
     rows.update(plan.rows)
 
 
+def _gram_route(precision, use_simt, dtype, rows, d, ptr, ldx, seg_stride):
+    """Which library call takes a GramCache activation of rows x d `dtype` elements at byte address ptr, row pitch ldx
+    and segment pitch seg_stride (0: plain rows) in elements: "i8x4", "f64" or "simt" (vlm_syrk_accum_i8x4 / _f64 /
+    _simt; simt: exact fp32 products on CUDA cores), "split" (vlm_tf32_split, then the Gram of its {hi, lo} planes) or
+    "library" (vlm_syrk_accum / _strided / _batch, which pick the CTA-pair or the CUDA-core kernel themselves)."""
+    if precision in ("int8x4", "fp64"):
+        aligned = ptr % 16 == 0 and ldx % 4 == 0 and seg_stride % 4 == 0
+        return "i8x4" if precision == "int8x4" and d % 128 == 0 and rows * d >= 1 << 20 and aligned else "f64"
+    if use_simt:
+        return "simt"
+    if precision == "tf32x3" and dtype == torch.float32:   # what vlm_tf32_split and the split kernel take
+        return "simt" if d % 32 or ptr % 16 or ldx % 4 or seg_stride % 4 else "split"
+    return "library"
+
+
+_DEFERRED_ROUTES = ("split", "library")   # the routes vlm_syrk_accum_batch takes: no CUDA-core-only or fp64 form
+
+
+class _GramLaunch(NamedTuple):
+    """One hooked activation on its way to a Gram entry point (GramCache._launch); GramCache._pending holds the
+    deferred ones.  bench.py's TimedCache reads fields 4 and 5 of a pending record as (rows, d): keep the order."""
+    code: int             # _DTYPES code of the activation
+    keep: torch.Tensor    # the tensor the activation is read from, referenced until its launch is issued
+    g: torch.Tensor       # the Gram buffer
+    ptr: int              # byte address of the first row
+    rows: int
+    d: int
+    ldx: int              # row pitch, elements
+    seg_rows: int         # row slice: rows per segment (0: plain rows)
+    seg_stride: int       # row slice: elements between the first rows of consecutive segments
+    name: str
+    version: int          # keep._version at hook time
+    route: str            # _gram_route
+
+
 class GramCache:
     """Accumulates G[name] += X^T X for every hooked module call, on the GPU (fp32 Grams from one TF32 tensor-core pass by
     default; exact fp64 Grams from the integer tensor cores or the fp64 pipe on request: `precision`).
@@ -263,7 +298,7 @@ class GramCache:
         self._finalized = True
         self.enabled = True    # False: the hooks stay registered but ignore their calls
         self.defer_bytes, self.max_pending, self.max_pending_bytes = int(defer_bytes), int(max_pending), int(max_pending_bytes)
-        self._pending = []     # (dtype code, keep-alive tensor, g, ptr, rows, d, ldx, seg_rows, seg_stride)
+        self._pending = []     # _GramLaunch records of the deferred activations
         self._pending_bytes = 0
         self.symmetric, self._symm = bool(symmetric), None   # symmetric-memory arena and its rendezvous handle
         self._side = torch.cuda.Stream(self.device) if side_stream else None
@@ -327,13 +362,8 @@ class GramCache:
                 x2 = x2.contiguous()
             rows, ldx, keep = x2.shape[0], (x2.stride(0) if x2.shape[0] > 1 else d), x2
         ptr = keep.data_ptr()
-        # tf32x3 splits fp32 activations that vlm_tf32_split and the split kernel take (d % 32 == 0, 16-byte aligned x,
-        # ldx and seg_stride multiples of 4); any other one goes to the CUDA-core kernel (exact fp32 products) at once:
-        # it must not join a deferred group, which flush() issues as split planes
-        split = self.precision == "tf32x3" and keep.dtype == torch.float32
-        simt = self._use_simt or (split and bool(d % 32 or ptr % 16 or ldx % 4 or seg_stride % 4))
-        split = split and not simt
-        if simt and seg_rows:
+        route = _gram_route(self.precision, self._use_simt, keep.dtype, rows, d, ptr, ldx, seg_stride)
+        if route == "simt" and seg_rows:
             keep = x.contiguous()        # the CUDA-core kernel takes plain rows only
             ptr, ldx, seg_rows, seg_stride = keep.data_ptr(), d, 0, 0
         g = self.buffers.get(name)
@@ -344,37 +374,44 @@ class GramCache:
         self.calls[name] += 1
         self.rows[name] += rows
         self._finalized = False
-        code = _DTYPES[keep.dtype]
+        rec = _GramLaunch(_DTYPES[keep.dtype], keep, g, ptr, rows, d, ldx, seg_rows, seg_stride, name, keep._version, route)
         nbytes = rows * ldx * elem
-        if self.precision == "int8x4" and d % 128 == 0 and rows * d >= (1 << 20) \
-                and ptr % 16 == 0 and ldx % 4 == 0 and seg_stride % 4 == 0:
-            nbytes = int(self._lib.vlm_syrk_i8x4_scratch_bytes(rows, d))
-            scratch = self._plane_scratch((nbytes + 3) // 4)
-            _lib.check(self._lib.vlm_syrk_accum_i8x4(ptr, code, rows, d, ldx, seg_rows, seg_stride, scratch.data_ptr(),
-                                                     nbytes, g.data_ptr(), g.stride(0), self._launch_stream(keep)))
-            return
-        if self.dtype == torch.float64:
-            _lib.check(self._lib.vlm_syrk_accum_f64(ptr, code, rows, d, ldx, seg_rows, seg_stride,
-                                                    g.data_ptr(), g.stride(0), self._launch_stream(keep)))
-            return
-        if 0 < nbytes <= self.defer_bytes and not simt:
-            self._pending.append((code, keep, g, ptr, rows, d, ldx, seg_rows, seg_stride, name, keep._version))
+        if route in _DEFERRED_ROUTES and 0 < nbytes <= self.defer_bytes:
+            self._pending.append(rec)
             self._pending_bytes += nbytes
             if len(self._pending) >= self.max_pending or self._pending_bytes >= self.max_pending_bytes:
                 self.flush()
             return
-        stream = self._launch_stream(keep)
-        if split:
-            planes = self._plane_scratch(2 * rows * d)
-            _lib.check(self._lib.vlm_tf32_split(ptr, rows, d, ldx, seg_rows, seg_stride, planes.data_ptr(), stream))
-            _lib.check(self._lib.vlm_syrk_accum(planes.data_ptr(), _lib.VLM_TF32X2, rows, d, d, g.data_ptr(),
-                                                g.stride(0), stream))
-        elif seg_rows:
-            _lib.check(self._lib.vlm_syrk_accum_strided(ptr, code, rows, d, ldx, seg_rows, seg_stride, g.data_ptr(),
-                                                        g.stride(0), stream))
+        self._launch([rec], self._launch_stream(keep), grouped=False)
+
+    def _launch(self, recs, stream, grouped):
+        """Issue the Gram launches of `recs` on `stream`: one record on its route's single-launch entry point, or
+        (grouped) records of one dtype and route as ONE vlm_syrk_accum_batch, whose schedule is not the single launch's."""
+        lib, route = self._lib, recs[0].route
+        if route == "split":   # each record's {hi, lo} planes, back to back in the scratch, stand in for its activation
+            planes = self._plane_scratch(sum(2 * r.rows * r.d for r in recs)).data_ptr()
+            recs = list(recs)
+            for i, r in enumerate(recs):
+                _lib.check(lib.vlm_tf32_split(r.ptr, r.rows, r.d, r.ldx, r.seg_rows, r.seg_stride, planes, stream))
+                recs[i] = r._replace(code=_lib.VLM_TF32X2, ptr=planes, ldx=r.d, seg_rows=0, seg_stride=0)
+                planes += 8 * r.rows * r.d
+        if grouped:
+            probs = (_lib.SyrkProblem * len(recs))(*(_lib.SyrkProblem(x=r.ptr, rows=r.rows, ldx=r.ldx, g=r.g.data_ptr(),
+                ldg=r.g.stride(0), d=r.d, seg_rows=r.seg_rows, seg_stride=r.seg_stride) for r in recs))
+            return _lib.check(lib.vlm_syrk_accum_batch(probs, len(recs), recs[0].code, stream))
+        (r,) = recs
+        g, ldg = r.g.data_ptr(), r.g.stride(0)
+        if route == "i8x4":
+            nbytes = int(lib.vlm_syrk_i8x4_scratch_bytes(r.rows, r.d))
+            scratch = self._plane_scratch((nbytes + 3) // 4).data_ptr()
+            _lib.check(lib.vlm_syrk_accum_i8x4(r.ptr, r.code, r.rows, r.d, r.ldx, r.seg_rows, r.seg_stride, scratch, nbytes,
+                                               g, ldg, stream))
+        elif route == "f64" or r.seg_rows:
+            fn = lib.vlm_syrk_accum_f64 if route == "f64" else lib.vlm_syrk_accum_strided
+            _lib.check(fn(r.ptr, r.code, r.rows, r.d, r.ldx, r.seg_rows, r.seg_stride, g, ldg, stream))
         else:
-            fn = self._lib.vlm_syrk_accum_simt if simt else self._lib.vlm_syrk_accum
-            _lib.check(fn(ptr, code, rows, d, ldx, g.data_ptr(), g.stride(0), stream))
+            fn = lib.vlm_syrk_accum_simt if route == "simt" else lib.vlm_syrk_accum
+            _lib.check(fn(r.ptr, r.code, r.rows, r.d, r.ldx, g, ldg, stream))
 
     def _plane_scratch(self, numel):
         """fp32 scratch of at least `numel` elements for the {hi, lo} planes.  One buffer, reused by every launch:
@@ -421,31 +458,13 @@ class GramCache:
             return self._join()
         pending, self._pending, self._pending_bytes = self._pending, [], 0
         for p in pending:   # an in-place write to a held activation bumps its version counter: refuse to use it
-            if p[1]._version != p[10]:
+            if p.keep._version != p.version:
                 raise RuntimeError(
-                    f"GramCache: the activation hooked for {p[9]} was modified in place before the deferred Gram launch "
+                    f"GramCache: the activation hooked for {p.name} was modified in place before the deferred Gram launch "
                     "(its Gram would be taken of the modified values); use defer_bytes=0 for this model")
-        pending = [p[:9] for p in pending]
         stream = self._launch_stream()
-        for code in sorted({p[0] for p in pending}):
-            group = [p for p in pending if p[0] == code]
-            probs = (_lib.SyrkProblem * len(group))()
-            # split mode: accumulate() defers only fp32 activations the split takes, so all of this group is split; the
-            # planes of every problem, back to back in the scratch
-            split = self.precision == "tf32x3" and code == _lib.VLM_F32
-            if split:
-                planes = self._plane_scratch(sum(2 * p[4] * p[5] for p in group))
-                off = 0
-            for q, (_, _keep, g, ptr, rows, d, ldx, seg_rows, seg_stride) in zip(probs, group):
-                if split:
-                    dst = planes.data_ptr() + off * 4
-                    _lib.check(self._lib.vlm_tf32_split(ptr, rows, d, ldx, seg_rows, seg_stride, dst, stream))
-                    off += 2 * rows * d
-                    q.x, q.rows, q.ldx, q.g, q.ldg, q.d, q.seg_rows, q.seg_stride = dst, rows, d, g.data_ptr(), g.stride(0), d, 0, 0
-                else:
-                    q.x, q.rows, q.ldx, q.g, q.ldg, q.d = ptr, rows, ldx, g.data_ptr(), g.stride(0), d
-                    q.seg_rows, q.seg_stride = seg_rows, seg_stride
-            _lib.check(self._lib.vlm_syrk_accum_batch(probs, len(group), _lib.VLM_TF32X2 if split else code, stream))
+        for key in sorted({(p.code, p.route) for p in pending}):   # a cache defers each dtype on one route only
+            self._launch([p for p in pending if (p.code, p.route) == key], stream, grouped=True)
         self._join()
         # `pending` (and with it the activations) is released here: the launches are already ordered on the stream
 
